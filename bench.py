@@ -7,7 +7,13 @@ frame of a bundled scene.  A "step" is one frame: generateRays -> shade -> blend
 repeat.scene at 7680x4320, 64 jittered spp (configs[4]; it fits one GPU).  The other eight
 configs ride in the same JSON line under `per_config` (N = 1).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes, after the timed steps, the frames the last timed step of each timed path returned, as float32
+DIR/<name>.npy: `frame` (the device-resident step's RGB frame), `frame_rgba8` (the RGBA8 frame the e2e step downloaded)
+and `per_config_<workload>` (each per-config frame).  A frame of more than DUMP_PIXELS pixels is cut to a fixed, seeded
+sample of DUMP_PIXELS pixels (rows of the [H*W, C] view, ascending), so that two builds run with the same arguments can
+be compared output for output: every input (scene, assets, jitter pattern, RNG seed) is fixed by the arguments.
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL): the frame's 16x16 tiles are dealt
 round-robin to the ranks, each rank renders its tiles from its own atomic tile queue and its kernel
@@ -53,6 +59,41 @@ E2E_BANDS = 4
 CPU_SAMPLE_PRIMARY = 40e6   # primary samples of the headline's CPU sample (~10-20 s on 16-32 cores)
 REF_STEP_PRIMARY = 9e6      # primary samples per step of the reference arm (cfg1 / cfg2: the whole frame)
 MINI_SAMPLE_PRIMARY = 2.5e6  # per_config parity samples
+DUMP_PIXELS = 1 << 18       # --dump-outputs: pixels kept per frame (10 frames of <= 16 B / pixel: at most 31 MB in all)
+DUMP_SEED = 2024
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_rows(W, H):
+    """The pixels --dump-outputs keeps of a W x H frame, as ascending row indices of its [H*W, C] view: None (all of them)
+    up to DUMP_PIXELS pixels, else the same seeded sample of DUMP_PIXELS for every run at this size."""
+    import numpy as np
+    if W * H <= DUMP_PIXELS:
+        return None
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(W * H, DUMP_PIXELS, replace=False))
+
+
+def dump_frame(frame, rows):
+    """float32 host copy of `frame` ([H, W, C], a torch tensor on the device or a numpy array), cut to `rows` (dump_rows)."""
+    import numpy as np
+    import torch
+    if torch.is_tensor(frame):
+        if rows is not None:
+            frame = frame.reshape(-1, frame.shape[-1])[torch.from_numpy(rows).to(frame.device)]
+        return frame.float().cpu().numpy()
+    if rows is not None:
+        frame = frame.reshape(-1, frame.shape[-1])[rows]
+    return frame.astype(np.float32)
+
+
+def write_dumps(directory, arrays):
+    """--dump-outputs: every array as <directory>/<name>.npy."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, "dumped outputs would take %d bytes" % total
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def _peaks():
@@ -282,16 +323,21 @@ def gpu_parity(run, res, windows, margin):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline and e2e arms (the f64, in-process and per-config arms time min(K, 5))")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-per-config", action="store_true")
     ap.add_argument("--no-inprocess", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frames of the last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU path's frames; --impl reference has none")
         return run_reference(args)
 
     import numpy as np
@@ -373,6 +419,10 @@ def main():
     if sampler:
         sampler.start()
     total_ms, kern_total_ms = time_device(run, device_step, barrier, args.steps, 0, flush)
+    dumps = {}
+    if args.dump_outputs and rank == 0:
+        dump_sel = dump_rows(W, H)
+        dumps["frame"] = dump_frame(frame, dump_sel)
     t = torch.tensor([total_ms, kern_total_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -435,6 +485,8 @@ def main():
         return float(tt.item())
 
     e2e_s = time_e2e("u8", out_u8, args.steps)
+    if args.dump_outputs and rank == 0:
+        dumps["frame_rgba8"] = dump_frame(out_u8, dump_sel)
     e2e_value = rays_per_frame * args.steps / e2e_s / 1e6
     clocks = sampler.stop() if sampler else None  # sampled over both timed regions
     # the same with the f64 frame (24 B / pixel: Bitmap.pixels, Image.fs:30), a few steps
@@ -554,8 +606,10 @@ def main():
                     ev[1].record()
                 api.assemble_device(r.p_f32, [r.tiles.data_ptr()], r.frame.data_ptr(), stream=stream)
 
-            k = 5
+            k = min(args.steps, 5)
             tot, kern = time_device(r, step, torch.cuda.synchronize, k, 3, flush)
+            if args.dump_outputs:
+                dumps["per_config_" + name] = dump_frame(r.frame, dump_rows(r.W, r.H))
             host = np.empty((r.H, r.W, 4), dtype=np.uint8)
             pu8 = api.make_params(r.W, r.H, r.spp, r.jit, seed=RNG_SEED, out_format=abi.OUT_RGBA8)
             for _ in range(2):
@@ -578,6 +632,8 @@ def main():
             r.close()
         line["per_config"] = per
     if rank == 0:
+        if args.dump_outputs:
+            write_dumps(args.dump_outputs, dumps)
         print(json.dumps(line))
     if world > 1 or args.no_per_config:
         scene.close()

@@ -1,7 +1,7 @@
-"""The workloads of bench.py / the parity suites are emitted by functracer_b200/scenes.py because /root/reference does
-not exist on the GPU box.  This test (CPU, runs where the reference checkout is present) parses the reference's OWN
-scene files - /root/reference/Scenes/*.scene with only the BASELINE.md §3 edits: `res` / `samples` lines inserted, the
-three unshipped asset paths substituted, house.scene:17 dropped - and asserts that they flatten to the same
+"""The workloads of bench.py / the parity suites are emitted by functracer_b200/scenes.py because the reference's scene
+files are not part of this repository.  This test (CPU, runs where FTB_REFERENCE_DIR names a checkout of the reference)
+parses the reference's OWN scene files - Scenes/*.scene with only the BASELINE.md §3 edits: `res` / `samples` lines
+inserted, the three unshipped asset paths substituted, house.scene:17 dropped - and asserts that they flatten to the same
 ftb_scene_desc, camera and options, field for field, as the builders' texts.  So every number measured on a
 scenes.py workload is a number for the reference's scene file."""
 import os
@@ -12,7 +12,8 @@ import pytest
 from functracer_b200 import scenes
 from util import REFERENCE_SCENES, desc_tables, parse, reference_scene_text
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REFERENCE_SCENES), reason="the reference checkout is not on this machine")
+pytestmark = pytest.mark.skipif(not (REFERENCE_SCENES and os.path.isdir(REFERENCE_SCENES)),
+                                reason="set FTB_REFERENCE_DIR to a checkout of antonburger/FuncTracer to compare with its scene files")
 
 # BASELINE.json config -> the reference file it names
 FILES = {

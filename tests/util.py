@@ -1,4 +1,6 @@
 """Shared helpers for the parity tests."""
+import os
+
 import numpy as np
 
 from functracer_b200 import abi, frontend, scenes
@@ -29,8 +31,9 @@ def colour_stats(a, b):
     return dict(max=float(d.max()), frac_within=float((d <= 1.0 / 255.0).mean()))
 
 
-# ---- the reference's own scene files ---------------------------------------------------------------------------
-REFERENCE_SCENES = "/root/reference/Scenes"
+# ---- the reference's own scene files: Scenes/ of an antonburger/FuncTracer checkout named by FTB_REFERENCE_DIR ----
+# (not part of this repository; the tests that read them skip without it)
+REFERENCE_SCENES = os.path.join(os.environ["FTB_REFERENCE_DIR"], "Scenes") if os.environ.get("FTB_REFERENCE_DIR") else None
 # the three assets the reference does not ship -> the generated stand-ins (functracer_b200/scenes.py)
 ASSET_SUBSTITUTES = {
     "c:\\Temp\\env4.jpg": "env4.ppm",
@@ -40,11 +43,10 @@ ASSET_SUBSTITUTES = {
 
 
 def reference_scene_text(file_name, res=None, spp=None, mesh=None, depth=None):
-    """The text of /root/reference/Scenes/<file_name> with only what BASELINE.md §3 allows changed: `res` / `samples`
+    """The text of the reference's Scenes/<file_name> with only what BASELINE.md §3 allows changed: `res` / `samples`
     option lines inserted after the scene's own option lines (the grammar is options -> objects -> lights and later
     setters win, SceneParser.fs:357-364), the three missing asset paths substituted, and house.scene:17 (a comment
     inside a group: a parse error at HEAD) dropped."""
-    import os
     import re
     lines = open(os.path.join(REFERENCE_SCENES, file_name), encoding="utf-8").read().splitlines()
     if file_name == "house.scene":
