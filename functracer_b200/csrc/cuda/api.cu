@@ -92,21 +92,19 @@ __global__ void widen_kernel(const R* in, double* out, long long n)
 namespace ftb {
 static_assert((unsigned)FT_TABLE == kFeatOriginTable, "lower.h and device_scene.h disagree on the table feature bit");
 // kernel variants compiled by the Makefile (render_variant.cu), listed through -DFTB_FEAT_LIST_F32 / _F64
-#define X(feat) cudaError_t launch_f32_##feat(const DevScene<float>&, const DevFrame<float>&, bool, int, cudaStream_t, int*); \
-    cudaError_t launch_wf_f32_##feat(const DevScene<float>&, const DevFrame<float>&, int, int, bool, int, void*, size_t, cudaStream_t, int*);
+#define X(feat) cudaError_t launch_f32_##feat(const DevScene<float>&, const DevFrame<float>&, bool, int, cudaStream_t, int*);
 FTB_FEAT_LIST_F32
 #undef X
-#define X(feat) cudaError_t launch_f64_##feat(const DevScene<double>&, const DevFrame<double>&, bool, int, cudaStream_t, int*); \
-    cudaError_t launch_wf_f64_##feat(const DevScene<double>&, const DevFrame<double>&, int, int, bool, int, void*, size_t, cudaStream_t, int*);
+#define X(feat) cudaError_t launch_f64_##feat(const DevScene<double>&, const DevFrame<double>&, bool, int, cudaStream_t, int*);
 FTB_FEAT_LIST_F64
 #undef X
 static const Variant<float> kVariantsF32[] = {
-#define X(feat) {(unsigned)(feat), UnitCap<float, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f32_##feat, launch_wf_f32_##feat},
+#define X(feat) {(unsigned)(feat), UnitCap<float, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f32_##feat},
     FTB_FEAT_LIST_F32
 #undef X
 };
 static const Variant<double> kVariantsF64[] = {
-#define X(feat) {(unsigned)(feat), UnitCap<double, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f64_##feat, launch_wf_f64_##feat},
+#define X(feat) {(unsigned)(feat), UnitCap<double, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f64_##feat},
     FTB_FEAT_LIST_F64
 #undef X
 };
@@ -234,7 +232,7 @@ struct PerDevice {
     SceneStorage<double> f64;
     cudaStream_t stream = nullptr;  // owned; used by the host-buffer entry points
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, done = nullptr;
-    DevBuf control, jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order, wavefront;
+    DevBuf control, jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order;
     std::vector<int> chunk_first;          // first position in the tile order of every chunk (+ end)
     cudaStream_t copy_stream = nullptr;    // assembly / D2H of finished bands while later bands render (highest priority)
     std::vector<cudaEvent_t> band_events;
@@ -257,7 +255,7 @@ struct PerDevice {
             if (stream) cudaStreamSynchronize(stream);
             if (copy_stream) cudaStreamSynchronize(copy_stream);
             f32.release(); f64.release();
-            for (DevBuf* b : {&control, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order, &wavefront}) b->release();
+            for (DevBuf* b : {&control, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order}) b->release();
             for (DevBuf& b : peer_tiles) b.release();
             copier.release();
             if (ev0) cudaEventDestroy(ev0);
@@ -715,8 +713,7 @@ int launchFrame(ftb_scene* sc, PerDevice* pd, const ftb_camera* cam, const ftb_r
             }
             pd->order_key.swap(key);
         }
-        static const bool noOrder = std::getenv("FTB_NO_TILE_ORDER") != nullptr;  // A/B switch for measurements
-        F.tile_order = (pd->order_valid && (!noOrder || n_chunks > 1)) ? static_cast<const int*>(pd->order.p) : nullptr;
+        F.tile_order = pd->order_valid ? static_cast<const int*>(pd->order.p) : nullptr;
     }
     const int* orderBase = F.tile_order;
     Control* ctl = static_cast<Control*>(pd->control.p);
@@ -746,21 +743,6 @@ int launchFrame(ftb_scene* sc, PerDevice* pd, const ftb_camera* cam, const ftb_r
             F.bw_log = bw == 8 ? 3 : (bw == 4 ? 2 : (bw == 2 ? 1 : 0));
             F.bh_log = bh == 4 ? 2 : (bh == 2 ? 1 : 0);
             F.n_blocks = ntile * (FTB_TILE_PIXELS / ppb);
-            // A/B arm (FTB_WAVEFRONT=1): the same frame through the wavefront kernels of wavefront.cuh, where the variant has them
-            static const bool wantWavefront = std::getenv("FTB_WAVEFRONT") != nullptr;
-            if (wantWavefront && !wantStats) {
-                int rph = 0;
-                for (const ftb_light& l : sc->lights) rph += l.kind == FTB_LIGHT_SOFT_DIRECTIONAL ? std::max(l.samples, 0) : 1;
-                rph = std::max(rph, 1);
-                const size_t perPath = 4 * sizeof(typename V4<R>::type) + 3 * sizeof(int) + 3 * sizeof(R) + (size_t)rph * (2 * sizeof(typename V4<R>::type) + 2 * sizeof(int));
-                const size_t want = std::min<size_t>((size_t)ntile * FTB_TILE_PIXELS * (size_t)g.spp * perPath + 65536, (size_t)8 << 30);
-                CK(pd->wavefront.reserve(want));
-                F.s_base = 0; F.s_count = g.spp; F.run = 1; F.rpp_magic = 0;
-                cudaError_t we = var->launch_wavefront(st.view, F, ntile, rph, sc->L.has_reflection, pd->sm_count, pd->wavefront.p, pd->wavefront.cap, stream, &launches);
-                if (we == cudaSuccess) { if (chunkDone) { int rc = (*chunkDone)(chunk); if (rc != FTB_OK) return rc; } continue; }
-                if (we != cudaErrorNotSupported) return cudaFail(we, "wavefront launch");
-                (void)cudaGetLastError();  // this variant has no wavefront arm: the megakernel below
-            }
             for (int s_base = 0; s_base < g.spp; s_base += var->unit_cap) {
                 F.s_base = s_base;
                 F.s_count = std::min(var->unit_cap, g.spp - s_base);
@@ -769,8 +751,7 @@ int launchFrame(ftb_scene* sc, PerDevice* pd, const ftb_camera* cam, const ftb_r
                 // Large meshes deal single samples: a traversal's cost varies so much between neighbouring samples that a lane
                 // stuck with a run of them holds its warp back (measured -11..-14 % on the 355 k mesh; +3 % on the 960-triangle
                 // one and +7 % on moon the other way).
-                static const int runEnv = [] { const char* e = std::getenv("FTB_RUN_MAX"); int v = e ? std::atoi(e) : 0; return v > 8 ? 8 : v; }();  // A/B switch
-                const int runMax = runEnv > 0 ? runEnv : (largeMesh(sc->L) ? 1 : 8);
+                const int runMax = largeMesh(sc->L) ? 1 : 8;
                 int run = 1;
                 while (run < runMax && F.s_count % (run * 2) == 0 && F.s_count / (run * 2) >= 8) run *= 2;
                 F.run = run;
@@ -902,17 +883,14 @@ int ftb_scene_create(const ftb_scene_desc* desc, ftb_scene** out)
     CK(cudaGetDevice(&dev));
     if (sc->L.has_mesh) {
         // BspMesh.fs:30-65 builds the reference's tree; the device's own index over the same triangles is built here: on the
-        // GPU for large meshes (bvh_build.cu), on the host for small ones (and as fallback / A/B arm: FTB_HOST_BVH=1)
-        static const bool hostBvh = std::getenv("FTB_HOST_BVH") != nullptr;
-        static const bool deviceBvh = std::getenv("FTB_DEVICE_BVH") != nullptr;  // A/B: the device build also for small meshes
-        static const int radiusEnv = [] { const char* e = std::getenv("FTB_PLOC_RADIUS"); return e ? std::atoi(e) : 0; }();
+        // GPU for large meshes (bvh_build.cu), on the host for small ones and as the fallback
         std::vector<std::vector<int32_t>> order;
         ftb::enumerateMeshes(*desc, sc->L, order);
         size_t meshTriangles = 0;
         for (const auto& o : order) meshTriangles += o.size();
         bool done = false;
-        if (!hostBvh && (deviceBvh || meshTriangles >= kLargeMesh)) {
-            const int radii[3] = {radiusEnv > 0 ? radiusEnv : 16, 8, 4};
+        if (meshTriangles >= kLargeMesh) {
+            const int radii[3] = {16, 8, 4};
             for (int k = 0; k < 3 && !done; ++k) {
                 std::string why;
                 done = ftb::buildMeshIndexDevice(desc->triangles, desc->n_triangles, order, ftb::kBspStack, radii[k], sc->L, sc->bvh_stats, why);
@@ -1092,9 +1070,8 @@ int ftb_render(ftb_scene* scene, const ftb_camera* camera, const ftb_render_para
     // The frame is rendered in bands of tile rows, on every device; a finished band is assembled and sent to the host while
     // the next bands render, so only the last, smallest band's copy is exposed.  Four bands also for small downloads: a 1080p
     // RGBA8 frame (8 MB) measured 1.44 ms with four bands against 1.71 ms in one piece (hollow-sphere, 1.17 ms device-resident).
-    static const int bandsEnv = [] { const char* e = std::getenv("FTB_BANDS"); return e ? std::atoi(e) : 0; }();  // A/B switch for measurements
     const bool bandable = !dbg && !stats && !full.corner && (long long)p.width * p.height >= 262144 && full.tiles_y >= 8;
-    const int kBands = bandable ? (bandsEnv > 0 ? std::min(bandsEnv, 4) : 4) : 1;
+    const int kBands = bandable ? 4 : 1;
     const int primary = devs[0];
 
     struct Shard { PerDevice* pd; FrameGeom g; ftb_render_params ps; void* target; bool direct; };
@@ -1142,8 +1119,6 @@ int ftb_render(ftb_scene* scene, const ftb_camera* camera, const ftb_render_para
                 if (pe == cudaSuccess || pe == cudaErrorPeerAccessAlreadyEnabled) S.direct = true;
                 (void)cudaGetLastError();
             }
-            static const bool noP2P = std::getenv("FTB_NO_P2P") != nullptr;  // A/B switch
-            if (noP2P) S.direct = false;
             if (S.direct) S.target = p0->peer_tiles[(size_t)k].p;
             bufs[(size_t)k] = p0->peer_tiles[(size_t)k].p;
         } else bufs[0] = pd->tiles.p;

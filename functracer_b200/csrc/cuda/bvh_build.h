@@ -7,7 +7,7 @@
 // sorted order, nearest = smallest surface area of the joint box), which gives trees close to a top-down SAH build in a
 // few dozen small launches.  Subtrees of <= 4 triangles become the leaves.  The host builder (lower.cpp buildMeshIndex,
 // binned SAH) stays: for small meshes, where it takes 0.2-3 ms against the device build's 2-10 ms of fixed cost and gives
-// 3-9 % faster walks; as the fallback (tree deeper than the traversal stack); and as the A/B arm (FTB_HOST_BVH=1).
+// 3-9 % faster walks; and as the fallback (tree deeper than the traversal stack).
 // Measured on the 355 k-triangle mesh: index in 4.9 ms of device time (host: 135 ms), frames 8 % slower than on the host's tree.
 #pragma once
 

@@ -178,9 +178,6 @@ struct Variant {
     int unit_cap;    // UnitCap<R, feat>: samples per pixel one launch covers
     bool has_stats;  // the counting kernel is only compiled into the FT_ALL variants
     cudaError_t (*launch)(const DevScene<R>& s, const DevFrame<R>& f, bool stats, int sm_count, cudaStream_t stream, int* launches);
-    // the wavefront formulation of the same frame (wavefront.cuh), compiled into the variants of the A/B (else null)
-    cudaError_t (*launch_wavefront)(const DevScene<R>& s, const DevFrame<R>& f, int n_tiles, int rays_per_hit, bool reflective, int sm_count, void* scratch, size_t scratch_bytes,
-                                    cudaStream_t stream, int* launches);
 };
 
 }  // namespace ftb

@@ -193,7 +193,6 @@ struct Lowerer {
         if (it != surfaceIndex.end()) return it->second;
         L.surfaces.push_back(s);
         if (s.roughness != 0.0) L.has_rough = true;
-        if (s.reflectance > 0.0) L.has_reflection = true;
         return surfaceIndex[key] = (int)L.surfaces.size() - 1;
     }
 

@@ -138,7 +138,7 @@ struct Lowered {
     int32_t max_csg_lists = 0;  // deepest list stack any program needs
     int32_t max_bsp_depth = 0;
     bool has_csg = false, has_mesh = false, has_texture = false, has_image = false;
-    bool has_soft_light = false, has_rough = false, has_reflection = false;
+    bool has_soft_light = false, has_rough = false;
     // Kernel features this scene needs, as device_scene.h `Feature` bits (cube 1, round 2, mesh 4, csg 8,
     // texture 16, Oren-Nayar 32, rng 64, general CSG 128, top-level planar leaf 256, bound table 512, shared-copy pairs 1024; api.cu adds 2048 for a large mesh);
     // camera depth of field adds rng at render time.

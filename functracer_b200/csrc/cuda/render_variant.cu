@@ -2,7 +2,6 @@
 //   -DFTB_FEAT=0x.. [-DFTB_F64]     FP64 variants are built with --fmad=false so that a*b+c rounds
 //                                   twice like the reference's JIT and the oracle.
 #include "render.cuh"
-#include "wavefront.cuh"
 
 #ifndef FTB_FEAT
 #error "FTB_FEAT must be defined"
@@ -22,23 +21,5 @@ typedef float VR;
 cudaError_t FTB_VNAME(const DevScene<VR>& s, const DevFrame<VR>& f, bool stats, int sm_count, cudaStream_t stream, int* launches)
 {
     return launch_render_impl<VR, (unsigned)(FTB_FEAT), (FTB_FEAT) == FT_ALL>(s, f, stats, sm_count, stream, launches);
-}
-
-// The wavefront arm is compiled for the variants of the A/B it was built for: the house family (0x74b), hollow-sphere (0x209),
-// moon (0x030); the other variants return "not available" and the frame takes the megakernel.
-#ifdef FTB_F64
-#define FTB_WNAME FTB_CAT(launch_wf_f64_, FTB_FEAT)
-#else
-#define FTB_WNAME FTB_CAT(launch_wf_f32_, FTB_FEAT)
-#endif
-cudaError_t FTB_WNAME(const DevScene<VR>& s, const DevFrame<VR>& f, int n_tiles, int rays_per_hit, bool reflective, int sm_count, void* scratch, size_t scratch_bytes,
-                      cudaStream_t stream, int* launches)
-{
-#if !defined(FTB_F64) && (FTB_FEAT == 0x74b || FTB_FEAT == 0x209 || FTB_FEAT == 0x030)
-    return launch_wavefront_impl<VR, (unsigned)(FTB_FEAT)>(s, f, n_tiles, rays_per_hit, reflective, sm_count, scratch, scratch_bytes, stream, launches);
-#else
-    (void)s; (void)f; (void)n_tiles; (void)rays_per_hit; (void)reflective; (void)sm_count; (void)scratch; (void)scratch_bytes; (void)stream; (void)launches;
-    return cudaErrorNotSupported;
-#endif
 }
 }  // namespace ftb

@@ -3,7 +3,7 @@
 #   tools/ab_build.sh NAME ["extra nvcc flags for the FP32 kernels"] [GIT_REV]
 # With GIT_REV the library is built from that commit's sources, else from the working tree.  The copy is selected
 # at run time with FTB_LIB=$PWD/ab/libftb_NAME.so (functracer_b200/api.py); see tools/ab_bench.sh.
-# AB_MAKE_ARGS in the environment is appended to the make command line (through eval, e.g. AB_MAKE_ARGS="EXTRA=-DFTB_PAIR_GROUPS=1 'F32_FEATS=0x3ff 0x34b'").
+# AB_MAKE_ARGS in the environment is appended to the make command line (through eval, e.g. AB_MAKE_ARGS="EXTRA=-DFTB_UNIT_CAP=128 'F32_FEATS=0xfff 0x74b'").
 # Prints the SASS size and the spill summary of every FP32 variant, the numbers to look at before spending GPU time.
 set -e
 name=$1; flags=$2; rev=$3

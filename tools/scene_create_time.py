@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Times ftb_scene_create for the mesh workloads (FTB_VERBOSE=1 prints the phases to stderr): device-built index vs FTB_HOST_BVH=1."""
+"""Times ftb_scene_create for the mesh workloads (FTB_VERBOSE=1 prints the phases to stderr)."""
 import os
 import sys
 import time
