@@ -11,8 +11,6 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <deque>
-#include <functional>
 #include <map>
 #include <memory>
 #include <string>
@@ -183,6 +181,34 @@ struct Control {  // device control block of one launch
     unsigned long long stats[ST_COUNT];
 };
 
+// The per-device control block and everything that resets, wires or reads it.  The queue counter is reset before every
+// launch, the counters only when they are asked for; the overflow flag stays up until somebody reads it (finishStats /
+// ftb_check_overflow), so that the banded and the device paths cannot lose it.
+struct ControlBlock {
+    DevBuf buf;
+    bool zeroed = false;  // zeroed once by a frame launch (ftb_shade_rays zeroes the whole block itself)
+    Control* ctl() const { return static_cast<Control*>(buf.p); }
+    bool used() const { return buf.p != nullptr; }  // something has been launched on this device
+    cudaError_t reserve() { return buf.reserve(sizeof(Control)); }
+    // a frame launch: the block is zeroed the first time, the counters whenever they are counted
+    cudaError_t prepare(bool counting, cudaStream_t s)
+    {
+        cudaError_t e = zeroed ? cudaSuccess : cudaMemsetAsync(buf.p, 0, sizeof(Control), s);
+        zeroed = e == cudaSuccess;
+        return e != cudaSuccess || !counting ? e : cudaMemsetAsync(ctl()->stats, 0, sizeof(Control::stats), s);
+    }
+    cudaError_t resetAll(cudaStream_t s) { cudaError_t e = reserve(); return e != cudaSuccess ? e : cudaMemsetAsync(buf.p, 0, sizeof(Control), s); }
+    cudaError_t resetQueue(cudaStream_t s) { return cudaMemsetAsync(&ctl()->tile_counter, 0, sizeof(unsigned int), s); }
+    template <typename R> void wire(DevFrame<R>& F) const { F.tile_counter = &ctl()->tile_counter; F.overflow = &ctl()->overflow; F.stats = ctl()->stats; }
+    // D2H copy into h, synchronising `s`; a raised overflow flag is cleared on the device
+    cudaError_t read(Control& h, cudaStream_t s)
+    {
+        cudaError_t e = cudaMemcpyAsync(&h, buf.p, sizeof(h), cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        return e != cudaSuccess || !h.overflow ? e : cudaMemsetAsync(&ctl()->overflow, 0, sizeof(unsigned int), s);
+    }
+};
+
 template <typename R>
 struct SceneStorage {
     DevScene<R> view;
@@ -193,7 +219,6 @@ struct SceneStorage {
 
 struct PerDevice;
 template <typename R> SceneStorage<R>& storageOf(PerDevice* pd);
-typedef std::function<int(int)> ChunkDone;  // called after the launches of chunk k have been queued
 
 // Device -> host copies of finished bands.  The destination is whatever the caller owns: usually ordinary pageable memory
 // (a GC-pinned .NET array, a std::vector, numpy), sometimes CUDA page-locked memory.  A cudaMemcpyAsync into pageable
@@ -222,7 +247,6 @@ struct HostCopier {
         used.clear();
         return e;
     }
-    void release() { used.clear(); }
 };
 
 struct PerDevice {
@@ -232,14 +256,14 @@ struct PerDevice {
     SceneStorage<double> f64;
     cudaStream_t stream = nullptr;  // owned; used by the host-buffer entry points
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, done = nullptr;
-    DevBuf control, jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order;
+    ControlBlock control;
+    DevBuf jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order;
     std::vector<int> chunk_first;          // first position in the tile order of every chunk (+ end)
     cudaStream_t copy_stream = nullptr;    // assembly / D2H of finished bands while later bands render (highest priority)
     std::vector<cudaEvent_t> band_events;
     HostCopier copier;
     std::vector<unsigned char> order_key;  // what the cached tile order was computed for
     bool order_valid = false;
-    bool control_ready = false;      // the control block has been zeroed once
     std::vector<DevBuf> peer_tiles;  // on the gather device: one per remote shard
 
     PerDevice() = default;
@@ -255,9 +279,8 @@ struct PerDevice {
             if (stream) cudaStreamSynchronize(stream);
             if (copy_stream) cudaStreamSynchronize(copy_stream);
             f32.release(); f64.release();
-            for (DevBuf* b : {&control, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order}) b->release();
+            for (DevBuf* b : {&control.buf, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order}) b->release();
             for (DevBuf& b : peer_tiles) b.release();
-            copier.release();
             if (ev0) cudaEventDestroy(ev0);
             if (ev1) cudaEventDestroy(ev1);
             if (done) cudaEventDestroy(done);
@@ -278,9 +301,6 @@ template <> SceneStorage<double>& storageOf<double>(PerDevice* pd) { return pd->
 struct ftb_scene {
     ftb::Lowered L;
     // host copies of the tables the upload needs
-    std::vector<ftb_bsp_node> bsp_nodes;
-    std::vector<ftb_bsp_leaf> bsp_leaves;
-    std::vector<ftb_mesh> meshes;
     std::vector<double> triangles;
     std::vector<ftb_light> lights;
     struct Img { int w, h; std::vector<uint8_t> rgb; };
@@ -521,27 +541,35 @@ inline V3 normalise(V3 v)
     return {s * v.x, s * v.y, s * v.z};
 }
 
-// ImagePlane.create / fromCamera (Image.fs:48-53, 67-81), evaluated in double on the host; the
-// FP32 kernels receive the narrowed results.
+// ImagePlane.create / fromCamera (Image.fs:48-53, 67-81), evaluated in double on the host: the camera's basis, the image
+// plane's size, the pixel pitch and the centre of the top-left pixel.  resH = frame width, resV = frame height.
+struct CameraBasis { V3 o, k, i, j; double width, height, pw, ph, tlx, tly; };
+CameraBasis cameraBasis(const ftb_camera& c, int resH, int resV)
+{
+    const V3 o = {c.o[0], c.o[1], c.o[2]}, la = {c.look_at[0], c.look_at[1], c.look_at[2]}, up = {c.up[0], c.up[1], c.up[2]};
+    const V3 k = normalise(sub(la, o));
+    const V3 i = normalise(cross(up, k));
+    const V3 j = cross(k, i);
+    const double height = std::tan(c.fov_y_rad / 2.0) * 2.0;
+    const double width = height * c.aspect_ratio;
+    const double ph = height / (double)(resH - 1);  // the reference's swapped axes (Image.fs:71-72)
+    const double pw = width / (double)(resV - 1);
+    return {o, k, i, j, width, height, pw, ph, -width / 2.0 + pw / 2.0, height / 2.0 - ph / 2.0};
+}
+
+// the FP32 kernels receive the narrowed results
 template <typename R>
 void fillCamera(DevFrame<R>& F, const ftb_camera& c, int resH, int resV)
 {
-    V3 o = {c.o[0], c.o[1], c.o[2]}, la = {c.look_at[0], c.look_at[1], c.look_at[2]}, up = {c.up[0], c.up[1], c.up[2]};
-    V3 k = normalise(sub(la, o));
-    V3 i = normalise(cross(up, k));
-    V3 j = cross(k, i);
-    double height = std::tan(c.fov_y_rad / 2.0) * 2.0;
-    double width = height * c.aspect_ratio;
-    double pixelHeight = height / (double)(resH - 1);  // the reference's swapped axes (Image.fs:71-72)
-    double pixelWidth = width / (double)(resV - 1);
+    const CameraBasis b = cameraBasis(c, resH, resV);
+    const V3 &o = b.o, &k = b.k, &i = b.i, &j = b.j;
     F.cam_o[0] = (R)o.x; F.cam_o[1] = (R)o.y; F.cam_o[2] = (R)o.z;
     F.primary_slack = (R)(2e-4 * std::sqrt(o.x * o.x + o.y * o.y + o.z * o.z));
     F.cam_k[0] = (R)k.x; F.cam_k[1] = (R)k.y; F.cam_k[2] = (R)k.z;
     F.cam_i[0] = (R)i.x; F.cam_i[1] = (R)i.y; F.cam_i[2] = (R)i.z;
     F.cam_j[0] = (R)j.x; F.cam_j[1] = (R)j.y; F.cam_j[2] = (R)j.z;
-    F.pw = (R)pixelWidth; F.ph = (R)pixelHeight;
-    F.tlx = (R)(-width / 2.0 + pixelWidth / 2.0);
-    F.tly = (R)(height / 2.0 - pixelHeight / 2.0);
+    F.pw = (R)b.pw; F.ph = (R)b.ph;
+    F.tlx = (R)b.tlx; F.tly = (R)b.tly;
     F.has_focus = c.has_focus;
     F.focal = (R)c.focal_length;
     F.tan_half_aperture = (R)std::tan(c.aperture_rad / 2.0);
@@ -583,6 +611,8 @@ inline int bandOfRow(int row, int n, int tiles_y)
     while (k + 1 < n && row >= bandFirstRow(k + 1, n, tiles_y)) ++k;
     return k;
 }
+// band k of n = pixel rows [bandPixelRow(k), bandPixelRow(k + 1))
+inline int bandPixelRow(int k, int n, int tiles_y, int height) { return std::min(height, bandFirstRow(k, n, tiles_y) * FTB_TILE_H); }
 
 // Longest-processing-time-first tile order.  The persistent kernel hands tiles out from an atomic queue; a lane
 // keeps its pixel for all samples and all bounce generations, so the last tiles handed out set the tail.  A
@@ -594,13 +624,7 @@ bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render
                       std::vector<int>& chunk_first)
 {
     const double kPiHalf = 1.5707963267948966;
-    V3 o = {c.o[0], c.o[1], c.o[2]}, la = {c.look_at[0], c.look_at[1], c.look_at[2]}, up = {c.up[0], c.up[1], c.up[2]};
-    V3 k = normalise(sub(la, o));
-    V3 i = normalise(cross(up, k));
-    V3 j = cross(k, i);
-    const double height = std::tan(c.fov_y_rad / 2.0) * 2.0, width = height * c.aspect_ratio;
-    const double ph = height / (double)(p.width - 1), pw = width / (double)(p.height - 1);  // Image.fs:71-72 (swapped axes)
-    const double tlx = -width / 2.0 + pw / 2.0, tly = height / 2.0 - ph / 2.0;
+    const CameraBasis b = cameraBasis(c, p.width, p.height);
     std::vector<float> cost((size_t)g.n_tiles, 1.0f);
     bool any = false;
     auto range = [&](double a, double z, double r, double& lo, double& hi) {
@@ -630,12 +654,12 @@ bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render
         }
         w *= (1.0 + (double)sc.lights.size());                              // a shaded hit adds one shadow ray per light
         if (reflective) w *= 1.0 + (double)std::max(0, p.recursion_limit);   // and up to `limit` more generations
-        V3 v = {it.bound_c[0] - o.x, it.bound_c[1] - o.y, it.bound_c[2] - o.z};
-        const double x = v.x * i.x + v.y * i.y + v.z * i.z, y = v.x * j.x + v.y * j.y + v.z * j.z, z = v.x * k.x + v.y * k.y + v.z * k.z;
+        V3 v = {it.bound_c[0] - b.o.x, it.bound_c[1] - b.o.y, it.bound_c[2] - b.o.z};
+        const double x = v.x * b.i.x + v.y * b.i.y + v.z * b.i.z, y = v.x * b.j.x + v.y * b.j.y + v.z * b.j.z, z = v.x * b.k.x + v.y * b.k.y + v.z * b.k.z;
         double xl, xh, yl, yh;
         if (!range(x, z, it.bound_r, xl, xh) || !range(y, z, it.bound_r, yl, yh)) continue;
         // image-plane coordinates -> sample-grid pixels (rayThroughPixel, Image.fs:83-89), one pixel of slack for jitter
-        const double px0 = (xl - tlx) / pw - 1.5, px1 = (xh - tlx) / pw + 1.5, py0 = (tly - yh) / ph - 1.5, py1 = (tly - yl) / ph + 1.5;
+        const double px0 = (xl - b.tlx) / b.pw - 1.5, px1 = (xh - b.tlx) / b.pw + 1.5, py0 = (b.tly - yh) / b.ph - 1.5, py1 = (b.tly - yl) / b.ph + 1.5;
         if (px1 < 0 || py1 < 0 || px0 >= g.gw || py0 >= g.gh) continue;
         const int tx0 = (int)std::max(0.0, std::floor(px0 / FTB_TILE_W)), tx1 = (int)std::min((double)g.tiles_x - 1, std::floor(px1 / FTB_TILE_W));
         const int ty0 = (int)std::max(0.0, std::floor(py0 / FTB_TILE_H)), ty1 = (int)std::min((double)g.tiles_y - 1, std::floor(py1 / FTB_TILE_H));
@@ -660,45 +684,53 @@ bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render
     return true;
 }
 
-// Renders one shard's tiles (mode 0) on the CURRENT device into d_tiles.  Everything is queued on
-// `stream`; nothing here synchronises unless stats are requested.
+// Runs fn(R()) with R the real type of `precision`.
+template <typename Fn> int byPrecision(int precision, Fn&& fn) { return precision == FTB_PRECISION_FP64_VERIFY ? fn(double()) : fn(float()); }
+
+// The kernel launches of one frame on the CURRENT device.  begin() does what both modes share; a mode-0 frame (one shard of a
+// camera grid) is then set up by prepareFrame, launched one chunk (band of tile rows) at a time by launchChunk and closed by
+// finishFrame.  Everything is queued on the given stream; nothing here synchronises unless the tile order changes.
 template <typename R>
-int launchFrame(ftb_scene* sc, PerDevice* pd, const ftb_camera* cam, const ftb_render_params* p, const FrameGeom& g, void* d_tiles,
-                const ftb_debug_out* d_dbg, ftb_stats* stats, cudaStream_t stream, bool timeKernel, int n_chunks, const ChunkDone* chunkDone, int only_chunk)
-{
-    SceneStorage<R>& st = storageOf<R>(pd);
-    if (!st.ready) { int rc = uploadScene<R>(*sc, st); if (rc != FTB_OK) return rc; }
-    CK(pd->control.reserve(sizeof(Control)));
-    if (!pd->control_ready) { CK(cudaMemset(pd->control.p, 0, sizeof(Control))); pd->control_ready = true; }
-    // The queue counter is reset before every launch, the counters only when they are asked for; the overflow flag stays
-    // up until somebody reads it (finishStats / ftb_check_overflow), so that the banded and the device paths cannot lose it.
-    if (stats && p->collect_stats) CK(cudaMemsetAsync(static_cast<Control*>(pd->control.p)->stats, 0, sizeof(static_cast<Control*>(pd->control.p)->stats), stream));
+struct Launch {
+    PerDevice* pd = nullptr;
+    const DevScene<R>* scene = nullptr;  // this device's copy
+    const Variant<R>* var = nullptr;
     DevFrame<R> F;
-    std::memset(&F, 0, sizeof(F));
-    F.mode = 0;
-    F.gw = g.gw; F.gh = g.gh; F.spp = g.spp; F.tiles_x = g.tiles_x;
-    // floor(2^32 / tiles_x) + 1 does not fit 32 bits for tiles_x == 1 (frames <= 16 sample columns wide): those divide
-    F.tiles_x_magic = (g.tiles_x > 1 && (unsigned long long)g.n_tiles * (unsigned long long)g.tiles_x < (1ull << 32)) ? (unsigned)((1ull << 32) / (unsigned)g.tiles_x) + 1u : 0u;
-    F.n_local_tiles = g.n_local_tiles; F.shard_index = g.shard_index; F.shard_count = g.shard_count;
-    fillCamera<R>(F, *cam, p->width, p->height);
-    if (!g.corner) {
-        std::vector<R> j(2 * (size_t)g.spp);
-        for (size_t k = 0; k < j.size(); ++k) j[k] = (R)p->jitter_xy[k];
+    bool counting = false;  // the counting kernel: stats asked for with collect_stats
+    int launches = 0;
+    // The scene on this device (uploaded on first use), the DevFrame fields of both modes and the variant that covers `need`.
+    int begin(ftb_scene* sc, PerDevice* pd, const ftb_render_params* p, unsigned need, bool counting, void* out, const ftb_debug_out* dbg)
+    {
+        SceneStorage<R>& st = storageOf<R>(pd);
+        if (!st.ready) { int rc = uploadScene<R>(*sc, st); if (rc != FTB_OK) return rc; }
+        CK(pd->control.reserve());
+        this->pd = pd; this->counting = counting; scene = &st.view;
+        std::memset(&F, 0, sizeof(F));
+        F.recursion_limit = p->recursion_limit; F.seed = p->seed; F.out = static_cast<R*>(out);
+        if (dbg) { F.dbg_prim = dbg->prim_id; F.dbg_sub = dbg->sub_id; F.dbg_t = dbg->t; }
+        pd->control.wire(F);
+        var = pickVariant<R>(need, counting);
+        return var ? FTB_OK : fail(FTB_ERR_UNSUPPORTED, "no kernel variant covers this scene's feature mask");
+    }
+    cudaError_t launchKernel(cudaStream_t s) { return var->launch(*scene, F, counting, pd->sm_count, s, &launches); }
+    int prepareFrame(ftb_scene* sc, PerDevice* pd, const ftb_camera* cam, const ftb_render_params* p, const FrameGeom& g, void* d_tiles,
+                     const ftb_debug_out* d_dbg, ftb_stats* stats, cudaStream_t stream, int n_chunks)
+    {
+        int rc = begin(sc, pd, p, sc->L.features | (cam->has_focus ? (unsigned)FT_RNG : 0u), stats && p->collect_stats, d_tiles, d_dbg);
+        if (rc != FTB_OK) return rc;
+        CK(pd->control.prepare(counting, stream));
+        F.mode = 0; F.gw = g.gw; F.gh = g.gh; F.spp = g.spp; F.tiles_x = g.tiles_x;
+        // floor(2^32 / tiles_x) + 1 does not fit 32 bits for tiles_x == 1 (frames <= 16 sample columns wide): those divide
+        F.tiles_x_magic = (g.tiles_x > 1 && (unsigned long long)g.n_tiles * (unsigned long long)g.tiles_x < (1ull << 32)) ? (unsigned)((1ull << 32) / (unsigned)g.tiles_x) + 1u : 0u;
+        F.n_local_tiles = g.n_local_tiles; F.shard_index = g.shard_index; F.shard_count = g.shard_count;
+        fillCamera<R>(F, *cam, p->width, p->height);
+        // CornerSampling.generateRays (Image.fs:128-132): every corner ray uses the offset (-0.5, +0.5)
+        std::vector<R> j = {R(-0.5), R(0.5)};
+        if (!g.corner) j.assign(p->jitter_xy, p->jitter_xy + 2 * (size_t)g.spp);
         CK(pd->jitter.reserve(j.size() * sizeof(R)));
         CK(cudaMemcpyAsync(pd->jitter.p, j.data(), j.size() * sizeof(R), cudaMemcpyHostToDevice, stream));  // pageable source: staged before return
         F.jitter = static_cast<const R*>(pd->jitter.p);
-    } else {
-        // CornerSampling.generateRays (Image.fs:128-132): every corner ray uses the offset (-0.5, +0.5)
-        const R j[2] = {R(-0.5), R(0.5)};
-        CK(pd->jitter.reserve(sizeof(j)));
-        CK(cudaMemcpyAsync(pd->jitter.p, j, sizeof(j), cudaMemcpyHostToDevice, stream));
-        F.jitter = static_cast<const R*>(pd->jitter.p);
-    }
-    F.recursion_limit = p->recursion_limit;
-    F.seed = p->seed;
-    F.out = static_cast<R*>(d_tiles);
-    if (d_dbg) { F.dbg_prim = d_dbg->prim_id; F.dbg_sub = d_dbg->sub_id; F.dbg_t = d_dbg->t; }
-    {  // tile order: cached per (camera, frame geometry, recursion limit); recomputed + uploaded only when they change
+        // tile order: cached per (camera, frame geometry, recursion limit); recomputed + uploaded only when they change
         std::vector<unsigned char> key(sizeof(ftb_camera) + 7 * sizeof(int));
         std::memcpy(key.data(), cam, sizeof(ftb_camera));
         const int kk[7] = {p->width, p->height, p->sampling, g.shard_index, g.shard_count, p->recursion_limit, n_chunks};
@@ -713,102 +745,83 @@ int launchFrame(ftb_scene* sc, PerDevice* pd, const ftb_camera* cam, const ftb_r
             }
             pd->order_key.swap(key);
         }
-        F.tile_order = pd->order_valid ? static_cast<const int*>(pd->order.p) : nullptr;
+        if (stats) CK(cudaEventRecord(pd->ev0, stream));
+        return FTB_OK;
     }
-    const int* orderBase = F.tile_order;
-    Control* ctl = static_cast<Control*>(pd->control.p);
-    F.tile_counter = &ctl->tile_counter; F.overflow = &ctl->overflow; F.stats = ctl->stats;
-    const bool wantStats = stats && p->collect_stats;
-    if (timeKernel) CK(cudaEventRecord(pd->ev0, stream));
-    int launches = 0;
-    const Variant<R>* var = pickVariant<R>(sc->L.features | (cam->has_focus ? (unsigned)FT_RNG : 0u), wantStats);
-    if (!var) return fail(FTB_ERR_UNSUPPORTED, "no kernel variant covers this scene's feature mask");
-    // one launch covers at most UnitCap samples per pixel; more samples = more passes over the same tiles, each
-    // continuing the left fold of the previous one (so the blend order is still Array.average's)
-    // Work-queue granularity.  A lane takes runs of samples, a warp takes blocks of pixels from the atomic queue.  The
-    // block is the indivisible quantum of the tail, so it shrinks (32 = 8x4 ... 1 pixel) until there are >= 24 blocks
-    // per resident warp, but never below one warp-round of samples per block (and big frames keep big blocks, which
-    // also bounds the number of atomics on the queue counter).
-    for (int chunk = 0; chunk < n_chunks; ++chunk) {
-        if (only_chunk >= 0 && chunk != only_chunk) continue;
-        const int first = n_chunks > 1 ? pd->chunk_first[(size_t)chunk] : 0;
-        const int ntile = n_chunks > 1 ? pd->chunk_first[(size_t)chunk + 1] - first : g.n_local_tiles;
-        if (ntile > 0) {
-            F.tile_order = orderBase ? orderBase + first : nullptr;
-            const long long warps = (long long)pd->sm_count * 5 * (kBlockThreads / 32);
-            const long long pixels = (long long)ntile * FTB_TILE_PIXELS;
-            int ppb = 32;
-            while (ppb > 1 && pixels / ppb < 24 * warps && (long long)(ppb / 2) * g.spp >= 32) ppb /= 2;
-            int bw = ppb >= 8 ? 8 : ppb, bh = ppb / bw;
-            F.bw_log = bw == 8 ? 3 : (bw == 4 ? 2 : (bw == 2 ? 1 : 0));
-            F.bh_log = bh == 4 ? 2 : (bh == 2 ? 1 : 0);
-            F.n_blocks = ntile * (FTB_TILE_PIXELS / ppb);
-            for (int s_base = 0; s_base < g.spp; s_base += var->unit_cap) {
-                F.s_base = s_base;
-                F.s_count = std::min(var->unit_cap, g.spp - s_base);
-                // run length: cheap samples amortise the dealing over up to 8 consecutive samples of a pixel, as long as
-                // every pixel still splits into >= 8 runs (the chain a lane can be stuck with stays 1/8 of a pixel)
-                // Large meshes deal single samples: a traversal's cost varies so much between neighbouring samples that a lane
-                // stuck with a run of them holds its warp back (measured -11..-14 % on the 355 k mesh; +3 % on the 960-triangle
-                // one and +7 % on moon the other way).
-                const int runMax = largeMesh(sc->L) ? 1 : 8;
-                int run = 1;
-                while (run < runMax && F.s_count % (run * 2) == 0 && F.s_count / (run * 2) >= 8) run *= 2;
-                F.run = run;
-                const unsigned rpp = (unsigned)(F.s_count / run);
-                F.rpp_magic = rpp <= 1 ? 0u : (unsigned)((1ull << 32) / rpp) + 1u;
-                CK(cudaMemsetAsync(&ctl->tile_counter, 0, sizeof(unsigned int), stream));
-                CK(var->launch(st.view, F, wantStats, pd->sm_count, stream, &launches));
-            }
+    // One launch covers at most UnitCap samples per pixel; more samples = more passes over the same tiles, each continuing the
+    // left fold of the previous one (so the blend order is still Array.average's).
+    // Work-queue granularity.  A lane takes runs of samples, a warp takes blocks of pixels from the atomic queue.  The block is
+    // the indivisible quantum of the tail, so it shrinks (32 = 8x4 ... 1 pixel) until there are >= 24 blocks per resident
+    // warp, but never below one warp-round of samples per block (and big frames keep big blocks, which also bounds the number
+    // of atomics on the queue counter).
+    int launchChunk(int chunk, cudaStream_t stream)
+    {
+        const int first = pd->chunk_first[(size_t)chunk], ntile = pd->chunk_first[(size_t)chunk + 1] - first;
+        if (ntile <= 0) return FTB_OK;
+        F.tile_order = pd->order_valid ? static_cast<const int*>(pd->order.p) + first : nullptr;
+        const long long warps = (long long)pd->sm_count * 5 * (kBlockThreads / 32);
+        const long long pixels = (long long)ntile * FTB_TILE_PIXELS;
+        int ppb = 32;
+        while (ppb > 1 && pixels / ppb < 24 * warps && (long long)(ppb / 2) * F.spp >= 32) ppb /= 2;
+        int bw = ppb >= 8 ? 8 : ppb, bh = ppb / bw;
+        F.bw_log = bw == 8 ? 3 : (bw == 4 ? 2 : (bw == 2 ? 1 : 0));
+        F.bh_log = bh == 4 ? 2 : (bh == 2 ? 1 : 0);
+        F.n_blocks = ntile * (FTB_TILE_PIXELS / ppb);
+        for (int s_base = 0; s_base < F.spp; s_base += var->unit_cap) {
+            F.s_base = s_base;
+            F.s_count = std::min(var->unit_cap, F.spp - s_base);
+            // run length: cheap samples amortise the dealing over up to 8 consecutive samples of a pixel, as long as
+            // every pixel still splits into >= 8 runs (the chain a lane can be stuck with stays 1/8 of a pixel)
+            // Large meshes deal single samples: a traversal's cost varies so much between neighbouring samples that a lane
+            // stuck with a run of them holds its warp back (measured -11..-14 % on the 355 k mesh; +3 % on the 960-triangle
+            // one and +7 % on moon the other way).
+            const int runMax = scene->mesh_packet ? 1 : 8;
+            int run = 1;
+            while (run < runMax && F.s_count % (run * 2) == 0 && F.s_count / (run * 2) >= 8) run *= 2;
+            F.run = run;
+            const unsigned rpp = (unsigned)(F.s_count / run);
+            F.rpp_magic = rpp <= 1 ? 0u : (unsigned)((1ull << 32) / rpp) + 1u;
+            CK(pd->control.resetQueue(stream));
+            CK(launchKernel(stream));
         }
-        if (chunkDone) { int rc = (*chunkDone)(chunk); if (rc != FTB_OK) return rc; }
+        return FTB_OK;
     }
-    if (timeKernel) CK(cudaEventRecord(pd->ev1, stream));
-    if (stats) stats->kernel_launches += launches + 1;  // + the control-block memset
-    return FTB_OK;
-}
+    int finishFrame(ftb_stats* stats, cudaStream_t stream)
+    {
+        if (stats) { CK(cudaEventRecord(pd->ev1, stream)); stats->kernel_launches += launches + 1; }  // + the control-block memset
+        return FTB_OK;
+    }
+};
 
-int launchFrameAny(ftb_scene* sc, PerDevice* pd, const ftb_camera* cam, const ftb_render_params* p, const FrameGeom& g, void* d_tiles,
-                   const ftb_debug_out* d_dbg, ftb_stats* stats, cudaStream_t stream, bool timeKernel, int n_chunks = 1, const ChunkDone* chunkDone = nullptr,
-                   int only_chunk = -1)
-{
-    if (p->precision == FTB_PRECISION_FP64_VERIFY) return launchFrame<double>(sc, pd, cam, p, g, d_tiles, d_dbg, stats, stream, timeKernel, n_chunks, chunkDone, only_chunk);
-    return launchFrame<float>(sc, pd, cam, p, g, d_tiles, d_dbg, stats, stream, timeKernel, n_chunks, chunkDone, only_chunk);
-}
+int overflowError() { return fail(FTB_ERR_HIT_OVERFLOW, "a CSG operand produced more than 32 crossings on one ray"); }
 
-// Reads the control block back (synchronises the stream) and folds it into stats.
-int finishStats(ftb_scene* sc, PerDevice* pd, ftb_stats* stats, cudaStream_t stream, bool timed, bool* overflow)
+// Reads the control block back (synchronises the stream) and, with stats, folds its counters and the kernel time into them.
+int finishStats(ftb_scene* sc, PerDevice* pd, ftb_stats* stats, cudaStream_t stream, bool* overflow)
 {
     Control h;
-    CK(cudaMemcpyAsync(&h, pd->control.p, sizeof(h), cudaMemcpyDeviceToHost, stream));
-    CK(cudaStreamSynchronize(stream));
-    if (h.overflow) {
-        *overflow = true;
-        CK(cudaMemsetAsync(&static_cast<Control*>(pd->control.p)->overflow, 0, sizeof(unsigned int), stream));
-    }
+    CK(pd->control.read(h, stream));
+    if (h.overflow) *overflow = true;
     if (stats) {
         fillStats(h, *sc, stats);
         if (h.overflow) stats->hit_overflow = 1;
-        if (timed) { float ms = 0; CK(cudaEventElapsedTime(&ms, pd->ev0, pd->ev1)); if ((double)ms > stats->kernel_ms) stats->kernel_ms = ms; }
+        float ms = 0; CK(cudaEventElapsedTime(&ms, pd->ev0, pd->ev1)); if ((double)ms > stats->kernel_ms) stats->kernel_ms = ms;
     }
     return FTB_OK;
 }
 
-int launchAssemble(const ftb_render_params* p, const FrameGeom& g, const void* const* bufs, void* d_out, cudaStream_t stream, int y0 = 0, int y1 = -1)
+int launchAssemble(const ftb_render_params* p, const FrameGeom& g, const void* const* bufs, void* d_out, cudaStream_t stream, int y0, int y1)
 {
     TilePtrs tp;
     std::memset(&tp, 0, sizeof(tp));
     for (int i = 0; i < g.shard_count; ++i) tp.p[i] = bufs[i];
-    if (y1 < 0) y1 = p->height;
     const long long n = (long long)p->width * (y1 - y0);
     if (n <= 0) return FTB_OK;
     int grid = (int)std::min<long long>((n + 255) / 256, 148 * 16);
-    if (p->precision == FTB_PRECISION_FP64_VERIFY)
-        assemble_kernel<double><<<grid, 256, 0, stream>>>(tp, g.shard_count, g.tiles_x, p->width, y0, y1, g.corner ? 1 : 0, p->out_format, d_out);
-    else
-        assemble_kernel<float><<<grid, 256, 0, stream>>>(tp, g.shard_count, g.tiles_x, p->width, y0, y1, g.corner ? 1 : 0, p->out_format, d_out);
-    CK(cudaGetLastError());
-    return FTB_OK;
+    return byPrecision(p->precision, [&](auto r) -> int {
+        assemble_kernel<decltype(r)><<<grid, 256, 0, stream>>>(tp, g.shard_count, g.tiles_x, p->width, y0, y1, g.corner ? 1 : 0, p->out_format, d_out);
+        CK(cudaGetLastError());
+        return FTB_OK;
+    });
 }
 
 inline size_t outBytes(const ftb_render_params* p)
@@ -837,6 +850,91 @@ struct DeviceRestore {
     ~DeviceRestore() { if (dev >= 0) cudaSetDevice(dev); }
 };
 
+int currentDevice(ftb_scene* sc, PerDevice** out)
+{
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device"); }
+    return getDevice(sc, dev, out);
+}
+
+// BspMesh.fs:30-65 builds the reference's tree; the device's own index over the same triangles is built here: on the GPU for
+// large meshes (bvh_build.cu), on the host for small ones and as the fallback
+int buildMeshIndex(const ftb_scene_desc& desc, ftb_scene& sc)
+{
+    std::vector<std::vector<int32_t>> order;
+    ftb::enumerateMeshes(desc, sc.L, order);
+    size_t meshTriangles = 0;
+    for (const auto& o : order) meshTriangles += o.size();
+    bool done = false;
+    if (meshTriangles >= kLargeMesh) {
+        const int radii[3] = {16, 8, 4};
+        for (int k = 0; k < 3 && !done; ++k) {
+            std::string why;
+            done = ftb::buildMeshIndexDevice(desc.triangles, desc.n_triangles, order, ftb::kBspStack, radii[k], sc.L, sc.bvh_stats, why);
+            if (!done && std::getenv("FTB_VERBOSE")) std::fprintf(stderr, "functracer_b200: device BVH build not used (%s)\n", why.c_str());
+        }
+        sc.bvh_on_device = done;
+    }
+    if (!done) {
+        const auto t0 = std::chrono::steady_clock::now();
+        ftb::buildMeshIndexHost(desc, sc.L);
+        sc.bvh_stats.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    if (sc.L.max_bvh_depth + 2 > ftb::kBspStack) return fail(FTB_ERR_UNSUPPORTED, "mesh index deeper than the 64-entry traversal stack");
+    if (largeMesh(sc.L)) sc.L.features |= (unsigned)FT_MESHPK;  // the warp-packet walk (render.cuh)
+    return FTB_OK;
+}
+
+// One device's part of an ftb_render frame; the primary device's assembly reads its tiles from `gather` (== target if direct).
+struct Shard { PerDevice* pd; FrameGeom g; ftb_render_params ps; ftb_debug_out dbg; void* target; void* gather; bool direct; };
+
+// Device k's shard: geometry, tile buffer, band events, debug planes.  Shards of the other devices: the render kernel's fold
+// stores finished pixels straight into a buffer on the primary device over NVLink (peer access), so there is no gather step;
+// without peer access the shard is rendered locally and every finished band is copied with cudaMemcpyPeerAsync.
+int setUpShard(ftb_scene* sc, const ftb_render_params& p, const FrameGeom& full, const ftb_debug_out* dbg, const std::vector<int>& devs, int kBands, std::vector<Shard>& sh, int k)
+{
+    const int dev = devs[(size_t)k], primary = devs[0], n_gpus = (int)devs.size();
+    CK(cudaSetDevice(dev));
+    Shard& S = sh[(size_t)k];
+    int rc = getDevice(sc, dev, &S.pd);
+    if (rc != FTB_OK) return rc;
+    PerDevice* pd = S.pd;
+    S.ps = p; S.ps.shard_index = n_gpus > 1 ? k : 0; S.ps.shard_count = n_gpus;
+    if ((rc = frameGeom(&S.ps, S.g)) != FTB_OK) return rc;
+    const size_t tileBytes = (size_t)S.g.n_local_tiles * FTB_TILE_PIXELS * 3 * realSize(p.precision);
+    CK(pd->tiles.reserve(tileBytes));
+    while ((int)pd->band_events.size() < kBands) {
+        cudaEvent_t e;
+        CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        pd->band_events.push_back(e);
+    }
+    S.dbg = {nullptr, nullptr, nullptr};
+    if (dbg && dbg->prim_id) {
+        CK(pd->dbg_prim.reserve((size_t)full.n_samples * 4));
+        CK(cudaMemsetAsync(pd->dbg_prim.p, 0xff, (size_t)full.n_samples * 4, pd->stream));
+        S.dbg.prim_id = static_cast<int32_t*>(pd->dbg_prim.p);
+        if (dbg->sub_id) { CK(pd->dbg_sub.reserve((size_t)full.n_samples * 4)); CK(cudaMemsetAsync(pd->dbg_sub.p, 0, (size_t)full.n_samples * 4, pd->stream)); S.dbg.sub_id = static_cast<int32_t*>(pd->dbg_sub.p); }
+        if (dbg->t) { CK(pd->dbg_t.reserve((size_t)full.n_samples * 8)); CK(cudaMemsetAsync(pd->dbg_t.p, 0, (size_t)full.n_samples * 8, pd->stream)); S.dbg.t = static_cast<double*>(pd->dbg_t.p); }
+    }
+    S.target = S.gather = pd->tiles.p; S.direct = false;
+    if (k > 0) {
+        PerDevice* p0 = sh[0].pd;
+        if ((int)p0->peer_tiles.size() < n_gpus) p0->peer_tiles.resize((size_t)n_gpus);
+        CK(cudaSetDevice(primary));
+        CK(p0->peer_tiles[(size_t)k].reserve(tileBytes));
+        CK(cudaSetDevice(dev));
+        int can = 0;
+        if (cudaDeviceCanAccessPeer(&can, dev, primary) == cudaSuccess && can) {
+            cudaError_t pe = cudaDeviceEnablePeerAccess(primary, 0);
+            if (pe == cudaSuccess || pe == cudaErrorPeerAccessAlreadyEnabled) S.direct = true;
+            (void)cudaGetLastError();
+        }
+        S.gather = p0->peer_tiles[(size_t)k].p;
+        if (S.direct) S.target = S.gather;
+    }
+    return FTB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -863,9 +961,6 @@ int ftb_scene_create(const ftb_scene_desc* desc, ftb_scene** out)
     if (rc != FTB_OK) return fail(rc, err);
     if (sc->L.max_csg_lists > ftb::kMaxLists) return fail(FTB_ERR_UNSUPPORTED, "CSG nesting needs more than 12 pending hit lists");
     if (sc->L.leaves.size() >= (1u << 22)) return fail(FTB_ERR_UNSUPPORTED, "more than 4M leaves");
-    sc->bsp_nodes.assign(desc->bsp_nodes, desc->bsp_nodes + desc->n_bsp_nodes);
-    sc->bsp_leaves.assign(desc->bsp_leaves, desc->bsp_leaves + desc->n_bsp_leaves);
-    sc->meshes.assign(desc->meshes, desc->meshes + desc->n_meshes);
     sc->triangles.assign(desc->triangles, desc->triangles + 9 * (size_t)desc->n_triangles);
     sc->lights.assign(desc->lights, desc->lights + desc->n_lights);
     for (int i = 0; i < desc->n_images; ++i) {
@@ -881,31 +976,7 @@ int ftb_scene_create(const ftb_scene_desc* desc, ftb_scene** out)
     if (cudaGetDeviceCount(&n) != cudaSuccess || n < 1) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device: functracer_b200 has no CPU path"); }
     int dev = 0;
     CK(cudaGetDevice(&dev));
-    if (sc->L.has_mesh) {
-        // BspMesh.fs:30-65 builds the reference's tree; the device's own index over the same triangles is built here: on the
-        // GPU for large meshes (bvh_build.cu), on the host for small ones and as the fallback
-        std::vector<std::vector<int32_t>> order;
-        ftb::enumerateMeshes(*desc, sc->L, order);
-        size_t meshTriangles = 0;
-        for (const auto& o : order) meshTriangles += o.size();
-        bool done = false;
-        if (meshTriangles >= kLargeMesh) {
-            const int radii[3] = {16, 8, 4};
-            for (int k = 0; k < 3 && !done; ++k) {
-                std::string why;
-                done = ftb::buildMeshIndexDevice(desc->triangles, desc->n_triangles, order, ftb::kBspStack, radii[k], sc->L, sc->bvh_stats, why);
-                if (!done && std::getenv("FTB_VERBOSE")) std::fprintf(stderr, "functracer_b200: device BVH build not used (%s)\n", why.c_str());
-            }
-            sc->bvh_on_device = done;
-        }
-        if (!done) {
-            const auto t0 = std::chrono::steady_clock::now();
-            ftb::buildMeshIndexHost(*desc, sc->L);
-            sc->bvh_stats.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-        }
-        if (sc->L.max_bvh_depth + 2 > ftb::kBspStack) return fail(FTB_ERR_UNSUPPORTED, "mesh index deeper than the 64-entry traversal stack");
-        if (largeMesh(sc->L)) sc->L.features |= (unsigned)FT_MESHPK;  // the warp-packet walk (render.cuh)
-    }
+    if (sc->L.has_mesh && (rc = buildMeshIndex(*desc, *sc)) != FTB_OK) return rc;
     lap("mesh index");
     PerDevice* pd = nullptr;
     rc = getDevice(sc.get(), dev, &pd);
@@ -948,30 +1019,25 @@ int ftb_render_tiles_device(ftb_scene* scene, const ftb_camera* camera, const ft
     FrameGeom g;
     int rc = frameGeom(params, g);
     if (rc != FTB_OK) return rc;
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device"); }
     PerDevice* pd = nullptr;
-    if ((rc = getDevice(scene, dev, &pd)) != FTB_OK) return rc;
+    if ((rc = currentDevice(scene, &pd)) != FTB_OK) return rc;
     if (stats) std::memset(stats, 0, sizeof(*stats));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if ((rc = launchFrameAny(scene, pd, camera, params, g, d_tiles, d_dbg, stats, s, stats != nullptr, g.band_count, nullptr, g.band_count > 1 ? g.band_index : -1)) != FTB_OK) return rc;
-    if (stats) {  // the only synchronising path of this entry point
-        bool overflow = false;
-        if ((rc = finishStats(scene, pd, stats, s, true, &overflow)) != FTB_OK) return rc;
-        if (overflow) return fail(FTB_ERR_HIT_OVERFLOW, "a CSG operand produced more than 32 crossings on one ray");
-    }
-    return FTB_OK;
+    rc = byPrecision(params->precision, [&](auto r) {  // band band_index of band_count (without bands: band 0 of 1, all tiles)
+        Launch<decltype(r)> fr;
+        int e = fr.prepareFrame(scene, pd, camera, params, g, d_tiles, d_dbg, stats, s, g.band_count);
+        if (e == FTB_OK) e = fr.launchChunk(g.band_index, s);
+        return e == FTB_OK ? fr.finishFrame(stats, s) : e;
+    });
+    if (rc != FTB_OK) return rc;
+    bool overflow = false;
+    if (stats && (rc = finishStats(scene, pd, stats, s, &overflow)) != FTB_OK) return rc;  // the only synchronising path of this entry point
+    return overflow ? overflowError() : FTB_OK;
 }
 
 int ftb_assemble_device(const ftb_render_params* params, const void* const* d_tile_buffers, void* d_out, void* stream)
 {
-    if (!params || !d_tile_buffers || !d_out) return fail(FTB_ERR_BAD_ARG, "null argument");
-    FrameGeom g;
-    int rc = frameGeom(params, g);
-    if (rc != FTB_OK) return rc;
-    for (int i = 0; i < g.shard_count; ++i)
-        if (!d_tile_buffers[i]) return fail(FTB_ERR_BAD_ARG, "null tile buffer");
-    return launchAssemble(params, g, d_tile_buffers, d_out, static_cast<cudaStream_t>(stream));
+    return ftb_assemble_rows_device(params, d_tile_buffers, d_out, 0, params ? params->height : 0, stream);
 }
 
 int ftb_band_rows(const ftb_render_params* params, int band_index, int band_count, int* y0, int* y1)
@@ -982,8 +1048,8 @@ int ftb_band_rows(const ftb_render_params* params, int band_index, int band_coun
     if (rc != FTB_OK) return rc;
     if (band_count < 1 || band_count > 64 || band_index < 0 || band_index >= band_count) return fail(FTB_ERR_BAD_ARG, "bad band");
     if (g.corner && band_count > 1) return fail(FTB_ERR_UNSUPPORTED, "corner sampling blends across tile rows: render it as one band");
-    *y0 = std::min(params->height, bandFirstRow(band_index, band_count, g.tiles_y) * FTB_TILE_H);
-    *y1 = std::min(params->height, bandFirstRow(band_index + 1, band_count, g.tiles_y) * FTB_TILE_H);
+    *y0 = bandPixelRow(band_index, band_count, g.tiles_y, params->height);
+    *y1 = bandPixelRow(band_index + 1, band_count, g.tiles_y, params->height);
     return FTB_OK;
 }
 
@@ -1002,10 +1068,8 @@ int ftb_assemble_rows_device(const ftb_render_params* params, const void* const*
 int ftb_host_copy_begin(ftb_scene* scene, const void* d_src, void* host_dst, int64_t bytes, void* stream)
 {
     if (!scene || bytes < 0 || (bytes > 0 && (!d_src || !host_dst))) return fail(FTB_ERR_BAD_ARG, "null argument");
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device"); }
     PerDevice* pd = nullptr;
-    int rc = getDevice(scene, dev, &pd);
+    int rc = currentDevice(scene, &pd);
     if (rc != FTB_OK) return rc;
     CK(pd->copier.begin(d_src, host_dst, (size_t)bytes, static_cast<cudaStream_t>(stream)));
     return FTB_OK;
@@ -1014,10 +1078,8 @@ int ftb_host_copy_begin(ftb_scene* scene, const void* d_src, void* host_dst, int
 int ftb_host_copy_finish(ftb_scene* scene)
 {
     if (!scene) return fail(FTB_ERR_BAD_ARG, "null argument");
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device"); }
     PerDevice* pd = nullptr;
-    int rc = getDevice(scene, dev, &pd);
+    int rc = currentDevice(scene, &pd);
     if (rc != FTB_OK) return rc;
     CK(pd->copier.finish());
     return FTB_OK;
@@ -1026,16 +1088,13 @@ int ftb_host_copy_finish(ftb_scene* scene)
 int ftb_check_overflow(ftb_scene* scene, void* stream)
 {
     if (!scene) return fail(FTB_ERR_BAD_ARG, "null argument");
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device"); }
     PerDevice* pd = nullptr;
-    int rc = getDevice(scene, dev, &pd);
+    int rc = currentDevice(scene, &pd);
     if (rc != FTB_OK) return rc;
-    if (!pd->control.p) { CK(cudaStreamSynchronize(static_cast<cudaStream_t>(stream))); return FTB_OK; }  // nothing rendered yet
+    if (!pd->control.used()) { CK(cudaStreamSynchronize(static_cast<cudaStream_t>(stream))); return FTB_OK; }  // nothing rendered yet
     bool overflow = false;
-    if ((rc = finishStats(scene, pd, nullptr, static_cast<cudaStream_t>(stream), false, &overflow)) != FTB_OK) return rc;
-    if (overflow) return fail(FTB_ERR_HIT_OVERFLOW, "a CSG operand produced more than 32 crossings on one ray");
-    return FTB_OK;
+    if ((rc = finishStats(scene, pd, nullptr, static_cast<cudaStream_t>(stream), &overflow)) != FTB_OK) return rc;
+    return overflow ? overflowError() : FTB_OK;
 }
 
 int ftb_render(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params, void* out, const ftb_debug_out* dbg, ftb_stats* stats)
@@ -1074,90 +1133,48 @@ int ftb_render(ftb_scene* scene, const ftb_camera* camera, const ftb_render_para
     const int kBands = bandable ? 4 : 1;
     const int primary = devs[0];
 
-    struct Shard { PerDevice* pd; FrameGeom g; ftb_render_params ps; void* target; bool direct; };
     std::vector<Shard> sh((size_t)n_gpus);
-    std::vector<const void*> bufs((size_t)n_gpus);
     // ---- render: one shard per device, every band of every device queued before anything is waited on ----------------
     for (int k = 0; k < n_gpus; ++k) {
-        const int dev = devs[(size_t)k];
-        CK(cudaSetDevice(dev));
-        Shard& S = sh[(size_t)k];
-        if ((rc = getDevice(scene, dev, &S.pd)) != FTB_OK) return rc;
-        PerDevice* pd = S.pd;
-        S.ps = p;
-        S.ps.shard_index = n_gpus > 1 ? k : 0; S.ps.shard_count = n_gpus;
-        if ((rc = frameGeom(&S.ps, S.g)) != FTB_OK) return rc;
-        const size_t tileBytes = (size_t)S.g.n_local_tiles * FTB_TILE_PIXELS * 3 * rs;
-        CK(pd->tiles.reserve(tileBytes));
-        while ((int)pd->band_events.size() < kBands) {
-            cudaEvent_t e;
-            CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            pd->band_events.push_back(e);
-        }
-        ftb_debug_out ddbg = {nullptr, nullptr, nullptr};
-        if (dbg && dbg->prim_id) {
-            CK(pd->dbg_prim.reserve((size_t)full.n_samples * 4));
-            CK(cudaMemsetAsync(pd->dbg_prim.p, 0xff, (size_t)full.n_samples * 4, pd->stream));
-            ddbg.prim_id = static_cast<int32_t*>(pd->dbg_prim.p);
-            if (dbg->sub_id) { CK(pd->dbg_sub.reserve((size_t)full.n_samples * 4)); CK(cudaMemsetAsync(pd->dbg_sub.p, 0, (size_t)full.n_samples * 4, pd->stream)); ddbg.sub_id = static_cast<int32_t*>(pd->dbg_sub.p); }
-            if (dbg->t) { CK(pd->dbg_t.reserve((size_t)full.n_samples * 8)); CK(cudaMemsetAsync(pd->dbg_t.p, 0, (size_t)full.n_samples * 8, pd->stream)); ddbg.t = static_cast<double*>(pd->dbg_t.p); }
-        }
-        // Shards of the other devices: the render kernel's fold stores finished pixels straight into a buffer on the
-        // primary device over NVLink (peer access), so there is no gather step; without peer access the shard is
-        // rendered locally and every finished band is copied with cudaMemcpyPeerAsync.
-        S.target = pd->tiles.p;
-        S.direct = false;
-        if (k > 0) {
-            PerDevice* p0 = sh[0].pd;
-            if ((int)p0->peer_tiles.size() < n_gpus) p0->peer_tiles.resize((size_t)n_gpus);
-            CK(cudaSetDevice(primary));
-            CK(p0->peer_tiles[(size_t)k].reserve(tileBytes));
-            CK(cudaSetDevice(dev));
-            int can = 0;
-            if (cudaDeviceCanAccessPeer(&can, dev, primary) == cudaSuccess && can) {
-                cudaError_t pe = cudaDeviceEnablePeerAccess(primary, 0);
-                if (pe == cudaSuccess || pe == cudaErrorPeerAccessAlreadyEnabled) S.direct = true;
-                (void)cudaGetLastError();
+        if ((rc = setUpShard(scene, p, full, dbg, devs, kBands, sh, k)) != FTB_OK) return rc;
+        const Shard& S = sh[(size_t)k];
+        rc = byPrecision(p.precision, [&](auto r) -> int {
+            Launch<decltype(r)> fr;
+            int e = fr.prepareFrame(scene, S.pd, camera, &S.ps, S.g, S.target, S.dbg.prim_id ? &S.dbg : nullptr, stats, S.pd->stream, kBands);
+            if (e != FTB_OK) return e;
+            for (int c = 0; c < kBands; ++c) {
+                if ((e = fr.launchChunk(c, S.pd->stream)) != FTB_OK) return e;
+                if (k > 0 && !S.direct) {  // the band's tiles are a contiguous run of local tiles (tile rows grow with the local index)
+                    const size_t l0 = (size_t)S.pd->chunk_first[(size_t)c], l1 = (size_t)S.pd->chunk_first[(size_t)c + 1], off = l0 * FTB_TILE_PIXELS * 3 * rs, n = (l1 - l0) * FTB_TILE_PIXELS * 3 * rs;
+                    if (n) CK(cudaMemcpyPeerAsync(static_cast<char*>(S.gather) + off, primary, static_cast<const char*>(S.pd->tiles.p) + off, S.pd->device, n, S.pd->stream));
+                    if (stats) stats->kernel_launches += 1;
+                }
+                CK(cudaEventRecord(S.pd->band_events[(size_t)c], S.pd->stream));
             }
-            if (S.direct) S.target = p0->peer_tiles[(size_t)k].p;
-            bufs[(size_t)k] = p0->peer_tiles[(size_t)k].p;
-        } else bufs[0] = pd->tiles.p;
-        ChunkDone bandDone = [&, k, dev](int c) -> int {
-            Shard& Sk = sh[(size_t)k];
-            if (k > 0 && !Sk.direct) {  // the band's tiles are a contiguous run of local tiles (tile rows grow with the local index)
-                const size_t l0 = kBands > 1 ? (size_t)Sk.pd->chunk_first[(size_t)c] : 0, l1 = kBands > 1 ? (size_t)Sk.pd->chunk_first[(size_t)c + 1] : (size_t)Sk.g.n_local_tiles;
-                const size_t off = l0 * FTB_TILE_PIXELS * 3 * rs, n = (l1 - l0) * FTB_TILE_PIXELS * 3 * rs;
-                if (n) CK(cudaMemcpyPeerAsync(static_cast<char*>(sh[0].pd->peer_tiles[(size_t)k].p) + off, primary, static_cast<const char*>(Sk.pd->tiles.p) + off, dev, n, Sk.pd->stream));
-                if (stats) stats->kernel_launches += 1;
-            }
-            CK(cudaEventRecord(Sk.pd->band_events[(size_t)c], Sk.pd->stream));
-            return FTB_OK;
-        };
-        if ((rc = launchFrameAny(scene, pd, camera, &S.ps, S.g, S.target, ddbg.prim_id ? &ddbg : nullptr, stats, pd->stream, stats != nullptr, kBands, &bandDone)) != FTB_OK) return rc;
+            return fr.finishFrame(stats, S.pd->stream);
+        });
+        if (rc != FTB_OK) return rc;
     }
     // ---- assemble + download on the primary device, band by band, behind the rendering ------------------------------------
     CK(cudaSetDevice(primary));
     PerDevice* p0 = sh[0].pd;
     CK(p0->out.reserve(frameBytes));
-    ftb_render_params pa = p;
-    pa.shard_index = 0; pa.shard_count = n_gpus;
-    FrameGeom ga;
-    if ((rc = frameGeom(&pa, ga)) != FTB_OK) return rc;
+    std::vector<const void*> bufs;
+    for (const Shard& S : sh) bufs.push_back(S.gather);
     for (int c = 0; c < kBands; ++c) {
-        const int r0 = bandFirstRow(c, kBands, full.tiles_y), r1 = bandFirstRow(c + 1, kBands, full.tiles_y);
-        const int y0 = kBands > 1 ? std::min(p.height, r0 * FTB_TILE_H) : 0, y1 = kBands > 1 ? std::min(p.height, r1 * FTB_TILE_H) : p.height;
+        const int y0 = bandPixelRow(c, kBands, full.tiles_y, p.height), y1 = bandPixelRow(c + 1, kBands, full.tiles_y, p.height);
         for (int k = 0; k < n_gpus; ++k) CK(cudaStreamWaitEvent(p0->copy_stream, sh[(size_t)k].pd->band_events[(size_t)c], 0));
         if (y1 <= y0) continue;
-        if ((rc = launchAssemble(&pa, ga, bufs.data(), p0->out.p, p0->copy_stream, y0, y1)) != FTB_OK) return rc;
+        if ((rc = launchAssemble(&sh[0].ps, sh[0].g, bufs.data(), p0->out.p, p0->copy_stream, y0, y1)) != FTB_OK) return rc;
         if (stats) stats->kernel_launches += 1;
         CK(p0->copier.begin(static_cast<const char*>(p0->out.p) + (size_t)y0 * rowBytes, static_cast<char*>(out) + (size_t)y0 * rowBytes, (size_t)(y1 - y0) * rowBytes, p0->copy_stream));
     }
     CK(p0->copier.finish());
     CK(cudaStreamSynchronize(p0->copy_stream));
     bool overflow = false;
-    for (int k = 0; k < n_gpus; ++k) {
-        CK(cudaSetDevice(sh[(size_t)k].pd->device));
-        if ((rc = finishStats(scene, sh[(size_t)k].pd, stats, sh[(size_t)k].pd->stream, stats != nullptr, &overflow)) != FTB_OK) return rc;
+    for (const Shard& S : sh) {
+        CK(cudaSetDevice(S.pd->device));
+        if ((rc = finishStats(scene, S.pd, stats, S.pd->stream, &overflow)) != FTB_OK) return rc;
     }
     CK(cudaSetDevice(primary));
     if (dbg && dbg->prim_id) {
@@ -1167,8 +1184,7 @@ int ftb_render(ftb_scene* scene, const ftb_camera* camera, const ftb_render_para
     }
     CK(cudaStreamSynchronize(p0->stream));
     if (stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    if (overflow) return fail(FTB_ERR_HIT_OVERFLOW, "a CSG operand produced more than 32 crossings on one ray");
-    return FTB_OK;
+    return overflow ? overflowError() : FTB_OK;
 }
 
 int ftb_shade_rays(ftb_scene* scene, const double* rays_od, int64_t n, const ftb_render_params* params, double* out_rgb,
@@ -1187,52 +1203,36 @@ int ftb_shade_rays(ftb_scene* scene, const double* rays_od, int64_t n, const ftb
     PerDevice* pd = nullptr;
     int rc = getDevice(scene, dev, &pd);
     if (rc != FTB_OK) return rc;
-    const bool f64 = params->precision == FTB_PRECISION_FP64_VERIFY;
-    const size_t rs = f64 ? 8 : 4;
     cudaStream_t s = pd->stream;
     CK(pd->rays.reserve((size_t)n * 48));
     CK(cudaMemcpyAsync(pd->rays.p, rays_od, (size_t)n * 48, cudaMemcpyHostToDevice, s));
-    CK(pd->tiles.reserve((size_t)n * 3 * rs));
+    CK(pd->tiles.reserve((size_t)n * 3 * realSize(params->precision)));
     CK(pd->out.reserve((size_t)n * 24));
-    CK(pd->control.reserve(sizeof(Control)));
-    CK(cudaMemsetAsync(pd->control.p, 0, sizeof(Control), s));
+    CK(pd->control.resetAll(s));
     ftb_debug_out ddbg = {nullptr, nullptr, nullptr};
     if (dbg && dbg->prim_id) {
         CK(pd->dbg_prim.reserve((size_t)n * 4)); ddbg.prim_id = static_cast<int32_t*>(pd->dbg_prim.p);
         if (dbg->sub_id) { CK(pd->dbg_sub.reserve((size_t)n * 4)); ddbg.sub_id = static_cast<int32_t*>(pd->dbg_sub.p); }
         if (dbg->t) { CK(pd->dbg_t.reserve((size_t)n * 8)); ddbg.t = static_cast<double*>(pd->dbg_t.p); }
     }
-    Control* ctl = static_cast<Control*>(pd->control.p);
-    const bool wantStats = stats && params->collect_stats;
-    int launches = 0;
-    auto run = [&](auto tag) -> int {
-        typedef decltype(tag) R;
-        SceneStorage<R>& st = storageOf<R>(pd);
-        if (!st.ready) { int r2 = uploadScene<R>(*scene, st); if (r2 != FTB_OK) return r2; }
-        DevFrame<R> F;
-        std::memset(&F, 0, sizeof(F));
+    rc = byPrecision(params->precision, [&](auto r) -> int {
+        typedef decltype(r) R;
+        Launch<R> fr;
+        int e = fr.begin(scene, pd, params, scene->L.features, stats && params->collect_stats, pd->tiles.p, &ddbg);
+        if (e != FTB_OK) return e;
+        DevFrame<R>& F = fr.F;
         F.mode = 1; F.spp = 1; F.s_base = 0; F.s_count = 1; F.run = 1; F.rpp_magic = 0;
-        F.n_blocks = (int)((n + 31) / 32);
-        F.n_rays = n;
-        F.n_local_tiles = (int)((n + FTB_TILE_PIXELS - 1) / FTB_TILE_PIXELS);
-        F.shard_count = 1;
-        F.rays = static_cast<const double*>(pd->rays.p);
-        F.recursion_limit = params->recursion_limit;
-        F.seed = params->seed;
-        F.out = static_cast<R*>(pd->tiles.p);
-        F.dbg_prim = ddbg.prim_id; F.dbg_sub = ddbg.sub_id; F.dbg_t = ddbg.t;
-        F.tile_counter = &ctl->tile_counter; F.overflow = &ctl->overflow; F.stats = ctl->stats;
+        F.n_blocks = (int)((n + 31) / 32); F.n_rays = n; F.rays = static_cast<const double*>(pd->rays.p);
+        F.n_local_tiles = (int)((n + FTB_TILE_PIXELS - 1) / FTB_TILE_PIXELS); F.shard_count = 1;
         CK(cudaEventRecord(pd->ev0, s));
-        const Variant<R>* var = pickVariant<R>(scene->L.features, wantStats);
-        if (!var) return fail(FTB_ERR_UNSUPPORTED, "no kernel variant covers this scene's feature mask");
-        CK(var->launch(st.view, F, wantStats, pd->sm_count, s, &launches));
+        CK(fr.launchKernel(s));
         CK(cudaEventRecord(pd->ev1, s));
         const long long m = 3 * (long long)n;
         widen_kernel<R><<<(int)std::min<long long>((m + 255) / 256, 148 * 16), 256, 0, s>>>(static_cast<const R*>(pd->tiles.p), static_cast<double*>(pd->out.p), m);
         CK(cudaGetLastError());
+        if (stats) stats->kernel_launches = fr.launches + 2;
         return FTB_OK;
-    };
-    rc = f64 ? run(double()) : run(float());
+    });
     if (rc != FTB_OK) return rc;
     CK(cudaMemcpyAsync(out_rgb, pd->out.p, (size_t)n * 24, cudaMemcpyDeviceToHost, s));
     if (ddbg.prim_id) {
@@ -1241,11 +1241,9 @@ int ftb_shade_rays(ftb_scene* scene, const double* rays_od, int64_t n, const ftb
         if (ddbg.t) CK(cudaMemcpyAsync(dbg->t, ddbg.t, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
     }
     bool overflow = false;
-    if (stats) stats->kernel_launches = launches + 2;
-    if ((rc = finishStats(scene, pd, stats, s, true, &overflow)) != FTB_OK) return rc;
+    if ((rc = finishStats(scene, pd, stats, s, &overflow)) != FTB_OK) return rc;
     if (stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    if (overflow) return fail(FTB_ERR_HIT_OVERFLOW, "a CSG operand produced more than 32 crossings on one ray");
-    return FTB_OK;
+    return overflow ? overflowError() : FTB_OK;
 }
 
 }  // extern "C"
