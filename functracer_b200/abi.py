@@ -131,5 +131,5 @@ EXPORTS = [
     "ftb_abi_version", "ftb_device_count", "ftb_last_error", "ftb_scene_create", "ftb_scene_destroy",
     "ftb_render", "ftb_tile_buffer_bytes", "ftb_render_tiles_device", "ftb_assemble_device",
     "ftb_shade_rays", "ftb_band_rows", "ftb_assemble_rows_device", "ftb_host_copy_begin", "ftb_host_copy_finish",
-    "ftb_check_overflow", "ftb_scene_build_info",
+    "ftb_check_overflow", "ftb_scene_build_info", "ftb_render_window", "ftb_render_window_tiles_device",
 ]

@@ -68,6 +68,15 @@ def lib():
         else:
             L.ftb_scene_build_info.argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(C.c_double), C.POINTER(C.c_double)]
             L.ftb_scene_build_info.restype = C.c_int
+        for name, args in (("ftb_render_window", [vp, C.POINTER(abi.Camera), C.POINTER(abi.RenderParams)] + [C.c_int32] * 4
+                            + [vp, C.POINTER(abi.DebugOut), C.POINTER(abi.Stats)]),
+                           ("ftb_render_window_tiles_device", [vp, C.POINTER(abi.Camera), C.POINTER(abi.RenderParams)] + [C.c_int32] * 4
+                            + [vp, C.POINTER(abi.DebugOut), C.POINTER(abi.Stats), vp])):
+            if os.environ.get("FTB_LIB") and not hasattr(L, name):
+                setattr(L, name, None)  # an older A/B build of the same ABI without windows
+            else:
+                getattr(L, name).argtypes = args
+                getattr(L, name).restype = C.c_int
         if L.ftb_abi_version() != abi.ABI_VERSION:
             raise RuntimeError("ABI version mismatch: library %d, bindings %d" % (L.ftb_abi_version(), abi.ABI_VERSION))
         _LIB = L
@@ -133,9 +142,20 @@ class Scene:
         p = make_params(width, height, spp, jitter_xy, **kw)
         return self.render_params(p, debug=debug, stats=stats, out=out, camera=camera)
 
-    def render_params(self, p, debug=False, stats=False, out=None, camera=None):
+    def render_window(self, window, width, height, spp, jitter_xy=None, debug=False, stats=False, out=None, camera=None, **kw):
+        """The pixels window = (x0, y0, x1, y1), i.e. [x0, x1) x [y0, y1), of the width x height frame, bit-identical to
+        render() there.  Returns render()'s dict with rgb[y1 - y0, x1 - x0, C] and the window's debug planes."""
+        if stats:
+            kw.setdefault("collect_stats", 1)
+        p = make_params(width, height, spp, jitter_xy, **kw)
+        return self.render_params(p, debug=debug, stats=stats, out=out, camera=camera, window=window)
+
+    def render_params(self, p, debug=False, stats=False, out=None, camera=None, window=None):
+        """window: optional (x0, y0, x1, y1); the outputs then hold the window's pixels and samples only."""
         dt, ch = _OUT_DTYPE[p.out_format]
         W, H = p.width, p.height
+        if window is not None:
+            W, H = window[2] - window[0], window[3] - window[1]
         if out is None:
             out = np.empty((H, W, ch), dtype=dt)
         assert out.dtype == dt and out.size == W * H * ch and out.flags["C_CONTIGUOUS"]
@@ -149,8 +169,11 @@ class Scene:
                                t.ctypes.data_as(C.POINTER(C.c_double)))
         st = abi.Stats() if stats else None
         cam = camera if camera is not None else self.parsed.camera_ptr
-        _check(lib().ftb_render(self._h, cam, C.byref(p), out.ctypes.data_as(C.c_void_p), C.byref(dbg) if dbg else None,
-                                C.byref(st) if st is not None else None))
+        args = (out.ctypes.data_as(C.c_void_p), C.byref(dbg) if dbg else None, C.byref(st) if st is not None else None)
+        if window is None:
+            _check(lib().ftb_render(self._h, cam, C.byref(p), *args))
+        else:
+            _check(_window_entry("ftb_render_window")(self._h, cam, C.byref(p), *[int(v) for v in window], *args))
         return dict(rgb=out, prim=prim, sub=sub, t=t, stats=st)
 
     # -- Shading.shade (Shading.fs:141-147) on explicit rays -----------------------------------------
@@ -175,17 +198,26 @@ class Scene:
         return dict(rgb=rgb, prim=prim, sub=sub, t=t, stats=st)
 
     # -- device-buffer entry points (one process per GPU; pointers are raw device addresses) -----
-    def render_tiles_device(self, p, d_tiles_ptr, stream=0, stats=False, camera=None, d_dbg=None):
-        """d_dbg: optional (prim_ptr, sub_ptr, t_ptr) DEVICE addresses of per-sample debug planes (0 / None = not wanted)."""
+    def render_tiles_device(self, p, d_tiles_ptr, stream=0, stats=False, camera=None, d_dbg=None, window=None):
+        """d_dbg: optional (prim_ptr, sub_ptr, t_ptr) DEVICE addresses of per-sample debug planes (0 / None = not wanted).
+        window: optional (x0, y0, x1, y1), see render_window_tiles_device."""
         st = abi.Stats() if stats else None
         cam = camera if camera is not None else self.parsed.camera_ptr
         dbg = None
         if d_dbg is not None:
             dbg = abi.DebugOut(C.cast(C.c_void_p(d_dbg[0] or None), C.POINTER(C.c_int32)), C.cast(C.c_void_p(d_dbg[1] or None), C.POINTER(C.c_int32)),
                                C.cast(C.c_void_p(d_dbg[2] or None), C.POINTER(C.c_double)))
-        _check(lib().ftb_render_tiles_device(self._h, cam, C.byref(p), C.c_void_p(d_tiles_ptr), C.byref(dbg) if dbg is not None else None,
-                                             C.byref(st) if st is not None else None, C.c_void_p(stream)))
+        args = (C.c_void_p(d_tiles_ptr), C.byref(dbg) if dbg is not None else None, C.byref(st) if st is not None else None, C.c_void_p(stream))
+        if window is None:
+            _check(lib().ftb_render_tiles_device(self._h, cam, C.byref(p), *args))
+        else:
+            _check(_window_entry("ftb_render_window_tiles_device")(self._h, cam, C.byref(p), *[int(v) for v in window], *args))
         return st
+
+    def render_window_tiles_device(self, p, window, d_tiles_ptr, stream=0, stats=False, camera=None, d_dbg=None):
+        """This shard's (band's) tiles of the window (x0, y0, x1, y1) of the frame p describes.  The buffer is that of a frame
+        of the window's size: size it, band it and assemble it with window_params(p, window)."""
+        return self.render_tiles_device(p, d_tiles_ptr, stream=stream, stats=stats, camera=camera, d_dbg=d_dbg, window=window)
 
     def build_info(self):
         """dict(bvh_on_device, bvh_build_ms, bvh_total_ms): how the scene's mesh index was built at create time."""
@@ -208,6 +240,22 @@ class Scene:
 
     def host_copy_finish(self):
         _check(lib().ftb_host_copy_finish(self._h))
+
+
+def _window_entry(name):
+    fn = getattr(lib(), name)
+    if fn is None:
+        raise RuntimeError("%s has no %s (an older build)" % (os.environ.get("FTB_LIB"), name))
+    return fn
+
+
+def window_params(p, window):
+    """A copy of params p with the width / height of window (x0, y0, x1, y1): the params that size (tile_buffer_bytes),
+    band (band_rows) and assemble (assemble_device, assemble_rows_device) a window's tile buffer."""
+    q = abi.RenderParams.from_buffer_copy(p)
+    q.width, q.height = window[2] - window[0], window[3] - window[1]
+    q._keep = getattr(p, "_keep", None)
+    return q
 
 
 def band_rows(p, band_index, band_count):

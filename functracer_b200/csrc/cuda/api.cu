@@ -492,14 +492,22 @@ int getDevice(ftb_scene* sc, int device, PerDevice** out)
     return FTB_OK;
 }
 
+// A pixel window [x0, x1) x [y0, y1) of the frame; the whole frame is {0, 0, width, height}.
+struct Window { int x0, y0, x1, y1; };
+
+// The geometry of one frame's work.  gw / gh are the whole frame's sample grid (ray directions, RNG keys); everything
+// else - tile grid, local tiles, samples, bands - is the window's, whose tile grid starts at its origin.
 struct FrameGeom {
-    int gw, gh, spp, tiles_x, tiles_y, n_tiles, shard_index, shard_count, n_local_tiles;
+    int gw, gh;                  // the whole frame's sample grid
+    int wx0, wy0, ww, wh;        // the window in the sample grid: origin and size ((w+1) x (h+1) corners in corner mode)
+    int width, height;           // the window in pixels: the frame that its tile buffer and assembly are those of
+    int spp, tiles_x, tiles_y, n_tiles, shard_index, shard_count, n_local_tiles;
     int band_index, band_count;  // ftb_render_tiles_device: only the tiles of one band of tile rows (band_count <= 1: all)
     long long n_samples;
     bool corner;
 };
 
-int frameGeom(const ftb_render_params* p, FrameGeom& g)
+int frameGeom(const ftb_render_params* p, FrameGeom& g, const Window* win = nullptr)
 {
     if (!p) return fail(FTB_ERR_BAD_ARG, "null params");
     if (p->width < 1 || p->height < 1) return fail(FTB_ERR_BAD_ARG, "bad resolution");
@@ -507,20 +515,27 @@ int frameGeom(const ftb_render_params* p, FrameGeom& g)
     if (p->sampling != FTB_SAMPLING_JITTER && p->sampling != FTB_SAMPLING_CORNER) return fail(FTB_ERR_BAD_ARG, "bad sampling mode");
     if (p->precision != FTB_PRECISION_FP32 && p->precision != FTB_PRECISION_FP64_VERIFY) return fail(FTB_ERR_BAD_ARG, "bad precision");
     if (p->out_format < FTB_OUT_RGB_F64 || p->out_format > FTB_OUT_RGBA8) return fail(FTB_ERR_BAD_ARG, "bad output format");
+    const Window w = win ? *win : Window{0, 0, p->width, p->height};
+    if (w.x0 < 0 || w.y0 < 0 || w.x0 >= w.x1 || w.y0 >= w.y1 || w.x1 > p->width || w.y1 > p->height)
+        return fail(FTB_ERR_BAD_ARG, "bad window: needs 0 <= x0 < x1 <= width and 0 <= y0 < y1 <= height");
     g.corner = p->sampling == FTB_SAMPLING_CORNER;
     if (!g.corner && (p->spp < 1 || !p->jitter_xy)) return fail(FTB_ERR_BAD_ARG, "jitter mode needs spp >= 1 and jitter_xy");
     g.gw = g.corner ? p->width + 1 : p->width;
     g.gh = g.corner ? p->height + 1 : p->height;
+    g.width = w.x1 - w.x0; g.height = w.y1 - w.y0;
+    g.wx0 = w.x0; g.wy0 = w.y0;
+    g.ww = g.corner ? g.width + 1 : g.width;  // the corners [x0, x1] x [y0, y1]
+    g.wh = g.corner ? g.height + 1 : g.height;
     g.spp = g.corner ? 1 : p->spp;
-    g.tiles_x = (g.gw + FTB_TILE_W - 1) / FTB_TILE_W;
-    g.tiles_y = (g.gh + FTB_TILE_H - 1) / FTB_TILE_H;
+    g.tiles_x = (g.ww + FTB_TILE_W - 1) / FTB_TILE_W;
+    g.tiles_y = (g.wh + FTB_TILE_H - 1) / FTB_TILE_H;
     g.n_tiles = g.tiles_x * g.tiles_y;
     g.shard_count = p->shard_count > 1 ? p->shard_count : 1;
     g.shard_index = p->shard_count > 1 ? p->shard_index : 0;
     if (g.shard_count > kMaxShards) return fail(FTB_ERR_BAD_ARG, "shard_count exceeds 64");
     if (g.shard_index < 0 || g.shard_index >= g.shard_count) return fail(FTB_ERR_BAD_ARG, "shard_index out of range");
     g.n_local_tiles = (g.n_tiles + g.shard_count - 1) / g.shard_count;  // one per group of shard_count tiles (device_scene.h tileOfLocal); the last group may lack this shard's
-    g.n_samples = (long long)g.gw * g.gh * g.spp;
+    g.n_samples = (long long)g.ww * g.wh * g.spp;
     g.band_count = p->band_count > 1 ? p->band_count : 1;
     g.band_index = p->band_count > 1 ? p->band_index : 0;
     if (g.band_count > 64) return fail(FTB_ERR_BAD_ARG, "band_count exceeds 64");
@@ -658,9 +673,11 @@ bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render
         const double x = v.x * b.i.x + v.y * b.i.y + v.z * b.i.z, y = v.x * b.j.x + v.y * b.j.y + v.z * b.j.z, z = v.x * b.k.x + v.y * b.k.y + v.z * b.k.z;
         double xl, xh, yl, yh;
         if (!range(x, z, it.bound_r, xl, xh) || !range(y, z, it.bound_r, yl, yh)) continue;
-        // image-plane coordinates -> sample-grid pixels (rayThroughPixel, Image.fs:83-89), one pixel of slack for jitter
-        const double px0 = (xl - b.tlx) / b.pw - 1.5, px1 = (xh - b.tlx) / b.pw + 1.5, py0 = (b.tly - yh) / b.ph - 1.5, py1 = (b.tly - yl) / b.ph + 1.5;
-        if (px1 < 0 || py1 < 0 || px0 >= g.gw || py0 >= g.gh) continue;
+        // image-plane coordinates -> sample-grid pixels (rayThroughPixel, Image.fs:83-89), one pixel of slack for jitter,
+        // relative to the window's origin
+        const double px0 = (xl - b.tlx) / b.pw - 1.5 - g.wx0, px1 = (xh - b.tlx) / b.pw + 1.5 - g.wx0;
+        const double py0 = (b.tly - yh) / b.ph - 1.5 - g.wy0, py1 = (b.tly - yl) / b.ph + 1.5 - g.wy0;
+        if (px1 < 0 || py1 < 0 || px0 >= g.ww || py0 >= g.wh) continue;
         const int tx0 = (int)std::max(0.0, std::floor(px0 / FTB_TILE_W)), tx1 = (int)std::min((double)g.tiles_x - 1, std::floor(px1 / FTB_TILE_W));
         const int ty0 = (int)std::max(0.0, std::floor(py0 / FTB_TILE_H)), ty1 = (int)std::min((double)g.tiles_y - 1, std::floor(py1 / FTB_TILE_H));
         for (int ty = ty0; ty <= ty1; ++ty)
@@ -720,7 +737,8 @@ struct Launch {
         if (rc != FTB_OK) return rc;
         CK(pd->control.prepare(counting, stream));
         F.mode = 0; F.gw = g.gw; F.gh = g.gh; F.spp = g.spp; F.tiles_x = g.tiles_x;
-        // floor(2^32 / tiles_x) + 1 does not fit 32 bits for tiles_x == 1 (frames <= 16 sample columns wide): those divide
+        F.wx0 = g.wx0; F.wy0 = g.wy0; F.wx1 = g.wx0 + g.ww; F.wy1 = g.wy0 + g.wh; F.dbg_w = g.ww;
+        // floor(2^32 / tiles_x) + 1 does not fit 32 bits for tiles_x == 1 (windows <= 16 sample columns wide): those divide
         F.tiles_x_magic = (g.tiles_x > 1 && (unsigned long long)g.n_tiles * (unsigned long long)g.tiles_x < (1ull << 32)) ? (unsigned)((1ull << 32) / (unsigned)g.tiles_x) + 1u : 0u;
         F.n_local_tiles = g.n_local_tiles; F.shard_index = g.shard_index; F.shard_count = g.shard_count;
         fillCamera<R>(F, *cam, p->width, p->height);
@@ -730,10 +748,11 @@ struct Launch {
         CK(pd->jitter.reserve(j.size() * sizeof(R)));
         CK(cudaMemcpyAsync(pd->jitter.p, j.data(), j.size() * sizeof(R), cudaMemcpyHostToDevice, stream));  // pageable source: staged before return
         F.jitter = static_cast<const R*>(pd->jitter.p);
-        // tile order: cached per (camera, frame geometry, recursion limit); recomputed + uploaded only when they change
-        std::vector<unsigned char> key(sizeof(ftb_camera) + 7 * sizeof(int));
+        // tile order: cached per (camera, frame geometry, window, recursion limit); recomputed + uploaded only when they change.
+        // The order lists the window's local tiles: an order cached for another window would name tiles this one lacks.
+        std::vector<unsigned char> key(sizeof(ftb_camera) + 11 * sizeof(int));
         std::memcpy(key.data(), cam, sizeof(ftb_camera));
-        const int kk[7] = {p->width, p->height, p->sampling, g.shard_index, g.shard_count, p->recursion_limit, n_chunks};
+        const int kk[11] = {p->width, p->height, p->sampling, g.shard_index, g.shard_count, p->recursion_limit, n_chunks, g.wx0, g.wy0, g.ww, g.wh};
         std::memcpy(key.data() + sizeof(ftb_camera), kk, sizeof(kk));
         if (key != pd->order_key) {
             std::vector<int> order;
@@ -814,20 +833,21 @@ int launchAssemble(const ftb_render_params* p, const FrameGeom& g, const void* c
     TilePtrs tp;
     std::memset(&tp, 0, sizeof(tp));
     for (int i = 0; i < g.shard_count; ++i) tp.p[i] = bufs[i];
-    const long long n = (long long)p->width * (y1 - y0);
+    const long long n = (long long)g.width * (y1 - y0);
     if (n <= 0) return FTB_OK;
     int grid = (int)std::min<long long>((n + 255) / 256, 148 * 16);
     return byPrecision(p->precision, [&](auto r) -> int {
-        assemble_kernel<decltype(r)><<<grid, 256, 0, stream>>>(tp, g.shard_count, g.tiles_x, p->width, y0, y1, g.corner ? 1 : 0, p->out_format, d_out);
+        assemble_kernel<decltype(r)><<<grid, 256, 0, stream>>>(tp, g.shard_count, g.tiles_x, g.width, y0, y1, g.corner ? 1 : 0, p->out_format, d_out);
         CK(cudaGetLastError());
         return FTB_OK;
     });
 }
 
-inline size_t outBytes(const ftb_render_params* p)
+// bytes of the window's pixels in out_format
+inline size_t outBytes(int out_format, const FrameGeom& g)
 {
-    const size_t n = (size_t)p->width * p->height;
-    return p->out_format == FTB_OUT_RGB_F64 ? n * 24 : (p->out_format == FTB_OUT_RGB_F32 ? n * 12 : n * 4);
+    const size_t n = (size_t)g.width * g.height;
+    return out_format == FTB_OUT_RGB_F64 ? n * 24 : (out_format == FTB_OUT_RGB_F32 ? n * 12 : n * 4);
 }
 
 // CUDA ordinals of the devices this library runs on (compute capability 10.x), in ordinal order: what ftb_device_count
@@ -888,10 +908,11 @@ int buildMeshIndex(const ftb_scene_desc& desc, ftb_scene& sc)
 // One device's part of an ftb_render frame; the primary device's assembly reads its tiles from `gather` (== target if direct).
 struct Shard { PerDevice* pd; FrameGeom g; ftb_render_params ps; ftb_debug_out dbg; void* target; void* gather; bool direct; };
 
-// Device k's shard: geometry, tile buffer, band events, debug planes.  Shards of the other devices: the render kernel's fold
+// Device k's shard of the window `win`: geometry, tile buffer, band events, debug planes (buffers sized by the window).  Shards of the other devices: the render kernel's fold
 // stores finished pixels straight into a buffer on the primary device over NVLink (peer access), so there is no gather step;
 // without peer access the shard is rendered locally and every finished band is copied with cudaMemcpyPeerAsync.
-int setUpShard(ftb_scene* sc, const ftb_render_params& p, const FrameGeom& full, const ftb_debug_out* dbg, const std::vector<int>& devs, int kBands, std::vector<Shard>& sh, int k)
+int setUpShard(ftb_scene* sc, const ftb_render_params& p, const Window& win, const FrameGeom& full, const ftb_debug_out* dbg, const std::vector<int>& devs, int kBands,
+               std::vector<Shard>& sh, int k)
 {
     const int dev = devs[(size_t)k], primary = devs[0], n_gpus = (int)devs.size();
     CK(cudaSetDevice(dev));
@@ -900,7 +921,7 @@ int setUpShard(ftb_scene* sc, const ftb_render_params& p, const FrameGeom& full,
     if (rc != FTB_OK) return rc;
     PerDevice* pd = S.pd;
     S.ps = p; S.ps.shard_index = n_gpus > 1 ? k : 0; S.ps.shard_count = n_gpus;
-    if ((rc = frameGeom(&S.ps, S.g)) != FTB_OK) return rc;
+    if ((rc = frameGeom(&S.ps, S.g, &win)) != FTB_OK) return rc;
     const size_t tileBytes = (size_t)S.g.n_local_tiles * FTB_TILE_PIXELS * 3 * realSize(p.precision);
     CK(pd->tiles.reserve(tileBytes));
     while ((int)pd->band_events.size() < kBands) {
@@ -1015,9 +1036,17 @@ int64_t ftb_tile_buffer_bytes(const ftb_render_params* params)
 int ftb_render_tiles_device(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params, void* d_tiles,
                             const ftb_debug_out* d_dbg, ftb_stats* stats, void* stream)
 {
+    if (!params) return fail(FTB_ERR_BAD_ARG, "null argument");
+    return ftb_render_window_tiles_device(scene, camera, params, 0, 0, params->width, params->height, d_tiles, d_dbg, stats, stream);
+}
+
+int ftb_render_window_tiles_device(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params, int32_t x0, int32_t y0, int32_t x1,
+                                   int32_t y1, void* d_tiles, const ftb_debug_out* d_dbg, ftb_stats* stats, void* stream)
+{
     if (!scene || !camera || !params || !d_tiles) return fail(FTB_ERR_BAD_ARG, "null argument");
     FrameGeom g;
-    int rc = frameGeom(params, g);
+    const Window win = {x0, y0, x1, y1};
+    int rc = frameGeom(params, g, &win);
     if (rc != FTB_OK) return rc;
     PerDevice* pd = nullptr;
     if ((rc = currentDevice(scene, &pd)) != FTB_OK) return rc;
@@ -1099,12 +1128,20 @@ int ftb_check_overflow(ftb_scene* scene, void* stream)
 
 int ftb_render(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params, void* out, const ftb_debug_out* dbg, ftb_stats* stats)
 {
+    if (!params) return fail(FTB_ERR_BAD_ARG, "null argument");
+    return ftb_render_window(scene, camera, params, 0, 0, params->width, params->height, out, dbg, stats);
+}
+
+int ftb_render_window(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params, int32_t x0, int32_t y0, int32_t x1, int32_t y1,
+                      void* out, const ftb_debug_out* dbg, ftb_stats* stats)
+{
     const auto t0 = std::chrono::steady_clock::now();
     if (!scene || !camera || !params || !out) return fail(FTB_ERR_BAD_ARG, "null argument");
-    FrameGeom full;
+    FrameGeom g;  // the window's geometry
     ftb_render_params p = *params;
     p.band_index = 0; p.band_count = 0;  // banding is this call's own business
-    int rc = frameGeom(&p, full);
+    const Window win = {x0, y0, x1, y1};
+    int rc = frameGeom(&p, g, &win);
     if (rc != FTB_OK) return rc;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device: functracer_b200 has no CPU path"); }
@@ -1119,24 +1156,24 @@ int ftb_render(ftb_scene* scene, const ftb_camera* camera, const ftb_render_para
     } else devs.push_back(restore.dev);
     if (n_gpus > 1 && p.shard_count > 1) return fail(FTB_ERR_BAD_ARG, "n_gpus > 1 cannot be combined with an external shard");
     if (n_gpus > 1 && dbg) return fail(FTB_ERR_UNSUPPORTED, "debug planes need n_gpus <= 1");
-    if (full.shard_count > 1 && n_gpus == 1) {
-        // a single external shard cannot be assembled into a frame: the caller wants ftb_render_tiles_device
-        return fail(FTB_ERR_BAD_ARG, "ftb_render renders whole frames; use ftb_render_tiles_device for one shard");
+    if (g.shard_count > 1 && n_gpus == 1) {
+        // a single external shard cannot be assembled into a frame: the caller wants the device entry point
+        return fail(FTB_ERR_BAD_ARG, "ftb_render / ftb_render_window assemble all shards; use ftb_render_(window_)tiles_device for one shard");
     }
     const size_t rs = realSize(p.precision);
-    const size_t frameBytes = outBytes(&p);
-    const size_t rowBytes = frameBytes / (size_t)p.height;
+    const size_t frameBytes = outBytes(p.out_format, g);
+    const size_t rowBytes = frameBytes / (size_t)g.height;
     // The frame is rendered in bands of tile rows, on every device; a finished band is assembled and sent to the host while
     // the next bands render, so only the last, smallest band's copy is exposed.  Four bands also for small downloads: a 1080p
     // RGBA8 frame (8 MB) measured 1.44 ms with four bands against 1.71 ms in one piece (hollow-sphere, 1.17 ms device-resident).
-    const bool bandable = !dbg && !stats && !full.corner && (long long)p.width * p.height >= 262144 && full.tiles_y >= 8;
+    const bool bandable = !dbg && !stats && !g.corner && (long long)g.width * g.height >= 262144 && g.tiles_y >= 8;
     const int kBands = bandable ? 4 : 1;
     const int primary = devs[0];
 
     std::vector<Shard> sh((size_t)n_gpus);
     // ---- render: one shard per device, every band of every device queued before anything is waited on ----------------
     for (int k = 0; k < n_gpus; ++k) {
-        if ((rc = setUpShard(scene, p, full, dbg, devs, kBands, sh, k)) != FTB_OK) return rc;
+        if ((rc = setUpShard(scene, p, win, g, dbg, devs, kBands, sh, k)) != FTB_OK) return rc;
         const Shard& S = sh[(size_t)k];
         rc = byPrecision(p.precision, [&](auto r) -> int {
             Launch<decltype(r)> fr;
@@ -1162,12 +1199,12 @@ int ftb_render(ftb_scene* scene, const ftb_camera* camera, const ftb_render_para
     std::vector<const void*> bufs;
     for (const Shard& S : sh) bufs.push_back(S.gather);
     for (int c = 0; c < kBands; ++c) {
-        const int y0 = bandPixelRow(c, kBands, full.tiles_y, p.height), y1 = bandPixelRow(c + 1, kBands, full.tiles_y, p.height);
+        const int r0 = bandPixelRow(c, kBands, g.tiles_y, g.height), r1 = bandPixelRow(c + 1, kBands, g.tiles_y, g.height);
         for (int k = 0; k < n_gpus; ++k) CK(cudaStreamWaitEvent(p0->copy_stream, sh[(size_t)k].pd->band_events[(size_t)c], 0));
-        if (y1 <= y0) continue;
-        if ((rc = launchAssemble(&sh[0].ps, sh[0].g, bufs.data(), p0->out.p, p0->copy_stream, y0, y1)) != FTB_OK) return rc;
+        if (r1 <= r0) continue;
+        if ((rc = launchAssemble(&sh[0].ps, sh[0].g, bufs.data(), p0->out.p, p0->copy_stream, r0, r1)) != FTB_OK) return rc;
         if (stats) stats->kernel_launches += 1;
-        CK(p0->copier.begin(static_cast<const char*>(p0->out.p) + (size_t)y0 * rowBytes, static_cast<char*>(out) + (size_t)y0 * rowBytes, (size_t)(y1 - y0) * rowBytes, p0->copy_stream));
+        CK(p0->copier.begin(static_cast<const char*>(p0->out.p) + (size_t)r0 * rowBytes, static_cast<char*>(out) + (size_t)r0 * rowBytes, (size_t)(r1 - r0) * rowBytes, p0->copy_stream));
     }
     CK(p0->copier.finish());
     CK(cudaStreamSynchronize(p0->copy_stream));
@@ -1178,9 +1215,9 @@ int ftb_render(ftb_scene* scene, const ftb_camera* camera, const ftb_render_para
     }
     CK(cudaSetDevice(primary));
     if (dbg && dbg->prim_id) {
-        CK(cudaMemcpyAsync(dbg->prim_id, p0->dbg_prim.p, (size_t)full.n_samples * 4, cudaMemcpyDeviceToHost, p0->stream));
-        if (dbg->sub_id) CK(cudaMemcpyAsync(dbg->sub_id, p0->dbg_sub.p, (size_t)full.n_samples * 4, cudaMemcpyDeviceToHost, p0->stream));
-        if (dbg->t) CK(cudaMemcpyAsync(dbg->t, p0->dbg_t.p, (size_t)full.n_samples * 8, cudaMemcpyDeviceToHost, p0->stream));
+        CK(cudaMemcpyAsync(dbg->prim_id, p0->dbg_prim.p, (size_t)g.n_samples * 4, cudaMemcpyDeviceToHost, p0->stream));
+        if (dbg->sub_id) CK(cudaMemcpyAsync(dbg->sub_id, p0->dbg_sub.p, (size_t)g.n_samples * 4, cudaMemcpyDeviceToHost, p0->stream));
+        if (dbg->t) CK(cudaMemcpyAsync(dbg->t, p0->dbg_t.p, (size_t)g.n_samples * 8, cudaMemcpyDeviceToHost, p0->stream));
     }
     CK(cudaStreamSynchronize(p0->stream));
     if (stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();

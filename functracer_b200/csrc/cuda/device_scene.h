@@ -140,16 +140,16 @@ struct DevScene {
 template <typename R>
 struct DevFrame {
     int mode;  // 0 = camera sample grid, 1 = explicit ray list
-    int gw, gh;  // sample grid (W x H, or (W+1) x (H+1) in corner mode)
+    int gw, gh;  // the whole frame's sample grid (W x H, or (W+1) x (H+1) in corner mode): ray directions and RNG keys
     int spp;              // samples per pixel of the whole frame
     int s_base, s_count;  // this launch renders samples [s_base, s_base + s_count) of every pixel (s_count <= UnitCap)
     int run;              // consecutive samples of one pixel a lane takes at a time (divides s_count)
     unsigned rpp_magic;   // floor(2^32 / (s_count / run)) + 1: q / rpp == __umulhi(q, rpp_magic) for q < 65536
     int bw_log, bh_log;   // the work queue hands out blocks of (1 << bw_log) x (1 << bh_log) pixels (bw <= 8)
     int n_blocks;         // blocks (mode 0) or groups of 32 rays (mode 1) in the queue
-    int tiles_x;
+    int tiles_x;             // 16 x 16 tiles per row of the WINDOW's tile grid, which starts at (wx0, wy0)
     unsigned tiles_x_magic;  // floor(2^32 / tiles_x) + 1: tile / tiles_x == __umulhi(tile, magic); 0 = frame too large for that, divide
-    int n_local_tiles;  // tiles this shard renders
+    int n_local_tiles;  // tiles of the window this shard renders
     int shard_index, shard_count;
     long long n_rays;  // mode 1
     R cam_o[3], cam_k[3], cam_i[3], cam_j[3];
@@ -169,6 +169,10 @@ struct DevFrame {
     unsigned int* tile_counter;
     unsigned int* overflow;
     unsigned long long* stats;  // ST_COUNT slots (stats kernels only)
+    // Last, so that the fields above keep their offsets (and the 16-byte alignment of the camera rows, which the kernels load
+    // as vectors) in the kernel's parameter block.
+    int wx0, wy0, wx1, wy1;  // mode 0: the window [wx0, wx1) x [wy0, wy1) of the sample grid this frame renders (whole frame: 0, 0, gw, gh)
+    int dbg_w;               // mode 0: row width of the debug planes (wx1 - wx0): they hold the window's samples only
 };
 
 // A compiled kernel variant (render_variant.cu, one translation unit per FEAT mask / precision).

@@ -1549,8 +1549,8 @@ __global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) render_
     // bits 0..11 = position in the slot, bits 12..15 = ring slot, bits 16.. = samples left in this lane's run
     int rpos = 0;
     int px = 0, py = 0, sj = 0;      // pixel, sample index within the pixel
-    // Index of the sample in the reference's full-frame ray list (RNG key, debug planes, explicit-ray index).  Variants with
-    // in-path randomness carry it; the others rebuild it from (px, py, sj) in the rare places that want it (two registers).
+    // Index of the sample in the reference's full-frame ray list (RNG key, explicit-ray index), also in a window.  Variants
+    // with in-path randomness carry it (two registers); nothing else needs it.
     constexpr bool kCarryIndex = (FEAT & FT_RNG) != 0;
     unsigned long long sampleIndex = 0;
     bool retire = false;             // a sample of this lane finished in the previous iteration (for the unit's count)
@@ -1612,12 +1612,13 @@ __global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) render_
                         const int ltile = F.tile_order ? __ldg(F.tile_order + tpos) : tpos;  // costliest tiles first
                         const int tile = tileOfLocal(ltile, F.shard_index, F.shard_count);
                         const int sx = (sub & ((1 << bpr_log) - 1)) << F.bw_log, sy = (sub >> bpr_log) << F.bh_log;
+                        // the tile grid is the window's; px / py are whole-frame sample-grid coordinates
                         const int tile_y = F.tiles_x_magic ? (int)__umulhi((unsigned)tile, F.tiles_x_magic) : tile / F.tiles_x;
-                        blk_x0 = (tile - tile_y * F.tiles_x) * FTB_TILE_W + sx;
-                        blk_y0 = tile_y * FTB_TILE_H + sy;
+                        blk_x0 = F.wx0 + (tile - tile_y * F.tiles_x) * FTB_TILE_W + sx;
+                        blk_y0 = F.wy0 + tile_y * FTB_TILE_H + sy;
                         blk_slot0 = ltile * FTB_TILE_PIXELS + sy * FTB_TILE_W + sx;
-                        blk_w = max(1, min(1 << F.bw_log, F.gw - blk_x0));
-                        blk_npix = max(0, min(1 << F.bw_log, F.gw - blk_x0)) * max(0, min(1 << F.bh_log, F.gh - blk_y0));
+                        blk_w = max(1, min(1 << F.bw_log, F.wx1 - blk_x0));
+                        blk_npix = max(0, min(1 << F.bw_log, F.wx1 - blk_x0)) * max(0, min(1 << F.bh_log, F.wy1 - blk_y0));
                     } else {
                         const long long first = (long long)c * 32;
                         blk_slot0 = (int)first;
@@ -1718,7 +1719,7 @@ __global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) render_
                     prim = meta.z;
                     sub = (kind == LEAF_CUBE || kind == LEAF_MESH || kind == LEAF_SOLIDCYL) ? h.sub : ((kind == LEAF_TRIANGLE) ? 0 : meta.w);
                 }
-                const unsigned long long at = F.mode == 0 ? ((unsigned long long)py * (unsigned)F.gw + (unsigned)px) * (unsigned)spp + (unsigned)sj
+                const unsigned long long at = F.mode == 0 ? ((unsigned long long)(unsigned)(py - F.wy0) * (unsigned)F.dbg_w + (unsigned)(px - F.wx0)) * (unsigned)spp + (unsigned)sj
                                                           : (unsigned long long)(unsigned)px;
                 F.dbg_prim[at] = prim;
                 if (F.dbg_sub) F.dbg_sub[at] = sub;

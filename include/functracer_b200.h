@@ -227,7 +227,7 @@ typedef struct ftb_render_params {
 } ftb_render_params;
 
 /* Optional per-primary-sample debug planes (W*H*spp each, sample-major within pixel,
- * pixels row-major), the device analogue of Program.printIntersectionAt (Program.fs:33-49).
+ * pixels row-major; a window's planes hold its own samples only, see ftb_render_window), the device analogue of Program.printIntersectionAt (Program.fs:33-49).
  * prim_id = depth-first index of the PRIMITIVE node instance that produced the nearest hit
  * (-1 = miss); sub_id = face 0..5 for cubes (bottom, top, left, right, front, back;
  * Cube.fs:24), part 0..2 for solidCylinder (top, bottom, sides; Cylinder.fs:29), index into
@@ -314,6 +314,28 @@ int ftb_assemble_device(const ftb_render_params* params, const void* const* d_ti
 int ftb_band_rows(const ftb_render_params* params, int band_index, int band_count, int* y0, int* y1);
 int ftb_assemble_rows_device(const ftb_render_params* params, const void* const* d_tile_buffers,
                              void* d_out, int y0, int y1, void* stream);
+
+/* Windows: the pixel rectangle [x0, x1) x [y0, y1) of the frame that params->width x params->height
+ * describes (0 <= x0 < x1 <= width, 0 <= y0 < y1 <= height; anything else is FTB_ERR_BAD_ARG), e.g. a crop,
+ * a one-pixel probe, or a rectangle of the caller's own tiling of a frame.  A window renders exactly what the
+ * whole frame renders there, bit for bit, in every out_format and precision, debug planes included: its
+ * rays, RNG keys and blend order are the whole frame's.  Only the outputs are packed to the window:
+ *   - out holds (x1-x0)*(y1-y0) pixels, row-major within the window;
+ *   - the debug planes hold (x1-x0)*(y1-y0)*spp entries, sample-major within a pixel, pixels row-major within
+ *     the window; in corner sampling the window's sample grid is the corners [x0, x1] x [y0, y1], so they
+ *     hold (x1-x0+1)*(y1-y0+1) entries.
+ * ftb_render_window takes everything ftb_render takes (n_gpus, pageable or page-locked out, stats).
+ * ftb_render_window_tiles_device takes everything ftb_render_tiles_device takes (shard_index / shard_count,
+ * band_index / band_count) over the window's tiles.  A window's tile buffer IS the tile buffer of a frame of
+ * the window's size: ftb_tile_buffer_bytes, ftb_band_rows, ftb_assemble_device and ftb_assemble_rows_device
+ * called with a copy of params whose width / height are x1-x0 / y1-y0 size it, band it and assemble it.
+ * ftb_render and ftb_render_tiles_device are the window (0, 0, width, height) of these two. */
+int ftb_render_window(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params,
+                      int32_t x0, int32_t y0, int32_t x1, int32_t y1,
+                      void* out, const ftb_debug_out* dbg, ftb_stats* stats);
+int ftb_render_window_tiles_device(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params,
+                                   int32_t x0, int32_t y0, int32_t x1, int32_t y1,
+                                   void* d_tiles, const ftb_debug_out* d_dbg, ftb_stats* stats, void* stream);
 
 /* Device -> host copy of a finished band behind the work already queued on `stream` (current device).
  * A page-locked destination makes the call asynchronous; with a pageable one it returns when that band has

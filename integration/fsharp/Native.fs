@@ -163,6 +163,10 @@ extern int ftb_scene_create(FtbSceneDesc& desc, nativeint& scene)
 extern void ftb_scene_destroy(nativeint scene)
 [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
 extern int ftb_render(nativeint scene, FtbCamera& camera, FtbRenderParams& p, nativeint outPixels, nativeint dbgOrNull, nativeint statsOrNull)
+/// the pixels [x0, x1) x [y0, y1) of the frame p describes, bit-identical to ftb_render there; outPixels and the debug
+/// planes hold the window only ((x1 - x0) * (y1 - y0) pixels, row-major)
+[<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+extern int ftb_render_window(nativeint scene, FtbCamera& camera, FtbRenderParams& p, int x0, int y0, int x1, int y1, nativeint outPixels, nativeint dbgOrNull, nativeint statsOrNull)
 [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
 extern int ftb_shade_rays(nativeint scene, nativeint raysOD, int64 n, FtbRenderParams& p, nativeint outRgb, nativeint dbgOrNull, nativeint statsOrNull)
 
