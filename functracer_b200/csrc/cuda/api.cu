@@ -20,6 +20,7 @@
 #include "bvh_build.h"
 #include "device_scene.h"
 #include "lower.h"
+#include "tiles.h"
 
 namespace ftb {
 
@@ -75,6 +76,41 @@ __global__ void assemble_kernel(TilePtrs bufs, int shard_count, int tiles_x, int
         } else {
             static_cast<uchar4*>(out)[i] = make_uchar4(toByte(r), toByte(g), toByte(b), 255);
         }
+    }
+}
+
+// The blocks of the clear tiles (tiles.h: no primary sample of theirs hits anything, so every sample's colour is exactly zero),
+// one warp per block, written without tracing: the render kernel's fold (render.cuh foldUnit) over all-zero samples - the
+// running sum of the earlier passes, divided by spp on the last - and a miss in every requested debug plane.  With `counting`
+// their samples are added to the primary rays, as the counting render kernel would.  A kernel of its own: the render kernel's
+// code is exactly what it was without clear tiles (an extra path in it changes its register allocation and costs 2-3 %).
+template <typename R>
+__global__ void clear_kernel(const __grid_constant__ DevFrame<R> F, int counting)
+{
+    const int lane = threadIdx.x & 31;
+    const int warps = gridDim.x * (blockDim.x >> 5);
+    for (int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); c < F.n_clear_blocks; c += warps) {
+        int slot0, x0, y0, w, npix;
+        openBlock<R>(F, (unsigned)(F.n_blocks + c), slot0, x0, y0, w, npix);
+        for (int i = lane; i < npix * 3; i += 32) {
+            const int pix = i / 3, ch = i - 3 * pix;
+            const int ly = pix / w;
+            const long long o = 3 * ((long long)slot0 + ly * FTB_TILE_W + (pix - ly * w)) + ch;
+            R acc = F.s_base > 0 ? F.out[o] : R(0);
+            if (F.s_base + F.s_count >= F.spp) acc = acc / (R)F.spp;
+            F.out[o] = acc;
+        }
+        if (F.dbg_prim) {
+            for (int i = lane; i < npix * F.s_count; i += 32) {
+                const int pix = i / F.s_count, s = F.s_base + (i - pix * F.s_count);
+                const int ly = pix / w;
+                const unsigned long long at = ((unsigned long long)(unsigned)(y0 + ly - F.wy0) * (unsigned)F.dbg_w + (unsigned)(x0 + pix - ly * w - F.wx0)) * (unsigned)F.spp + (unsigned)s;
+                F.dbg_prim[at] = -1;
+                if (F.dbg_sub) F.dbg_sub[at] = 0;
+                if (F.dbg_t) F.dbg_t[at] = -1.0;
+            }
+        }
+        if (counting && lane == 0 && npix > 0) atomicAdd(F.stats + ST_PRIMARY, (unsigned long long)npix * (unsigned long long)F.s_count);
     }
 }
 
@@ -259,6 +295,7 @@ struct PerDevice {
     ControlBlock control;
     DevBuf jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order;
     std::vector<int> chunk_first;          // first position in the tile order of every chunk (+ end)
+    std::vector<int> chunk_clear;          // position in the tile order where every chunk's clear tiles start
     cudaStream_t copy_stream = nullptr;    // assembly / D2H of finished bands while later bands render (highest priority)
     std::vector<cudaEvent_t> band_events;
     HostCopier copier;
@@ -545,33 +582,6 @@ int frameGeom(const ftb_render_params* p, FrameGeom& g, const Window* win = null
 
 inline size_t realSize(int precision) { return precision == FTB_PRECISION_FP64_VERIFY ? sizeof(double) : sizeof(float); }
 
-struct V3 { double x, y, z; };
-inline V3 sub(V3 a, V3 b) { return {a.x - b.x, a.y - b.y, a.z - b.z}; }
-inline V3 cross(V3 a, V3 b) { return {a.y * b.z - a.z * b.y, b.x * a.z - b.z * a.x, a.x * b.y - a.y * b.x}; }
-inline V3 normalise(V3 v)
-{
-    double l = std::sqrt(v.x * v.x + v.y * v.y + v.z * v.z);
-    if (l < 0.0000001) return v;
-    double s = 1.0 / l;
-    return {s * v.x, s * v.y, s * v.z};
-}
-
-// ImagePlane.create / fromCamera (Image.fs:48-53, 67-81), evaluated in double on the host: the camera's basis, the image
-// plane's size, the pixel pitch and the centre of the top-left pixel.  resH = frame width, resV = frame height.
-struct CameraBasis { V3 o, k, i, j; double width, height, pw, ph, tlx, tly; };
-CameraBasis cameraBasis(const ftb_camera& c, int resH, int resV)
-{
-    const V3 o = {c.o[0], c.o[1], c.o[2]}, la = {c.look_at[0], c.look_at[1], c.look_at[2]}, up = {c.up[0], c.up[1], c.up[2]};
-    const V3 k = normalise(sub(la, o));
-    const V3 i = normalise(cross(up, k));
-    const V3 j = cross(k, i);
-    const double height = std::tan(c.fov_y_rad / 2.0) * 2.0;
-    const double width = height * c.aspect_ratio;
-    const double ph = height / (double)(resH - 1);  // the reference's swapped axes (Image.fs:71-72)
-    const double pw = width / (double)(resV - 1);
-    return {o, k, i, j, width, height, pw, ph, -width / 2.0 + pw / 2.0, height / 2.0 - ph / 2.0};
-}
-
 // the FP32 kernels receive the narrowed results
 template <typename R>
 void fillCamera(DevFrame<R>& F, const ftb_camera& c, int resH, int resV)
@@ -632,72 +642,39 @@ inline int bandPixelRow(int k, int n, int tiles_y, int height) { return std::min
 // Longest-processing-time-first tile order.  The persistent kernel hands tiles out from an atomic queue; a lane
 // keeps its pixel for all samples and all bounce generations, so the last tiles handed out set the tail.  A
 // static estimate - the projected bounding spheres of the items, weighted by how much work a hit on them
-// causes (CSG programs, reflective surfaces spawn up to recursion_limit more generations) - puts the costly
+// causes (CSG programs, reflective surfaces spawn up to recursion_limit more generations), tiles.h - puts the costly
 // tiles first, so the tail consists of cheap ones.  Ordering cannot change any pixel: tiles are independent.
-// Returns false when every tile has the same estimate (no order needed).
+// Clear tiles (tiles.h: no primary sample hits anything) go last in each chunk, from chunk_clear[k] on: the kernel writes
+// their pixels without tracing.
+// Returns false when every tile has the same estimate and none is clear (no order needed).
 bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render_params& p, const FrameGeom& g, int n_chunks, std::vector<int>& order,
-                      std::vector<int>& chunk_first)
+                      std::vector<int>& chunk_first, std::vector<int>& chunk_clear)
 {
-    const double kPiHalf = 1.5707963267948966;
-    const CameraBasis b = cameraBasis(c, p.width, p.height);
-    std::vector<float> cost((size_t)g.n_tiles, 1.0f);
-    bool any = false;
-    auto range = [&](double a, double z, double r, double& lo, double& hi) {
-        const double d2 = a * a + z * z;
-        if (d2 <= r * r) { lo = -1e300; hi = 1e300; return true; }
-        const double th = std::atan2(a, z), al = std::asin(r / std::sqrt(d2));
-        const double t0 = th - al, t1 = th + al;
-        if (t0 >= kPiHalf || t1 <= -kPiHalf) return false;  // entirely behind the image plane
-        lo = t0 <= -kPiHalf ? -1e300 : std::tan(t0);
-        hi = t1 >= kPiHalf ? 1e300 : std::tan(t1);
-        return true;
-    };
-    for (const Item& it : sc.L.items) {
-        if (it.bound_r < 0) continue;  // unbounded (planes): the same everywhere
-        double w = 1.0;
-        bool reflective = false;
-        auto leafWork = [&](int leaf) {
-            const Leaf& lf = sc.L.leaves[leaf];
-            const Surface& sf = sc.L.surfaces[lf.surface];
-            if (sf.apply_lighting && sf.reflectance > 0.0) reflective = true;
-        };
-        if (it.kind == ITEM_LEAF) leafWork(it.a);
-        else {
-            w = 0.0;
-            for (int q = it.prog_first; q < it.prog_first + it.prog_count; ++q)
-                if (sc.L.ops[q].kind == OP_LEAF) { leafWork(sc.L.ops[q].arg); w += 2.0; }
-        }
-        w *= (1.0 + (double)sc.lights.size());                              // a shaded hit adds one shadow ray per light
-        if (reflective) w *= 1.0 + (double)std::max(0, p.recursion_limit);   // and up to `limit` more generations
-        V3 v = {it.bound_c[0] - b.o.x, it.bound_c[1] - b.o.y, it.bound_c[2] - b.o.z};
-        const double x = v.x * b.i.x + v.y * b.i.y + v.z * b.i.z, y = v.x * b.j.x + v.y * b.j.y + v.z * b.j.z, z = v.x * b.k.x + v.y * b.k.y + v.z * b.k.z;
-        double xl, xh, yl, yh;
-        if (!range(x, z, it.bound_r, xl, xh) || !range(y, z, it.bound_r, yl, yh)) continue;
-        // image-plane coordinates -> sample-grid pixels (rayThroughPixel, Image.fs:83-89), one pixel of slack for jitter,
-        // relative to the window's origin
-        const double px0 = (xl - b.tlx) / b.pw - 1.5 - g.wx0, px1 = (xh - b.tlx) / b.pw + 1.5 - g.wx0;
-        const double py0 = (b.tly - yh) / b.ph - 1.5 - g.wy0, py1 = (b.tly - yl) / b.ph + 1.5 - g.wy0;
-        if (px1 < 0 || py1 < 0 || px0 >= g.ww || py0 >= g.wh) continue;
-        const int tx0 = (int)std::max(0.0, std::floor(px0 / FTB_TILE_W)), tx1 = (int)std::min((double)g.tiles_x - 1, std::floor(px1 / FTB_TILE_W));
-        const int ty0 = (int)std::max(0.0, std::floor(py0 / FTB_TILE_H)), ty1 = (int)std::min((double)g.tiles_y - 1, std::floor(py1 / FTB_TILE_H));
-        for (int ty = ty0; ty <= ty1; ++ty)
-            for (int tx = tx0; tx <= tx1; ++tx) cost[(size_t)ty * g.tiles_x + tx] += (float)w;
-        any = true;
-    }
+    std::vector<float> cost;
+    std::vector<unsigned char> clear;
+    const TileGrid grid = {g.wx0, g.wy0, g.ww, g.wh, g.tiles_x, g.tiles_y};
+    const bool any = estimateTiles(sc.L, (int)sc.lights.size(), c, p.width, p.height, p.recursion_limit, sampleOffsetExtent(p), grid, cost, clear);
     // chunks = bands of tile rows (only used unsharded), see bandFirstRow
     auto tileOf = [&](int l) { return tileOfLocal(l, g.shard_index, g.shard_count); };
     auto chunkOf = [&](int l) { return n_chunks <= 1 ? 0 : bandOfRow(std::min(tileOf(l), g.n_tiles - 1) / g.tiles_x, n_chunks, g.tiles_y); };
+    auto clearOf = [&](int l) { const int t = tileOf(l); return t < g.n_tiles && clear[(size_t)t]; };
     chunk_first.assign((size_t)n_chunks + 1, 0);
-    for (int l = 0; l < g.n_local_tiles; ++l) chunk_first[(size_t)chunkOf(l) + 1]++;
+    int n_clear = 0;
+    for (int l = 0; l < g.n_local_tiles; ++l) { chunk_first[(size_t)chunkOf(l) + 1]++; n_clear += clearOf(l) ? 1 : 0; }
     for (int k = 0; k < n_chunks; ++k) chunk_first[(size_t)k + 1] += chunk_first[(size_t)k];
-    if (!any && n_chunks <= 1) return false;
+    chunk_clear.assign(chunk_first.begin() + 1, chunk_first.end());
+    if (!any && n_clear == 0 && n_chunks <= 1) return false;
     order.resize((size_t)g.n_local_tiles);
     for (int l = 0; l < g.n_local_tiles; ++l) order[l] = l;
     auto costOf = [&](int l) { const int t = tileOf(l); return t < g.n_tiles ? cost[(size_t)t] : 0.0f; };
     std::stable_sort(order.begin(), order.end(), [&](int a, int b) {
         const int ca = chunkOf(a), cb = chunkOf(b);
-        return ca != cb ? ca < cb : costOf(a) > costOf(b);
+        if (ca != cb) return ca < cb;
+        const bool za = clearOf(a), zb = clearOf(b);
+        return za != zb ? zb : costOf(a) > costOf(b);
     });
+    for (int l = 0; l < g.n_local_tiles; ++l)
+        if (clearOf(l)) chunk_clear[(size_t)chunkOf(l)]--;
     return true;
 }
 
@@ -748,15 +725,18 @@ struct Launch {
         CK(pd->jitter.reserve(j.size() * sizeof(R)));
         CK(cudaMemcpyAsync(pd->jitter.p, j.data(), j.size() * sizeof(R), cudaMemcpyHostToDevice, stream));  // pageable source: staged before return
         F.jitter = static_cast<const R*>(pd->jitter.p);
-        // tile order: cached per (camera, frame geometry, window, recursion limit); recomputed + uploaded only when they change.
-        // The order lists the window's local tiles: an order cached for another window would name tiles this one lacks.
-        std::vector<unsigned char> key(sizeof(ftb_camera) + 11 * sizeof(int));
+        // tile order: cached per (camera, frame geometry, window, recursion limit, sample offsets); recomputed + uploaded only
+        // when they change.  The order lists the window's local tiles: an order cached for another window would name tiles this
+        // one lacks.  Which tiles are clear depends on how far the samples stray from their pixel centres.
+        const double offset = sampleOffsetExtent(*p);
+        std::vector<unsigned char> key(sizeof(ftb_camera) + 11 * sizeof(int) + sizeof(double));
         std::memcpy(key.data(), cam, sizeof(ftb_camera));
         const int kk[11] = {p->width, p->height, p->sampling, g.shard_index, g.shard_count, p->recursion_limit, n_chunks, g.wx0, g.wy0, g.ww, g.wh};
         std::memcpy(key.data() + sizeof(ftb_camera), kk, sizeof(kk));
+        std::memcpy(key.data() + sizeof(ftb_camera) + sizeof(kk), &offset, sizeof(offset));
         if (key != pd->order_key) {
             std::vector<int> order;
-            pd->order_valid = computeTileOrder(*sc, *cam, *p, g, n_chunks, order, pd->chunk_first);
+            pd->order_valid = computeTileOrder(*sc, *cam, *p, g, n_chunks, order, pd->chunk_first, pd->chunk_clear);
             if (pd->order_valid) {
                 CK(pd->order.reserve(order.size() * sizeof(int)));
                 CK(cudaMemcpyAsync(pd->order.p, order.data(), order.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
@@ -778,6 +758,7 @@ struct Launch {
         const int first = pd->chunk_first[(size_t)chunk], ntile = pd->chunk_first[(size_t)chunk + 1] - first;
         if (ntile <= 0) return FTB_OK;
         F.tile_order = pd->order_valid ? static_cast<const int*>(pd->order.p) + first : nullptr;
+        const int traced = pd->order_valid ? pd->chunk_clear[(size_t)chunk] - first : ntile;  // the tiles before the clear ones
         const long long warps = (long long)pd->sm_count * 5 * (kBlockThreads / 32);
         const long long pixels = (long long)ntile * FTB_TILE_PIXELS;
         int ppb = 32;
@@ -785,7 +766,8 @@ struct Launch {
         int bw = ppb >= 8 ? 8 : ppb, bh = ppb / bw;
         F.bw_log = bw == 8 ? 3 : (bw == 4 ? 2 : (bw == 2 ? 1 : 0));
         F.bh_log = bh == 4 ? 2 : (bh == 2 ? 1 : 0);
-        F.n_blocks = ntile * (FTB_TILE_PIXELS / ppb);
+        F.n_blocks = traced * (FTB_TILE_PIXELS / ppb);
+        F.n_clear_blocks = (ntile - traced) * (FTB_TILE_PIXELS / ppb);
         for (int s_base = 0; s_base < F.spp; s_base += var->unit_cap) {
             F.s_base = s_base;
             F.s_count = std::min(var->unit_cap, F.spp - s_base);
@@ -802,6 +784,12 @@ struct Launch {
             F.rpp_magic = rpp <= 1 ? 0u : (unsigned)((1ull << 32) / rpp) + 1u;
             CK(pd->control.resetQueue(stream));
             CK(launchKernel(stream));
+            if (F.n_clear_blocks > 0) {
+                const int grid = (int)std::min<long long>((F.n_clear_blocks + 3) / 4, (long long)pd->sm_count * 16);
+                clear_kernel<R><<<grid, 128, 0, stream>>>(F, counting ? 1 : 0);
+                CK(cudaGetLastError());
+                ++launches;
+            }
         }
         return FTB_OK;
     }

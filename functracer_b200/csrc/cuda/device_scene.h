@@ -146,7 +146,7 @@ struct DevFrame {
     int run;              // consecutive samples of one pixel a lane takes at a time (divides s_count)
     unsigned rpp_magic;   // floor(2^32 / (s_count / run)) + 1: q / rpp == __umulhi(q, rpp_magic) for q < 65536
     int bw_log, bh_log;   // the work queue hands out blocks of (1 << bw_log) x (1 << bh_log) pixels (bw <= 8)
-    int n_blocks;         // blocks (mode 0) or groups of 32 rays (mode 1) in the queue
+    int n_blocks;         // blocks (mode 0: of the traced tiles) or groups of 32 rays (mode 1) in the queue
     int tiles_x;             // 16 x 16 tiles per row of the WINDOW's tile grid, which starts at (wx0, wy0)
     unsigned tiles_x_magic;  // floor(2^32 / tiles_x) + 1: tile / tiles_x == __umulhi(tile, magic); 0 = frame too large for that, divide
     int n_local_tiles;  // tiles of the window this shard renders
@@ -173,7 +173,33 @@ struct DevFrame {
     // as vectors) in the kernel's parameter block.
     int wx0, wy0, wx1, wy1;  // mode 0: the window [wx0, wx1) x [wy0, wy1) of the sample grid this frame renders (whole frame: 0, 0, gw, gh)
     int dbg_w;               // mode 0: row width of the debug planes (wx1 - wx0): they hold the window's samples only
+    // mode 0: the clear tiles (tiles.h) are the last ones of tile_order; their blocks, n_blocks ... n_blocks + n_clear_blocks - 1,
+    // are written without tracing by clear_kernel (api.cu), not by the render kernel
+    int n_clear_blocks;
 };
+
+#ifdef __CUDACC__
+// Block c of a mode-0 frame's work queue: its first pixel's slot in the tile buffer, its origin in the whole frame's sample
+// grid, its width and its pixel count (clipped to the window; 0 for a tile the last shard group lacks).
+template <typename R>
+__device__ __forceinline__ void openBlock(const DevFrame<R>& F, unsigned c, int& slot0, int& x0, int& y0, int& w, int& npix)
+{
+    // a 16x16 tile holds 2^(8 - bw_log - bh_log) blocks of (1 << bw_log) x (1 << bh_log) pixels
+    const int bpt_log = 8 - F.bw_log - F.bh_log, bpr_log = 4 - F.bw_log;
+    const int sub = (int)(c & ((1u << bpt_log) - 1u));
+    const int tpos = (int)(c >> bpt_log);
+    const int ltile = F.tile_order ? __ldg(F.tile_order + tpos) : tpos;  // costliest tiles first
+    const int tile = tileOfLocal(ltile, F.shard_index, F.shard_count);
+    const int sx = (sub & ((1 << bpr_log) - 1)) << F.bw_log, sy = (sub >> bpr_log) << F.bh_log;
+    // the tile grid is the window's; px / py are whole-frame sample-grid coordinates
+    const int tile_y = F.tiles_x_magic ? (int)__umulhi((unsigned)tile, F.tiles_x_magic) : tile / F.tiles_x;
+    x0 = F.wx0 + (tile - tile_y * F.tiles_x) * FTB_TILE_W + sx;
+    y0 = F.wy0 + tile_y * FTB_TILE_H + sy;
+    slot0 = ltile * FTB_TILE_PIXELS + sy * FTB_TILE_W + sx;
+    w = max(1, min(1 << F.bw_log, F.wx1 - x0));
+    npix = max(0, min(1 << F.bw_log, F.wx1 - x0)) * max(0, min(1 << F.bh_log, F.wy1 - y0));
+}
+#endif
 
 // A compiled kernel variant (render_variant.cu, one translation unit per FEAT mask / precision).
 template <typename R>

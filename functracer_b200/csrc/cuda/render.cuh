@@ -1605,20 +1605,7 @@ __global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) render_
                     if (c >= (unsigned)F.n_blocks) { exhausted = true; break; }
                     blk_pos = 0;
                     if (F.mode == 0) {
-                        // a 16x16 tile holds 2^(8 - bw_log - bh_log) blocks of (1 << bw_log) x (1 << bh_log) pixels
-                        const int bpt_log = 8 - F.bw_log - F.bh_log, bpr_log = 4 - F.bw_log;
-                        const int sub = (int)(c & ((1u << bpt_log) - 1u));
-                        const int tpos = (int)(c >> bpt_log);
-                        const int ltile = F.tile_order ? __ldg(F.tile_order + tpos) : tpos;  // costliest tiles first
-                        const int tile = tileOfLocal(ltile, F.shard_index, F.shard_count);
-                        const int sx = (sub & ((1 << bpr_log) - 1)) << F.bw_log, sy = (sub >> bpr_log) << F.bh_log;
-                        // the tile grid is the window's; px / py are whole-frame sample-grid coordinates
-                        const int tile_y = F.tiles_x_magic ? (int)__umulhi((unsigned)tile, F.tiles_x_magic) : tile / F.tiles_x;
-                        blk_x0 = F.wx0 + (tile - tile_y * F.tiles_x) * FTB_TILE_W + sx;
-                        blk_y0 = F.wy0 + tile_y * FTB_TILE_H + sy;
-                        blk_slot0 = ltile * FTB_TILE_PIXELS + sy * FTB_TILE_W + sx;
-                        blk_w = max(1, min(1 << F.bw_log, F.wx1 - blk_x0));
-                        blk_npix = max(0, min(1 << F.bw_log, F.wx1 - blk_x0)) * max(0, min(1 << F.bh_log, F.wy1 - blk_y0));
+                        openBlock<R>(F, c, blk_slot0, blk_x0, blk_y0, blk_w, blk_npix);
                     } else {
                         const long long first = (long long)c * 32;
                         blk_slot0 = (int)first;

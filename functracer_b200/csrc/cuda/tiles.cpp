@@ -1,0 +1,161 @@
+// tiles.cpp — see tiles.h.
+#include "tiles.h"
+
+#include <algorithm>
+#include <cmath>
+
+namespace ftb {
+
+V3 normalise(V3 v)
+{
+    double l = std::sqrt(v.x * v.x + v.y * v.y + v.z * v.z);
+    if (l < 0.0000001) return v;
+    double s = 1.0 / l;
+    return {s * v.x, s * v.y, s * v.z};
+}
+
+CameraBasis cameraBasis(const ftb_camera& c, int resH, int resV)
+{
+    const V3 o = {c.o[0], c.o[1], c.o[2]}, la = {c.look_at[0], c.look_at[1], c.look_at[2]}, up = {c.up[0], c.up[1], c.up[2]};
+    const V3 k = normalise(sub(la, o));
+    const V3 i = normalise(cross(up, k));
+    const V3 j = cross(k, i);
+    const double height = std::tan(c.fov_y_rad / 2.0) * 2.0;
+    const double width = height * c.aspect_ratio;
+    const double ph = height / (double)(resH - 1);  // the reference's swapped axes (Image.fs:71-72)
+    const double pw = width / (double)(resV - 1);
+    return {o, k, i, j, width, height, pw, ph, -width / 2.0 + pw / 2.0, height / 2.0 - ph / 2.0};
+}
+
+double sampleOffsetExtent(const ftb_render_params& p)
+{
+    if (p.sampling == FTB_SAMPLING_CORNER) return 0.5;  // CornerSampling.generateRays: (-0.5, +0.5)
+    double e = 0;
+    for (int k = 0; k < 2 * p.spp; ++k) e = std::max(e, std::fabs(p.jitter_xy[k]));
+    return e;
+}
+
+// The kernels trace primary rays in FP32 (the camera basis, pixel pitch and jitter narrowed to float, d = k + jx i + jy j
+// and the leaf transform evaluated in float): a few 1e-7 of the magnitudes involved.  Every margin below is 1e-5 of them.
+constexpr double kRel = 1e-5;
+
+bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int width, int height, int recursion_limit, double offset, const TileGrid& g,
+                   std::vector<float>& cost, std::vector<unsigned char>& clear)
+{
+    const double kPiHalf = 1.5707963267948966;
+    const CameraBasis b = cameraBasis(c, width, height);
+    const size_t n_tiles = (size_t)g.tiles_x * g.tiles_y;
+    cost.assign(n_tiles, 1.0f);
+    clear.assign(n_tiles, 0);
+    const double slack = offset + 0.05;  // pixels: the samples' offsets from their pixel centres and FP32 rounding of the image-plane position
+    const double camR = std::sqrt(dot(b.o, b.o));
+    const double primarySlack = 2e-4 * camR;  // DevFrame::primary_slack
+    auto range = [&](double a, double z, double r, double& lo, double& hi) {
+        const double d2 = a * a + z * z;
+        if (d2 <= r * r) { lo = -1e300; hi = 1e300; return true; }
+        const double th = std::atan2(a, z), al = std::asin(r / std::sqrt(d2));
+        const double t0 = th - al, t1 = th + al;
+        if (t0 >= kPiHalf || t1 <= -kPiHalf) return false;  // entirely behind the image plane
+        lo = t0 <= -kPiHalf ? -1e300 : std::tan(t0);
+        hi = t1 >= kPiHalf ? 1e300 : std::tan(t1);
+        return true;
+    };
+    // Clear tiles need the pinhole camera's rays (depth of field moves their origins) and an orthonormal basis (the projection
+    // below assumes one), and every unbounded item must be a top-level plane: (row . d, row . o + w) = the ray's y in the plane's frame.
+    bool clearable = !c.has_focus && std::isfinite(b.pw) && std::isfinite(b.ph) && b.pw > 0 && b.ph > 0 && std::isfinite(b.tlx) && std::isfinite(b.tly) &&
+                     std::isfinite(camR) && std::fabs(dot(b.i, b.i) - 1) < 1e-9 && std::fabs(dot(b.k, b.k) - 1) < 1e-9 && std::fabs(dot(b.i, b.k)) < 1e-9;
+    struct Plane { V3 row; double w; };
+    std::vector<Plane> planes;
+    std::vector<unsigned char> touched(n_tiles, 0);
+    bool any = false;
+    for (const Item& it : L.items) {
+        if (it.bound_r < 0) {  // unbounded: the same cost everywhere
+            const Leaf* lf = it.kind == ITEM_LEAF ? &L.leaves[(size_t)it.a] : nullptr;
+            if (!lf || lf->kind != LEAF_PLANE) clearable = false;
+            else planes.push_back(lf->identity ? Plane{{0, 1, 0}, 0} : Plane{{lf->w2m[4], lf->w2m[5], lf->w2m[6]}, lf->w2m[7]});
+            continue;
+        }
+        double w = 1.0;
+        bool reflective = false;
+        auto leafWork = [&](int leaf) {
+            const Leaf& lf = L.leaves[leaf];
+            const Surface& sf = L.surfaces[lf.surface];
+            if (sf.apply_lighting && sf.reflectance > 0.0) reflective = true;
+        };
+        if (it.kind == ITEM_LEAF) leafWork(it.a);
+        else {
+            w = 0.0;
+            for (int q = it.prog_first; q < it.prog_first + it.prog_count; ++q)
+                if (L.ops[q].kind == OP_LEAF) { leafWork(L.ops[q].arg); w += 2.0; }
+        }
+        w *= (1.0 + (double)n_lights);                                   // a shaded hit adds one shadow ray per light
+        if (reflective) w *= 1.0 + (double)std::max(0, recursion_limit);  // and up to `limit` more generations
+        const V3 cen = {it.bound_c[0], it.bound_c[1], it.bound_c[2]};
+        const V3 v = sub(cen, b.o);
+        const double x = dot(v, b.i), y = dot(v, b.j), z = dot(v, b.k), oc = std::sqrt(dot(v, v));
+        // The tiles a sphere of radius r can touch, with `pad` pixels of slack: image-plane coordinates -> sample-grid pixels
+        // (rayThroughPixel, Image.fs:83-89), relative to the window's origin.  False: none.
+        int tx0, tx1, ty0, ty1;
+        auto tileRect = [&](double r, double pad) {
+            double xl, xh, yl, yh;
+            if (!range(x, z, r, xl, xh) || !range(y, z, r, yl, yh)) return false;
+            const double px0 = (xl - b.tlx) / b.pw - pad - g.wx0, px1 = (xh - b.tlx) / b.pw + pad - g.wx0;
+            const double py0 = (b.tly - yh) / b.ph - pad - g.wy0, py1 = (b.tly - yl) / b.ph + pad - g.wy0;
+            if (px1 < 0 || py1 < 0 || px0 >= g.ww || py0 >= g.wh) return false;
+            tx0 = (int)std::max(0.0, std::floor(px0 / FTB_TILE_W)); tx1 = (int)std::min((double)g.tiles_x - 1, std::floor(px1 / FTB_TILE_W));
+            ty0 = (int)std::max(0.0, std::floor(py0 / FTB_TILE_H)); ty1 = (int)std::min((double)g.tiles_y - 1, std::floor(py1 / FTB_TILE_H));
+            return true;
+        };
+        // the cost estimate: the item's bound, one pixel of slack for jitter
+        if (tileRect(it.bound_r, 1.5)) {
+            for (int ty = ty0; ty <= ty1; ++ty)
+                for (int tx = tx0; tx <= tx1; ++tx) cost[(size_t)ty * g.tiles_x + tx] += (float)w;
+            any = true;
+        }
+        // the tiles that are not clear: the radius beyond which the kernel's bound test drops the item for every primary ray -
+        // the device's inflated radius (api.cu uploadScene), widened by the 1e-6 |oc|^2 of the general test or by the 8e-6 |oc|^2
+        // and the primary slack of the common-origin table (render.cuh), and by the FP32 rounding of the ray and of the bound's
+        // centre - and the samples' largest offset from their pixel centres
+        const double ri = it.bound_r * 1.002 + 1e-5;
+        const double r = std::sqrt(ri * ri + 2e-5 * oc * oc + 2.0 * oc * primarySlack + primarySlack * primarySlack) + kRel * (oc + camR + std::sqrt(dot(cen, cen)));
+        if (tileRect(r, slack))
+            for (int ty = ty0; ty <= ty1; ++ty)
+                for (int tx = tx0; tx <= tx1; ++tx) touched[(size_t)ty * g.tiles_x + tx] = 1;
+    }
+    if (!clearable) return any;
+    // A plane (y = 0 in its frame, Plane.fs) has no crossing at t >= 0 with a ray whose origin is strictly on one side and whose
+    // direction leads away from it: t = -oy / dy < 0.  Plane.fs answers t = 0 for a ray parallel to it (|dy| < 1e-7) from below
+    // or on it, so |dy| must stay clear of 1e-7 too.  dy is affine in the image-plane position (u, v) of the sample and the tile's
+    // samples lie in a rectangle of (u, v): its corners bound dy over the whole tile.  The offset origin camera + 1e-4 d only
+    // moves further away from the plane.
+    std::vector<double> side(planes.size());
+    for (size_t q = 0; q < planes.size(); ++q) {
+        const Plane& pl = planes[q];
+        const double oy = dot(pl.row, b.o) + pl.w;
+        side[q] = oy > 0 ? 1.0 : -1.0;
+    }
+    for (int ty = 0; ty < g.tiles_y; ++ty)
+        for (int tx = 0; tx < g.tiles_x; ++tx) {
+            const size_t t = (size_t)ty * g.tiles_x + tx;
+            if (touched[t]) continue;
+            const double c0 = g.wx0 + tx * FTB_TILE_W - slack, c1 = g.wx0 + tx * FTB_TILE_W + (FTB_TILE_W - 1) + slack;
+            const double r0 = g.wy0 + ty * FTB_TILE_H - slack, r1 = g.wy0 + ty * FTB_TILE_H + (FTB_TILE_H - 1) + slack;
+            const double us[2] = {b.tlx + c0 * b.pw, b.tlx + c1 * b.pw}, vs[2] = {b.tly - r0 * b.ph, b.tly - r1 * b.ph};
+            // the scale of the rounding errors of d (absolute errors of jx, jy next to |tlx|, |tly|)
+            const double dScale = std::sqrt(1.0 + std::max(us[0] * us[0], us[1] * us[1]) + std::max(vs[0] * vs[0], vs[1] * vs[1])) + std::fabs(b.tlx) + std::fabs(b.tly);
+            bool ok = true;
+            for (size_t q = 0; q < planes.size() && ok; ++q) {
+                const Plane& pl = planes[q];
+                const double n = std::sqrt(dot(pl.row, pl.row));
+                const double oy = dot(pl.row, b.o) + pl.w;
+                ok = side[q] * oy > kRel * (n * (camR + dScale) + std::fabs(pl.w));
+                const double dk = dot(pl.row, b.k), di = dot(pl.row, b.i), dj = dot(pl.row, b.j);
+                for (int a = 0; a < 2 && ok; ++a)
+                    for (int e = 0; e < 2 && ok; ++e) ok = side[q] * (dk + us[a] * di + vs[e] * dj) > 1.0001e-7 + kRel * n * dScale;
+            }
+            clear[t] = ok ? 1 : 0;
+        }
+    return any;
+}
+
+}  // namespace ftb

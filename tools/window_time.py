@@ -30,7 +30,7 @@ def gpu_info():
 def cases(W, H):
     cx, cy = W // 2, H // 2
     return [("ftb_render whole frame", None, False), ("window: whole frame", (0, 0, W, H), False),
-            ("window: centred quarter", (W // 4, H // 4, W // 4 + W // 2, H // 4 + H // 2), False),
+            ("window: centred quarter", (W // 4, H // 4, W // 4 + W // 2, H // 4 + H // 2), False), ("window: top quarter", (0, 0, W, H // 4), False),
             ("window: 8-px stripe", (cx - 4, 0, cx + 4, H), False), ("window: 64x64", (cx - 32, cy - 32, cx + 32, cy + 32), False),
             ("window: 1x1 + debug planes", (cx, cy, cx + 1, cy + 1), True)]
 
