@@ -48,6 +48,9 @@ FTB_DEV float abs_(float x) { return fabsf(x); }
 FTB_DEV double abs_(double x) { return fabs(x); }
 FTB_DEV float floor_(float x) { return floorf(x); }
 FTB_DEV double floor_(double x) { return floor(x); }
+// The next representable number above a finite x >= +0.
+FTB_DEV float nextUp(float x) { return __int_as_float(__float_as_int(x) + 1); }
+FTB_DEV double nextUp(double x) { return __longlong_as_double(__double_as_longlong(x) + 1); }
 // System.Math.Pow semantics that matter to specularShader (Shading.fs:85-87): a negative base with an integral exponent
 // gives +-|x|^y (sign by parity), with a non-integral exponent NaN.  Written out so that the product build can use the
 // hardware exp2/log2 path (-use_fast_math) without losing that quirk.
@@ -1150,8 +1153,12 @@ FTB_DEV HitInfo<R> traceScene(const DevScene<R>& S, const Ray<R>& wr, R limit, b
                 const bool want = ((meshCand >> j) & 1u) && !(any && best.found());
                 const Ray<R> r = toModel<PackedXform<R, FEAT>::value, R>(S, leaf, (meta.x >> 8) & 1, wr);
                 if (want) { cn.add(ST_LEAF0 + LEAF_MESH); if (!((meta.x >> 8) & 1)) cn.add(ST_XFORM); }
+                // The walk keeps hits with t < limit only.  When the winner so far comes later in the enumeration than this mesh,
+                // a triangle at exactly its t must still reach meshHit, which gives the tie to the mesh: the walk then runs with
+                // the next number above best.limit (finite and >= 0: a winner was found).
+                const R lim = (!any && best.found() && bestItem > it) ? nextUp(best.limit) : best.limit;
                 R bt; int btri;
-                packetMesh<R, STATS>(S, __ldg(S.mesh_root + meta.w), r, best.limit, any, want, tracing, wstack, bt, btri, cn);
+                packetMesh<R, STATS>(S, __ldg(S.mesh_root + meta.w), r, lim, any, want, tracing, wstack, bt, btri, cn);
                 if (want && btri >= 0) {
                     if (any) best.block(leaf);  // t < limit held inside the walk
                     else meshHit(best, bestItem, it, leaf, bt, btri);

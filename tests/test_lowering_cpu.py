@@ -61,12 +61,9 @@ extern "C" int ftb_probe_bounds(const ftb_scene_desc* d, int max_items, double* 
     return 0;
 }
 // The host-built mesh index (buildMeshIndexHost, the builder of meshes below 32 768 triangles and the device build's fallback):
-// checks, for every mesh a bspMesh primitive uses, that the walk from its root reaches every triangle slot exactly once, that
-// each child box (FP32, rounded outward, and FP64) contains every vertex below it, that leaves hold 1..7 slots, that the depth
-// fits the traversal stack, and that `seq` ranks the mesh's triangles in BspMesh.intersect's right-before-left order.
-// Returns the number of triangle slots checked, or a negative code naming the first violation.
-#include <cfloat>
-#include <functional>
+// tests/mesh_index_check.h's invariants with leaves of 1..7 slots, and a depth that agrees with the one the lowering reports
+// (api.cu refuses a scene whose index the traversal stack cannot hold).
+#include "%(tests)s/mesh_index_check.h"
 extern "C" long ftb_probe_mesh_index(const ftb_scene_desc* d, int* depth_out)
 {
     ftb::Lowered L;
@@ -74,58 +71,9 @@ extern "C" long ftb_probe_mesh_index(const ftb_scene_desc* d, int* depth_out)
     if (ftb::lower_scene(*d, L, e, true) != 0) return -1;
     std::vector<std::vector<int32_t>> order;
     ftb::enumerateMeshes(*d, L, order);
-    std::vector<int> seen(L.bvh_tri.size(), 0);
-    long checked = 0;
     int maxDepth = 0;
-    for (size_t m = 0; m < L.mesh_root.size(); ++m) {
-        if (!L.mesh_used[m]) continue;
-        std::vector<std::pair<int32_t, int32_t>> bySeq;  // (seq, triangle)
-        // returns the box of everything below `link` in double
-        std::function<int(int32_t, int, double*, double*)> walk = [&](int32_t link, int depth, double* lo, double* hi) -> int {
-            if (depth > maxDepth) maxDepth = depth;
-            for (int k = 0; k < 3; ++k) { lo[k] = DBL_MAX; hi[k] = -DBL_MAX; }
-            if (link < 0) {
-                const int code = ~link, first = code >> 3, count = code & 7;
-                if (count < 1 || first < 0 || (size_t)(first + count) > L.bvh_tri.size()) return -10;
-                for (int s = first; s < first + count; ++s) {
-                    if (seen[(size_t)s]++) return -11;
-                    const int32_t tri = L.bvh_tri[(size_t)s];
-                    if (tri < 0 || tri >= d->n_triangles) return -12;
-                    bySeq.push_back({L.bvh_seq[(size_t)s], tri});
-                    for (int v = 0; v < 3; ++v)
-                        for (int k = 0; k < 3; ++k) {
-                            const double x = d->triangles[9 * (size_t)tri + 3 * v + k];
-                            if (x < lo[k]) lo[k] = x;
-                            if (x > hi[k]) hi[k] = x;
-                        }
-                    ++checked;
-                }
-                return 0;
-            }
-            if ((size_t)link >= L.bvh_nodes.size()) return -13;
-            const ftb::BvhNode& n = L.bvh_nodes[(size_t)link];
-            for (int c = 0; c < 2; ++c) {
-                double clo[3], chi[3];
-                const int rc = walk(n.child[c], depth + 1, clo, chi);
-                if (rc) return rc;
-                for (int k = 0; k < 3; ++k) {
-                    if (!((double)n.lo[c][k] <= clo[k] && (double)n.hi[c][k] >= chi[k])) return -14;  // the FP32 box must contain its subtree
-                    if (!(n.dlo[c][k] <= clo[k] && n.dhi[c][k] >= chi[k])) return -15;                // and so must the FP64 one
-                    if (clo[k] < lo[k]) lo[k] = clo[k];
-                    if (chi[k] > hi[k]) hi[k] = chi[k];
-                }
-            }
-            return 0;
-        };
-        double lo[3], hi[3];
-        const int rc = walk(L.mesh_root[m], 0, lo, hi);
-        if (rc) return rc;
-        std::sort(bySeq.begin(), bySeq.end());
-        if (bySeq.size() != order[m].size()) return -16;
-        for (size_t i = 0; i < bySeq.size(); ++i)
-            if (bySeq[i].first != (int32_t)i || bySeq[i].second != order[m][i]) return -17;  // seq = rank in the reference's enumeration
-    }
-    for (size_t s = 0; s < seen.size(); ++s) if (seen[s] != 1) return -18;
+    const long checked = checkMeshIndex(d, L, order, 7, &maxDepth);
+    if (checked < 0) return checked;
     if (maxDepth != 0 && maxDepth > L.max_bvh_depth + 1) return -19;
     *depth_out = L.max_bvh_depth;
     return checked;
@@ -140,7 +88,7 @@ LARGE_MESH = 32768  # api.cu kLargeMesh
 def probe(tmp_path_factory):
     d = tmp_path_factory.mktemp("lower_probe")
     src, so = os.path.join(str(d), "probe.cpp"), os.path.join(str(d), "libprobe.so")
-    open(src, "w").write(PROBE % dict(csrc=CSRC))
+    open(src, "w").write(PROBE % dict(csrc=CSRC, tests=os.path.dirname(os.path.abspath(__file__))))
     subprocess.check_call(["g++", "-O1", "-std=c++17", "-fPIC", "-shared", "-o", so, src, os.path.join(CSRC, "cuda", "lower.cpp")])
     lib = C.CDLL(so)
     lib.ftb_probe_lower.argtypes = [C.POINTER(abi.SceneDesc), C.POINTER(C.c_uint), C.POINTER(C.c_int), C.c_char_p, C.c_int]
