@@ -20,6 +20,7 @@
 #include "bvh_build.h"
 #include "device_scene.h"
 #include "lower.h"
+#include "clear_boxes.h"
 #include "tiles.h"
 
 namespace ftb {
@@ -644,7 +645,7 @@ inline int bandPixelRow(int k, int n, int tiles_y, int height) { return std::min
 // static estimate - the projected bounding spheres of the items, weighted by how much work a hit on them
 // causes (CSG programs, reflective surfaces spawn up to recursion_limit more generations), tiles.h - puts the costly
 // tiles first, so the tail consists of cheap ones.  Ordering cannot change any pixel: tiles are independent.
-// Clear tiles (tiles.h: no primary sample hits anything) go last in each chunk, from chunk_clear[k] on: the kernel writes
+// Clear tiles (tiles.h: no primary sample hits anything, by the items' spheres and boxes, clear_boxes.h) go last in each chunk, from chunk_clear[k] on: the kernel writes
 // their pixels without tracing.
 // Returns false when every tile has the same estimate and none is clear (no order needed).
 bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render_params& p, const FrameGeom& g, int n_chunks, std::vector<int>& order,
@@ -653,7 +654,8 @@ bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render
     std::vector<float> cost;
     std::vector<unsigned char> clear;
     const TileGrid grid = {g.wx0, g.wy0, g.ww, g.wh, g.tiles_x, g.tiles_y};
-    const bool any = estimateTiles(sc.L, (int)sc.lights.size(), c, p.width, p.height, p.recursion_limit, sampleOffsetExtent(p), grid, cost, clear);
+    const std::vector<ImageRect> boxes = itemBoxRects(sc.L, c, p.width, p.height);
+    const bool any = estimateTiles(sc.L, (int)sc.lights.size(), c, p.width, p.height, p.recursion_limit, sampleOffsetExtent(p), grid, cost, clear, &boxes);
     // chunks = bands of tile rows (only used unsharded), see bandFirstRow
     auto tileOf = [&](int l) { return tileOfLocal(l, g.shard_index, g.shard_count); };
     auto chunkOf = [&](int l) { return n_chunks <= 1 ? 0 : bandOfRow(std::min(tileOf(l), g.n_tiles - 1) / g.tiles_x, n_chunks, g.tiles_y); };

@@ -94,6 +94,44 @@ Sphere boundOfPoints(const M34& m2w, const std::vector<std::array<double, 3>>& p
     return s;
 }
 
+// ||A||_F ||A^-1||_F of the linear parts of a transform and its inverse: at least A's condition number in the 2-norm
+double condition(const M34& a, const M34& inv)
+{
+    double s = 0, t = 0;
+    for (int r = 0; r < 3; ++r)
+        for (int k = 0; k < 3; ++k) { s += a.m[4 * r + k] * a.m[4 * r + k]; t += inv.m[4 * r + k] * inv.m[4 * r + k]; }
+    return std::sqrt(s * t);
+}
+
+// The box [lo, hi] carried to world space by m2w; invalid if not finite.
+ItemBoxes worldBox(const M34& m2w, double cond, const double* lo, const double* hi)
+{
+    WorldBox w;
+    w.cond = cond;
+    for (int i = 0; i < 8; ++i) {
+        const double p[3] = {(i & 1) ? hi[0] : lo[0], (i & 2) ? hi[1] : lo[1], (i & 4) ? hi[2] : lo[2]};
+        for (int r = 0; r < 3; ++r) {
+            w.corner[i][r] = m2w.m[4 * r] * p[0] + m2w.m[4 * r + 1] * p[1] + m2w.m[4 * r + 2] * p[2] + m2w.m[4 * r + 3];
+            if (!std::isfinite(w.corner[i][r])) return ItemBoxes();
+        }
+    }
+    if (!std::isfinite(cond)) return ItemBoxes();
+    ItemBoxes b;
+    b.valid = true;
+    b.boxes.push_back(w);
+    return b;
+}
+
+const ItemBoxes kNoBoxes = {true, {}};  // an item that reports nothing
+
+ItemBoxes join(const ItemBoxes& a, const ItemBoxes& b)
+{
+    if (!a.valid || !b.valid) return ItemBoxes();
+    ItemBoxes j = a;
+    j.boxes.insert(j.boxes.end(), b.boxes.begin(), b.boxes.end());
+    return j;
+}
+
 std::vector<std::array<double, 3>> boxCorners(double x0, double x1, double y0, double y1, double z0, double z1)
 {
     std::vector<std::array<double, 3>> p;
@@ -119,6 +157,7 @@ struct Lowerer {
     std::map<std::vector<double>, int> surfaceIndex;
     std::map<int, int> textureIndex;  // desc texture -> lowered texture
     std::vector<Sphere> leafBound;
+    std::vector<ItemBoxes> leafBox;  // the model-space box of leafBound's points in world space
     std::vector<int> meshDepth;
 
     Lowerer(const ftb_scene_desc& dd, Lowered& ll, std::string& e) : d(dd), L(ll), err(e) {}
@@ -224,13 +263,14 @@ struct Lowerer {
     }
     // Bounding sphere of a mesh's vertices in world space (centre of their box, farthest vertex), straight off the triangle
     // table: two passes, nothing stored (a 355 k-triangle mesh has a million vertices).
-    Sphere boundOfMesh(const M34& w2m, int root)
+    Sphere boundOfMesh(const M34& w2m, int root, ItemBoxes& box)
     {
         M34 m2w;
+        box = ItemBoxes();
         if (!invertAffine(w2m, m2w)) return kUnbounded;
         std::vector<std::pair<int, int>> ranges;
         bspRanges(root, ranges);
-        if (ranges.empty()) return kEmpty;
+        if (ranges.empty()) { box = kNoBoxes; return kEmpty; }
         double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
         auto world = [&](const double* p, double* w) {
             for (int r = 0; r < 3; ++r) w[r] = m2w.m[4 * r] * p[0] + m2w.m[4 * r + 1] * p[1] + m2w.m[4 * r + 2] * p[2] + m2w.m[4 * r + 3];
@@ -253,6 +293,7 @@ struct Lowerer {
             }
         s.r = std::sqrt(r2);
         if (!std::isfinite(s.r) || !std::isfinite(s.c[0]) || !std::isfinite(s.c[1]) || !std::isfinite(s.c[2])) return kUnbounded;
+        box = worldBox(kIdentity, condition(w2m, m2w), lo, hi);  // the vertices' world-space box
         return s;
     }
 
@@ -265,9 +306,19 @@ struct Lowerer {
         std::memcpy(lf.w2m, w2m.m, sizeof(lf.w2m));
         L.leaves.push_back(lf);
         Sphere b = kUnbounded;
+        ItemBoxes box;
         M34 m2w;
-        if (bounded && invertAffine(w2m, m2w)) b = boundOfPoints(m2w, modelPts);
+        if (bounded && invertAffine(w2m, m2w)) {
+            b = boundOfPoints(m2w, modelPts);
+            if (b.r >= 0 && !modelPts.empty()) {
+                double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
+                for (auto& p : modelPts)
+                    for (int r = 0; r < 3; ++r) { lo[r] = std::min(lo[r], p[r]); hi[r] = std::max(hi[r], p[r]); }
+                box = worldBox(m2w, condition(w2m, m2w), lo, hi);
+            }
+        }
         leafBound.push_back(b);
+        leafBox.push_back(box);
         return (int)L.leaves.size() - 1;
     }
 
@@ -304,7 +355,7 @@ struct Lowerer {
             if (L.mesh_used.size() < (size_t)d.n_meshes) L.mesh_used.resize((size_t)d.n_meshes, 0);
             L.mesh_used[n.b] = 1;
             out.push_back(addLeaf(LEAF_MESH, cx, cx.w2m, surface, prim, n.b, {}, false));
-            leafBound.back() = boundOfMesh(cx.w2m, d.meshes[n.b].root);
+            leafBound.back() = boundOfMesh(cx.w2m, d.meshes[n.b].root, leafBox.back());
             L.has_mesh = true;
             break;
         }
@@ -327,7 +378,8 @@ struct Lowerer {
     // (bound = A's) and `intersect A B` (bound = one operand's) that is only right if the bounding operand is closed: an open
     // one (cylinder, cone, square, circle, triangle) crossed once at t < 0 leaves Csg.constructedSolid's inA / inB state
     // true for all t > 0 (Csg.fs:74-94) and the reference then reports the OTHER operand's crossings ahead of the origin.
-    bool emitProgram(int node, Ctx cx, int depth, Sphere& bound, bool& empty, int& lists, bool& casts, bool& closed)
+    // `boxes` follows the same rules as `bound`.
+    bool emitProgram(int node, Ctx cx, int depth, Sphere& bound, ItemBoxes& boxes, bool& empty, int& lists, bool& casts, bool& closed)
     {
         if (!checkNode(node, depth)) return false;
         const ftb_node& n = d.nodes[node];
@@ -336,10 +388,11 @@ struct Lowerer {
             if (n.a == FTB_PRIM_BSPMESH) return fail(FTB_ERR_UNSUPPORTED, "bspMesh as a CSG operand is not supported (meshes emit no t<0 crossings, Triangle.fs:62)");
             std::vector<int> lv;
             if (!primitiveLeaves(n, cx, lv)) return false;
-            bound = kEmpty; empty = true;
+            bound = kEmpty; boxes = kNoBoxes; empty = true;
             for (int l : lv) {
                 L.ops.push_back({OP_LEAF, l});
                 bound = enclose(bound, leafBound[l], empty, false); empty = false;
+                boxes = join(boxes, leafBox[l]);
                 if (L.surfaces[L.leaves[l].surface].apply_lighting) casts = true;
             }
             if (lv.size() != 1) L.ops.push_back({OP_GROUP, (int)lv.size()});
@@ -350,22 +403,23 @@ struct Lowerer {
         case FTB_NODE_TRANSFORM:
             if (n.a < 0 || n.a >= d.n_transforms) return fail(FTB_ERR_BAD_SCENE, "bad transform index");
             { M34 t; std::memcpy(t.m, d.transforms[n.a].w2m, sizeof(t.m)); cx.w2m = mul(t, cx.w2m); }
-            return emitProgram(n.b, cx, depth + 1, bound, empty, lists, casts, closed);
+            return emitProgram(n.b, cx, depth + 1, bound, boxes, empty, lists, casts, closed);
         case FTB_NODE_MATERIAL:
             if (n.a < 0 || n.a >= d.n_materials) return fail(FTB_ERR_BAD_SCENE, "bad material index");
             cx.ops.push_back({n.kind, n.a});
-            return emitProgram(n.b, cx, depth + 1, bound, empty, lists, casts, closed);
+            return emitProgram(n.b, cx, depth + 1, bound, boxes, empty, lists, casts, closed);
         case FTB_NODE_TEXTURE: case FTB_NODE_HUESHIFT: case FTB_NODE_IGNORELIGHT:
             cx.ops.push_back({n.kind, n.a});
-            return emitProgram(n.b, cx, depth + 1, bound, empty, lists, casts, closed);
+            return emitProgram(n.b, cx, depth + 1, bound, boxes, empty, lists, casts, closed);
         case FTB_NODE_GROUP: {
             if (n.b < 0 || n.a < 0 || n.a + n.b > d.n_children) return fail(FTB_ERR_BAD_SCENE, "bad group range");
-            bound = kEmpty; empty = true; lists = 0; closed = true;
+            bound = kEmpty; boxes = kNoBoxes; empty = true; lists = 0; closed = true;
             if (n.b == 0) { L.ops.push_back({OP_EMPTY, 0}); lists = 1; return true; }
             for (int i = 0; i < n.b; ++i) {
-                Sphere b; bool e; int l; bool c = false;
-                if (!emitProgram(d.children[n.a + i], cx, depth + 1, b, e, l, casts, c)) return false;
+                Sphere b; ItemBoxes bx; bool e; int l; bool c = false;
+                if (!emitProgram(d.children[n.a + i], cx, depth + 1, b, bx, e, l, casts, c)) return false;
                 bound = enclose(bound, b, empty, e); empty = empty && e;
+                boxes = join(boxes, bx);
                 lists = std::max(lists, i + l);
                 closed = closed && c;
             }
@@ -373,27 +427,27 @@ struct Lowerer {
             return true;
         }
         case FTB_NODE_UNION: case FTB_NODE_INTERSECT: case FTB_NODE_SUBTRACT: case FTB_NODE_EXCLUDE: {
-            Sphere ba, bb; bool ea, eb; int la, lb; bool ca = false, cb = false;
-            if (!emitProgram(n.a, cx, depth + 1, ba, ea, la, casts, ca)) return false;
-            if (!emitProgram(n.b, cx, depth + 1, bb, eb, lb, casts, cb)) return false;
+            Sphere ba, bb; ItemBoxes xa, xb; bool ea, eb; int la, lb; bool ca = false, cb = false;
+            if (!emitProgram(n.a, cx, depth + 1, ba, xa, ea, la, casts, ca)) return false;
+            if (!emitProgram(n.b, cx, depth + 1, bb, xb, eb, lb, casts, cb)) return false;
             lists = std::max(la, 1 + lb);
             closed = ca && cb;
             switch (n.kind) {
-            case FTB_NODE_UNION: L.ops.push_back({OP_UNION, 0}); bound = enclose(ba, bb, ea, eb); empty = ea && eb; break;
-            case FTB_NODE_EXCLUDE: L.ops.push_back({OP_EXCLUDE, 0}); bound = enclose(ba, bb, ea, eb); empty = ea && eb; break;
+            case FTB_NODE_UNION: L.ops.push_back({OP_UNION, 0}); bound = enclose(ba, bb, ea, eb); boxes = join(xa, xb); empty = ea && eb; break;
+            case FTB_NODE_EXCLUDE: L.ops.push_back({OP_EXCLUDE, 0}); bound = enclose(ba, bb, ea, eb); boxes = join(xa, xb); empty = ea && eb; break;
             case FTB_NODE_SUBTRACT:  // every reported crossing lies inside A's bound - as long as A is closed (see above)
                 L.ops.push_back({OP_SUBTRACT, 0});
-                bound = ca ? ba : kUnbounded; empty = ea;
+                bound = ca ? ba : kUnbounded; boxes = ca ? xa : ItemBoxes(); empty = ea;
                 break;
             default:  // intersect: every reported crossing lies inside both operands' bounds; the bounding operand must be closed
                 L.ops.push_back({OP_INTERSECT, 0});
-                if (ea || eb) { bound = kEmpty; empty = true; }
+                if (ea || eb) { bound = kEmpty; boxes = kNoBoxes; empty = true; }
                 else {
                     const bool useA = ca && ba.r >= 0, useB = cb && bb.r >= 0;
-                    if (useA && useB) bound = (ba.r <= bb.r) ? ba : bb;
-                    else if (useA) bound = ba;
-                    else if (useB) bound = bb;
-                    else bound = kUnbounded;
+                    if (useA && useB) { bound = (ba.r <= bb.r) ? ba : bb; boxes = (ba.r <= bb.r) ? xa : xb; }
+                    else if (useA) { bound = ba; boxes = xa; }
+                    else if (useB) { bound = bb; boxes = xb; }
+                    else { bound = kUnbounded; boxes = ItemBoxes(); }
                     empty = false;
                 }
                 break;
@@ -405,13 +459,14 @@ struct Lowerer {
         }
     }
 
-    void pushItem(int kind, int a, int b, bool casts, const Sphere& bound, bool empty)
+    void pushItem(int kind, int a, int b, bool casts, const Sphere& bound, const ItemBoxes& boxes, bool empty)
     {
         Item it = {};
         it.kind = kind; it.a = a; it.b = b; it.casts_shadow = casts ? 1 : 0;
         Sphere s = empty ? Sphere{{0, 0, 0}, 0.0} : bound;
         it.bound_c[0] = s.c[0]; it.bound_c[1] = s.c[1]; it.bound_c[2] = s.c[2]; it.bound_r = s.r;
         L.items.push_back(it);
+        L.item_boxes.push_back(empty ? kNoBoxes : boxes);
     }
 
     // Top-level walk: everything outside CSG nodes is a flat, ordered list of items.
@@ -425,7 +480,7 @@ struct Lowerer {
             if (!primitiveLeaves(n, cx, lv)) return false;
             for (int l : lv) {
                 L.leaves[l].top_level = 1;
-                pushItem(ITEM_LEAF, l, 0, L.surfaces[L.leaves[l].surface].apply_lighting != 0, leafBound[l], false);
+                pushItem(ITEM_LEAF, l, 0, L.surfaces[L.leaves[l].surface].apply_lighting != 0, leafBound[l], leafBox[l], false);
             }
             return true;
         }
@@ -447,11 +502,11 @@ struct Lowerer {
             return true;
         case FTB_NODE_UNION: case FTB_NODE_INTERSECT: case FTB_NODE_SUBTRACT: case FTB_NODE_EXCLUDE: {
             int first = (int)L.ops.size();
-            Sphere b; bool e = true; int lists = 0; bool casts = false, closed = false;
-            if (!emitProgram(node, cx, depth, b, e, lists, casts, closed)) return false;
+            Sphere b; ItemBoxes bx; bool e = true; int lists = 0; bool casts = false, closed = false;
+            if (!emitProgram(node, cx, depth, b, bx, e, lists, casts, closed)) return false;
             L.max_csg_lists = std::max(L.max_csg_lists, lists);
             const int count = (int)L.ops.size() - first;
-            pushItem(ITEM_CSG, first, count, casts, b, e);
+            pushItem(ITEM_CSG, first, count, casts, b, bx, e);
             L.items.back().prog_first = first; L.items.back().prog_count = count;
             if (count == 3 && L.ops[first].kind == OP_LEAF && L.ops[first + 1].kind == OP_LEAF && L.ops[first + 2].kind >= OP_UNION) {
                 Item& it = L.items.back();

@@ -108,6 +108,19 @@ struct CsgOp {
     int32_t arg;
 };
 
+// A leaf's model-space bounding box carried to world space (a parallelepiped: its 8 transformed corners), and the
+// condition number of the leaf's transform, by which the intersectors' model-space rounding grows on the way to world space.
+struct WorldBox {
+    double corner[8][3];
+    double cond;
+};
+// Boxes whose union holds every crossing an item can report, combined by the rules of its bounding sphere (DESIGN.md §2).
+// valid = false: the item has no such boxes (its sphere is its only bound).  Host-only: tiles.h uses them to find clear tiles.
+struct ItemBoxes {
+    bool valid = false;
+    std::vector<WorldBox> boxes;
+};
+
 // The device-side index over a mesh's triangles.  BspMesh.intersect (BspMesh.fs:67-76) visits every branch
 // whose AABB the ray's line touches, right subtree before left, and Scene.closest then keeps the smallest
 // t >= 0, first in that order on ties.  Which triangle that is does not depend on the shape of the tree,
@@ -133,6 +146,7 @@ struct Lowered {
     std::vector<TexOp> tex_ops;
     std::vector<TexDef> textures;
     std::vector<Item> items;
+    std::vector<ItemBoxes> item_boxes;  // per item
     std::vector<CsgOp> ops;
     int32_t n_prims = 0;
     int32_t max_csg_lists = 0;  // deepest list stack any program needs

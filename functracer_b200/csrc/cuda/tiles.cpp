@@ -40,7 +40,7 @@ double sampleOffsetExtent(const ftb_render_params& p)
 constexpr double kRel = 1e-5;
 
 bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int width, int height, int recursion_limit, double offset, const TileGrid& g,
-                   std::vector<float>& cost, std::vector<unsigned char>& clear)
+                   std::vector<float>& cost, std::vector<unsigned char>& clear, const std::vector<ImageRect>* box_rects)
 {
     const double kPiHalf = 1.5707963267948966;
     const CameraBasis b = cameraBasis(c, width, height);
@@ -68,7 +68,8 @@ bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int widt
     std::vector<Plane> planes;
     std::vector<unsigned char> touched(n_tiles, 0);
     bool any = false;
-    for (const Item& it : L.items) {
+    for (size_t item = 0; item < L.items.size(); ++item) {
+        const Item& it = L.items[item];
         if (it.bound_r < 0) {  // unbounded: the same cost everywhere
             const Leaf* lf = it.kind == ITEM_LEAF ? &L.leaves[(size_t)it.a] : nullptr;
             if (!lf || lf->kind != LEAF_PLANE) clearable = false;
@@ -93,18 +94,22 @@ bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int widt
         const V3 cen = {it.bound_c[0], it.bound_c[1], it.bound_c[2]};
         const V3 v = sub(cen, b.o);
         const double x = dot(v, b.i), y = dot(v, b.j), z = dot(v, b.k), oc = std::sqrt(dot(v, v));
-        // The tiles a sphere of radius r can touch, with `pad` pixels of slack: image-plane coordinates -> sample-grid pixels
-        // (rayThroughPixel, Image.fs:83-89), relative to the window's origin.  False: none.
+        // The tiles that the image-plane rectangle [xl, xh] x [yl, yh] touches, with `pad` pixels of slack: image-plane
+        // coordinates -> sample-grid pixels (rayThroughPixel, Image.fs:83-89), relative to the window's origin.  False: none.
         int tx0, tx1, ty0, ty1;
-        auto tileRect = [&](double r, double pad) {
-            double xl, xh, yl, yh;
-            if (!range(x, z, r, xl, xh) || !range(y, z, r, yl, yh)) return false;
+        auto tilesOf = [&](double xl, double xh, double yl, double yh, double pad) {
+            if (xl > xh || yl > yh) return false;
             const double px0 = (xl - b.tlx) / b.pw - pad - g.wx0, px1 = (xh - b.tlx) / b.pw + pad - g.wx0;
             const double py0 = (b.tly - yh) / b.ph - pad - g.wy0, py1 = (b.tly - yl) / b.ph + pad - g.wy0;
             if (px1 < 0 || py1 < 0 || px0 >= g.ww || py0 >= g.wh) return false;
             tx0 = (int)std::max(0.0, std::floor(px0 / FTB_TILE_W)); tx1 = (int)std::min((double)g.tiles_x - 1, std::floor(px1 / FTB_TILE_W));
             ty0 = (int)std::max(0.0, std::floor(py0 / FTB_TILE_H)); ty1 = (int)std::min((double)g.tiles_y - 1, std::floor(py1 / FTB_TILE_H));
             return true;
+        };
+        // ... and those a sphere of radius r can touch
+        auto tileRect = [&](double r, double pad) {
+            double xl, xh, yl, yh;
+            return range(x, z, r, xl, xh) && range(y, z, r, yl, yh) && tilesOf(xl, xh, yl, yh, pad);
         };
         // the cost estimate: the item's bound, one pixel of slack for jitter
         if (tileRect(it.bound_r, 1.5)) {
@@ -118,9 +123,15 @@ bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int widt
         // centre - and the samples' largest offset from their pixel centres
         const double ri = it.bound_r * 1.002 + 1e-5;
         const double r = std::sqrt(ri * ri + 2e-5 * oc * oc + 2.0 * oc * primarySlack + primarySlack * primarySlack) + kRel * (oc + camR + std::sqrt(dot(cen, cen)));
-        if (tileRect(r, slack))
-            for (int ty = ty0; ty <= ty1; ++ty)
-                for (int tx = tx0; tx <= tx1; ++tx) touched[(size_t)ty * g.tiles_x + tx] = 1;
+        if (!tileRect(r, slack)) continue;
+        if (box_rects && (*box_rects)[item].valid) {  // and that the item's boxes leave traced
+            const ImageRect& q = (*box_rects)[item];
+            const int sx0 = tx0, sx1 = tx1, sy0 = ty0, sy1 = ty1;
+            if (!tilesOf(q.xl, q.xh, q.yl, q.yh, slack)) continue;
+            tx0 = std::max(tx0, sx0); tx1 = std::min(tx1, sx1); ty0 = std::max(ty0, sy0); ty1 = std::min(ty1, sy1);
+        }
+        for (int ty = ty0; ty <= ty1; ++ty)
+            for (int tx = tx0; tx <= tx1; ++tx) touched[(size_t)ty * g.tiles_x + tx] = 1;
     }
     if (!clearable) return any;
     // A plane (y = 0 in its frame, Plane.fs) has no crossing at t >= 0 with a ray whose origin is strictly on one side and whose

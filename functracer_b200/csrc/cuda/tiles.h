@@ -23,6 +23,10 @@ CameraBasis cameraBasis(const ftb_camera& c, int resH, int resV);
 // The window's tile grid: its origin and size in the whole frame's sample grid, and its tiles.
 struct TileGrid { int wx0, wy0, ww, wh, tiles_x, tiles_y; };
 
+// A rectangle of the image plane, in the coordinates of d = k + x i + y j (x to the right, y up), outside which no primary ray
+// has a crossing with an item at any t (clear_boxes.h).  valid = false: the item has none.  xl > xh: it has no crossings.
+struct ImageRect { bool valid; double xl, xh, yl, yh; };
+
 // The largest distance, in pixels along either axis, of a primary sample from its pixel's centre: the largest |jitter_xy|,
 // 0.5 in corner sampling.
 double sampleOffsetExtent(const ftb_render_params& p);
@@ -33,7 +37,9 @@ double sampleOffsetExtent(const ftb_render_params& p);
 //              touched, and every unbounded item is a top-level plane that all of the tile's rays leave behind.  Such a
 //              sample's colour is exactly zero.  Never set with depth of field or an unbounded item of another kind.
 // `offset` = sampleOffsetExtent.  Returns false when no bounded item touches the window (every cost is 1).
+// box_rects (per item, clear_boxes.h), when given: an item whose valid rectangle, widened by the samples' pixel slack, misses
+// a tile does not keep that tile from being clear even where its sphere is touched.  The costs use the spheres only.
 bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int width, int height, int recursion_limit, double offset, const TileGrid& g,
-                   std::vector<float>& cost, std::vector<unsigned char>& clear);
+                   std::vector<float>& cost, std::vector<unsigned char>& clear, const std::vector<ImageRect>* box_rects = nullptr);
 
 }  // namespace ftb
