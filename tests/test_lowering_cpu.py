@@ -129,8 +129,8 @@ def pick(need, variants):
     return v
 
 
-def lowered(probe, text):
-    sc = frontend.ParsedScene(text, scenes.asset_dir())
+def lowered(probe, text, assets=None):
+    sc = frontend.ParsedScene(text, assets or scenes.asset_dir())
     feats, counts, err = C.c_uint(0), (C.c_int * 4)(), C.create_string_buffer(256)
     rc = probe.ftb_probe_lower(sc.desc_ptr, C.byref(feats), counts, err, 256)
     assert rc == 0, err.value
