@@ -21,6 +21,7 @@
 #include "device_scene.h"
 #include "lower.h"
 #include "clear_boxes.h"
+#include "lit_tiles.h"
 #include "tiles.h"
 
 namespace ftb {
@@ -294,7 +295,7 @@ struct PerDevice {
     cudaStream_t stream = nullptr;  // owned; used by the host-buffer entry points
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, done = nullptr;
     ControlBlock control;
-    DevBuf jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order;
+    DevBuf jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order, lit;
     std::vector<int> chunk_first;          // first position in the tile order of every chunk (+ end)
     std::vector<int> chunk_clear;          // position in the tile order where every chunk's clear tiles start
     cudaStream_t copy_stream = nullptr;    // assembly / D2H of finished bands while later bands render (highest priority)
@@ -302,6 +303,7 @@ struct PerDevice {
     HostCopier copier;
     std::vector<unsigned char> order_key;  // what the cached tile order was computed for
     bool order_valid = false;
+    int lit_leaf = -1;  // the cached lit-tile mask's ground leaf (in `lit`); -1: no tile is lit
     std::vector<DevBuf> peer_tiles;  // on the gather device: one per remote shard
 
     PerDevice() = default;
@@ -317,7 +319,7 @@ struct PerDevice {
             if (stream) cudaStreamSynchronize(stream);
             if (copy_stream) cudaStreamSynchronize(copy_stream);
             f32.release(); f64.release();
-            for (DevBuf* b : {&control.buf, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order}) b->release();
+            for (DevBuf* b : {&control.buf, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order, &lit}) b->release();
             for (DevBuf& b : peer_tiles) b.release();
             if (ev0) cudaEventDestroy(ev0);
             if (ev1) cudaEventDestroy(ev1);
@@ -647,15 +649,17 @@ inline int bandPixelRow(int k, int n, int tiles_y, int height) { return std::min
 // tiles first, so the tail consists of cheap ones.  Ordering cannot change any pixel: tiles are independent.
 // Clear tiles (tiles.h: no primary sample hits anything, by the items' spheres and boxes, clear_boxes.h) go last in each chunk, from chunk_clear[k] on: the kernel writes
 // their pixels without tracing.
+// lit / lit_leaf: the window's lit ground tiles (lit_tiles.h), indexed by the window's tile, not the shard's.
 // Returns false when every tile has the same estimate and none is clear (no order needed).
 bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render_params& p, const FrameGeom& g, int n_chunks, std::vector<int>& order,
-                      std::vector<int>& chunk_first, std::vector<int>& chunk_clear)
+                      std::vector<int>& chunk_first, std::vector<int>& chunk_clear, std::vector<unsigned char>& lit, int& lit_leaf)
 {
     std::vector<float> cost;
     std::vector<unsigned char> clear;
     const TileGrid grid = {g.wx0, g.wy0, g.ww, g.wh, g.tiles_x, g.tiles_y};
     const std::vector<ImageRect> boxes = itemBoxRects(sc.L, c, p.width, p.height);
     const bool any = estimateTiles(sc.L, (int)sc.lights.size(), c, p.width, p.height, p.recursion_limit, sampleOffsetExtent(p), grid, cost, clear, &boxes);
+    lit_leaf = litTiles(sc.L, sc.lights.data(), (int)sc.lights.size(), c, p.width, p.height, sampleOffsetExtent(p), grid, lit);
     // chunks = bands of tile rows (only used unsharded), see bandFirstRow
     auto tileOf = [&](int l) { return tileOfLocal(l, g.shard_index, g.shard_count); };
     auto chunkOf = [&](int l) { return n_chunks <= 1 ? 0 : bandOfRow(std::min(tileOf(l), g.n_tiles - 1) / g.tiles_x, n_chunks, g.tiles_y); };
@@ -738,14 +742,21 @@ struct Launch {
         std::memcpy(key.data() + sizeof(ftb_camera) + sizeof(kk), &offset, sizeof(offset));
         if (key != pd->order_key) {
             std::vector<int> order;
-            pd->order_valid = computeTileOrder(*sc, *cam, *p, g, n_chunks, order, pd->chunk_first, pd->chunk_clear);
+            std::vector<unsigned char> lit;
+            pd->order_valid = computeTileOrder(*sc, *cam, *p, g, n_chunks, order, pd->chunk_first, pd->chunk_clear, lit, pd->lit_leaf);
             if (pd->order_valid) {
                 CK(pd->order.reserve(order.size() * sizeof(int)));
                 CK(cudaMemcpyAsync(pd->order.p, order.data(), order.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
-                CK(cudaStreamSynchronize(stream));  // `order` is a pageable local
             }
+            if (pd->lit_leaf >= 0) {
+                CK(pd->lit.reserve(lit.size()));
+                CK(cudaMemcpyAsync(pd->lit.p, lit.data(), lit.size(), cudaMemcpyHostToDevice, stream));
+            }
+            if (pd->order_valid || pd->lit_leaf >= 0) CK(cudaStreamSynchronize(stream));  // `order` and `lit` are pageable locals
             pd->order_key.swap(key);
         }
+        F.lit_tiles = pd->lit_leaf >= 0 ? static_cast<const unsigned char*>(pd->lit.p) : nullptr;
+        F.lit_leaf = pd->lit_leaf;
         if (stats) CK(cudaEventRecord(pd->ev0, stream));
         return FTB_OK;
     }

@@ -176,6 +176,10 @@ struct DevFrame {
     // mode 0: the clear tiles (tiles.h) are the last ones of tile_order; their blocks, n_blocks ... n_blocks + n_clear_blocks - 1,
     // are written without tracing by clear_kernel (api.cu), not by the render kernel
     int n_clear_blocks;
+    // mode 0, FP32 kernels with top-level planar leaves: one byte per tile of the window's grid (global tile index), bit k =
+    // every primary fragment of the tile on leaf lit_leaf sees directional light k unblocked (lit_tiles.h); nullptr: none
+    const unsigned char* lit_tiles;
+    int lit_leaf;
 };
 
 #ifdef __CUDACC__

@@ -1764,6 +1764,15 @@ __global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) render_
             if constexpr ((FEAT & FT_ROUGH) != 0) needShadow = needShadow && !(f.roughness != R(0) && !(f.shineyness > R(0)));
             if (!needShadow) { intensity = R(1); got = true; continue; }
             const int2 lk = __ldg(S.light_i + li);
+            if constexpr (sizeof(R) == 4 && (FEAT & FT_PLANAR) != 0) {
+                // A primary fragment on the ground of a lit tile (lit_tiles.h): the host proved this directional light's shadow
+                // rays unblocked, so their traced intensity would be 1 exactly ((n - 0) / n for a soft light).  Counted as traced.
+                if (F.lit_tiles && li < 8 && limit == F.recursion_limit && f.planarLeaf == F.lit_leaf && lk.x != FTB_LIGHT_POINT &&
+                    ((__ldg(F.lit_tiles + ((py - F.wy0) / FTB_TILE_H) * F.tiles_x + (px - F.wx0) / FTB_TILE_W) >> li) & 1)) {
+                    cn.add(ST_SHADOW, lk.x == FTB_LIGHT_SOFT_DIRECTIONAL ? (unsigned)lk.y : 1u);
+                    intensity = R(1); got = true; continue;
+                }
+            }
             const R4 la = ldg4<R>(S.light_a + li);
             const Vec<R> lv = mk<R>(la.x, la.y, la.z);
             if (lk.x == FTB_LIGHT_POINT) {  // shadowLightIntensity (Shading.fs:33-42)
