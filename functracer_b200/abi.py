@@ -110,6 +110,13 @@ class DebugOut(C.Structure):
                 ("t", C.POINTER(C.c_double))]
 
 
+class HitOut(C.Structure):
+    """ftb_hit_out: the planes of a nearest-hit query (any pointer may be NULL = not wanted)."""
+    _fields_ = [("t", C.POINTER(C.c_double)), ("prim_id", C.POINTER(C.c_int32)), ("sub_id", C.POINTER(C.c_int32)),
+                ("p", C.POINTER(C.c_double)), ("normal", C.POINTER(C.c_double)), ("colour", C.POINTER(C.c_double)),
+                ("surface", C.POINTER(C.c_double))]
+
+
 class Stats(C.Structure):
     _fields_ = [("primary_rays", C.c_uint64), ("shadow_rays", C.c_uint64), ("reflection_rays", C.c_uint64),
                 ("shaded_hits", C.c_uint64), ("leaf_tests", C.c_uint64 * 10),
@@ -132,4 +139,5 @@ EXPORTS = [
     "ftb_render", "ftb_tile_buffer_bytes", "ftb_render_tiles_device", "ftb_assemble_device",
     "ftb_shade_rays", "ftb_band_rows", "ftb_assemble_rows_device", "ftb_host_copy_begin", "ftb_host_copy_finish",
     "ftb_check_overflow", "ftb_scene_build_info", "ftb_render_window", "ftb_render_window_tiles_device",
+    "ftb_intersect_rays", "ftb_occluded_rays", "ftb_intersect_rays_device", "ftb_occluded_rays_device",
 ]

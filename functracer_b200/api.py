@@ -77,6 +77,17 @@ def lib():
             else:
                 getattr(L, name).argtypes = args
                 getattr(L, name).restype = C.c_int
+        dp, ip = C.POINTER(C.c_double), C.POINTER(C.c_int32)
+        for name, args in (("ftb_intersect_rays", [vp, dp, C.c_int64, C.POINTER(abi.RenderParams), C.POINTER(abi.HitOut), C.POINTER(abi.Stats)]),
+                           ("ftb_occluded_rays", [vp, dp, dp, C.c_int64, C.POINTER(abi.RenderParams), ip, C.POINTER(abi.Stats)]),
+                           ("ftb_intersect_rays_device", [vp, dp, C.c_int64, C.POINTER(abi.RenderParams), C.POINTER(abi.HitOut),
+                                                          C.POINTER(abi.Stats), vp]),
+                           ("ftb_occluded_rays_device", [vp, dp, dp, C.c_int64, C.POINTER(abi.RenderParams), ip, C.POINTER(abi.Stats), vp])):
+            if os.environ.get("FTB_LIB") and not hasattr(L, name):
+                setattr(L, name, None)  # an older A/B build of the same ABI without ray queries
+            else:
+                getattr(L, name).argtypes = args
+                getattr(L, name).restype = C.c_int
         if L.ftb_abi_version() != abi.ABI_VERSION:
             raise RuntimeError("ABI version mismatch: library %d, bindings %d" % (L.ftb_abi_version(), abi.ABI_VERSION))
         _LIB = L
@@ -106,6 +117,11 @@ def make_params(width, height, spp, jitter_xy=None, sampling=abi.SAMPLING_JITTER
 
 
 _OUT_DTYPE = {abi.OUT_RGB_F64: (np.float64, 3), abi.OUT_RGB_F32: (np.float32, 3), abi.OUT_RGBA8: (np.uint8, 4)}
+
+# the planes of a nearest-hit query (ftb_hit_out, in field order): ctypes element, numpy dtype, values per ray
+HIT_PLANES = ("t", "prim", "sub", "p", "normal", "colour", "surface")
+_PLANE_TYPES = ((C.c_double, np.float64, 1), (C.c_int32, np.int32, 1), (C.c_int32, np.int32, 1), (C.c_double, np.float64, 3),
+                (C.c_double, np.float64, 3), (C.c_double, np.float64, 3), (C.c_double, np.float64, 4))
 
 
 class Scene:
@@ -197,6 +213,45 @@ class Scene:
                                     C.byref(dbg) if dbg else None, C.byref(st) if st is not None else None))
         return dict(rgb=rgb, prim=prim, sub=sub, t=t, stats=st)
 
+    # -- Scene.closest / Scene.lightIsBocked (Scene.fs:112-121) on explicit rays, traced exactly as given -------------------
+    def intersect(self, rays_od, planes=HIT_PLANES, stats=None, **kw):
+        """Nearest hit of every ray [n, 6] (o.xyz d.xyz; no slightOffset, d need not be unit length).  Returns {plane: array}
+        for the requested planes of HIT_PLANES: t [n] (-1 on a miss), prim [n], sub [n], p / normal / colour [n, 3],
+        surface [n, 4] (roughness, reflectance, shineyness, apply_lighting).  stats: an abi.Stats to fill (collect_stats=1
+        for the counters).  kw: make_params' precision, collect_stats."""
+        rays = np.ascontiguousarray(rays_od, dtype=np.float64).reshape(-1, 6)
+        n = rays.shape[0]
+        out, hit = _hit_planes(planes, n)
+        _check(_query_entry("ftb_intersect_rays")(self._h, rays.ctypes.data_as(C.POINTER(C.c_double)), n, C.byref(make_params(1, 1, 1, None, **kw)),
+                                                   C.byref(hit), C.byref(stats) if stats is not None else None))
+        return out
+
+    def occluded(self, rays_od, max_t, stats=None, **kw):
+        """Whether a surface with applyLighting crosses each ray [n, 6] at 0 <= t < max_t [n] (+inf allowed).  Returns bool [n]."""
+        rays = np.ascontiguousarray(rays_od, dtype=np.float64).reshape(-1, 6)
+        n = rays.shape[0]
+        mt = np.ascontiguousarray(np.broadcast_to(np.asarray(max_t, dtype=np.float64), (n,)))
+        blocked = np.full(n, -1, dtype=np.int32)
+        dp = C.POINTER(C.c_double)
+        _check(_query_entry("ftb_occluded_rays")(self._h, rays.ctypes.data_as(dp), mt.ctypes.data_as(dp), n, C.byref(make_params(1, 1, 1, None, **kw)),
+                                                  blocked.ctypes.data_as(C.POINTER(C.c_int32)), C.byref(stats) if stats is not None else None))
+        return blocked != 0
+
+    def intersect_device(self, d_rays_ptr, n, d_planes, stream=0, stats=None, **kw):
+        """intersect() on DEVICE memory of the current device, queued on `stream`: d_rays_ptr = n * 6 doubles, d_planes =
+        {plane name of HIT_PLANES: device address} (missing / 0 = not wanted).  Does not synchronise unless stats is given."""
+        hit = abi.HitOut(*[C.cast(C.c_void_p(d_planes.get(name) or None), C.POINTER(ct)) for name, (ct, _, _) in zip(HIT_PLANES, _PLANE_TYPES)])
+        _check(_query_entry("ftb_intersect_rays_device")(self._h, C.cast(C.c_void_p(d_rays_ptr), C.POINTER(C.c_double)), n,
+                                                          C.byref(make_params(1, 1, 1, None, **kw)), C.byref(hit),
+                                                          C.byref(stats) if stats is not None else None, C.c_void_p(stream)))
+
+    def occluded_device(self, d_rays_ptr, d_max_t_ptr, n, d_blocked_ptr, stream=0, stats=None, **kw):
+        """occluded() on DEVICE memory: n * 6 ray doubles, n max_t doubles, n int32 results (1 = blocked)."""
+        dp = C.POINTER(C.c_double)
+        _check(_query_entry("ftb_occluded_rays_device")(self._h, C.cast(C.c_void_p(d_rays_ptr), dp), C.cast(C.c_void_p(d_max_t_ptr), dp), n,
+                                                         C.byref(make_params(1, 1, 1, None, **kw)), C.cast(C.c_void_p(d_blocked_ptr), C.POINTER(C.c_int32)),
+                                                         C.byref(stats) if stats is not None else None, C.c_void_p(stream)))
+
     # -- device-buffer entry points (one process per GPU; pointers are raw device addresses) -----
     def render_tiles_device(self, p, d_tiles_ptr, stream=0, stats=False, camera=None, d_dbg=None, window=None):
         """d_dbg: optional (prim_ptr, sub_ptr, t_ptr) DEVICE addresses of per-sample debug planes (0 / None = not wanted).
@@ -240,6 +295,28 @@ class Scene:
 
     def host_copy_finish(self):
         _check(lib().ftb_host_copy_finish(self._h))
+
+
+def _hit_planes(planes, n):
+    """({name: host array}, abi.HitOut pointing at them) for the requested planes."""
+    unknown = set(planes) - set(HIT_PLANES)
+    if unknown:
+        raise ValueError("unknown planes %s (choose from %s)" % (sorted(unknown), HIT_PLANES))
+    out, ptrs = {}, []
+    for name, (ct, dt, k) in zip(HIT_PLANES, _PLANE_TYPES):
+        if name in planes:
+            out[name] = np.empty((n, k) if k > 1 else n, dtype=dt)
+            ptrs.append(out[name].ctypes.data_as(C.POINTER(ct)))
+        else:
+            ptrs.append(None)
+    return out, abi.HitOut(*ptrs)
+
+
+def _query_entry(name):
+    fn = getattr(lib(), name)
+    if fn is None:
+        raise RuntimeError("%s has no %s (an older build)" % (os.environ.get("FTB_LIB"), name))
+    return fn
 
 
 def _window_entry(name):

@@ -128,19 +128,21 @@ __global__ void widen_kernel(const R* in, double* out, long long n)
 namespace ftb {
 static_assert((unsigned)FT_TABLE == kFeatOriginTable, "lower.h and device_scene.h disagree on the table feature bit");
 // kernel variants compiled by the Makefile (render_variant.cu), listed through -DFTB_FEAT_LIST_F32 / _F64
-#define X(feat) cudaError_t launch_f32_##feat(const DevScene<float>&, const DevFrame<float>&, bool, int, cudaStream_t, int*);
+#define X(feat) cudaError_t launch_f32_##feat(const DevScene<float>&, const DevFrame<float>&, bool, int, cudaStream_t, int*); \
+    cudaError_t query_f32_##feat(const DevScene<float>&, const DevQuery&, bool, int, cudaStream_t, int*);
 FTB_FEAT_LIST_F32
 #undef X
-#define X(feat) cudaError_t launch_f64_##feat(const DevScene<double>&, const DevFrame<double>&, bool, int, cudaStream_t, int*);
+#define X(feat) cudaError_t launch_f64_##feat(const DevScene<double>&, const DevFrame<double>&, bool, int, cudaStream_t, int*); \
+    cudaError_t query_f64_##feat(const DevScene<double>&, const DevQuery&, bool, int, cudaStream_t, int*);
 FTB_FEAT_LIST_F64
 #undef X
 static const Variant<float> kVariantsF32[] = {
-#define X(feat) {(unsigned)(feat), UnitCap<float, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f32_##feat},
+#define X(feat) {(unsigned)(feat), UnitCap<float, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f32_##feat, query_f32_##feat},
     FTB_FEAT_LIST_F32
 #undef X
 };
 static const Variant<double> kVariantsF64[] = {
-#define X(feat) {(unsigned)(feat), UnitCap<double, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f64_##feat},
+#define X(feat) {(unsigned)(feat), UnitCap<double, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f64_##feat, query_f64_##feat},
     FTB_FEAT_LIST_F64
 #undef X
 };
@@ -296,6 +298,7 @@ struct PerDevice {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, done = nullptr;
     ControlBlock control;
     DevBuf jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order, lit;
+    DevBuf query;  // the host-buffer ray queries: max_t and the requested output planes
     std::vector<int> chunk_first;          // first position in the tile order of every chunk (+ end)
     std::vector<int> chunk_clear;          // position in the tile order where every chunk's clear tiles start
     cudaStream_t copy_stream = nullptr;    // assembly / D2H of finished bands while later bands render (highest priority)
@@ -319,7 +322,7 @@ struct PerDevice {
             if (stream) cudaStreamSynchronize(stream);
             if (copy_stream) cudaStreamSynchronize(copy_stream);
             f32.release(); f64.release();
-            for (DevBuf* b : {&control.buf, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order, &lit}) b->release();
+            for (DevBuf* b : {&control.buf, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order, &lit, &query}) b->release();
             for (DevBuf& b : peer_tiles) b.release();
             if (ev0) cudaEventDestroy(ev0);
             if (ev1) cudaEventDestroy(ev1);
@@ -957,6 +960,112 @@ int setUpShard(ftb_scene* sc, const ftb_render_params& p, const Window& win, con
     return FTB_OK;
 }
 
+// ---- ray queries ---------------------------------------------------------------------------------------------------
+// The arguments every query entry point checks before it touches a device.  occlusion: max_t and blocked are required.
+int checkQuery(const ftb_scene* sc, const double* rays, const double* max_t, int64_t n, const ftb_render_params* p, bool occlusion,
+               const int32_t* blocked)
+{
+    if (!sc || !p || n < 0 || (n > 0 && (!rays || (occlusion && (!max_t || !blocked))))) return fail(FTB_ERR_BAD_ARG, "null argument or negative ray count");
+    if (p->precision != FTB_PRECISION_FP32 && p->precision != FTB_PRECISION_FP64_VERIFY) return fail(FTB_ERR_BAD_ARG, "bad precision");
+    if (n > 32LL * 0x7fffffffLL) return fail(FTB_ERR_BAD_ARG, "too many rays");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device: functracer_b200 has no CPU path"); }
+    return FTB_OK;
+}
+
+// The device entry points: one batch of queries (device pointers) queued on `s` on the current device, with the scene's own
+// variant (the one its frames run) and the per-device control block (queue counter, overflow flag, counters).  Nothing here
+// synchronises except the control block's read-back when stats are asked for.
+// occlusion: queries into `blocked` up to max_t, else nearest-hit queries into the planes of `out` (may be null).
+int queryDevice(ftb_scene* sc, bool occlusion, const double* rays, const double* max_t, int64_t n, const ftb_render_params* p,
+                const ftb_hit_out* out, int32_t* blocked, ftb_stats* stats, cudaStream_t s)
+{
+    int rc = checkQuery(sc, rays, max_t, n, p, occlusion, blocked);
+    if (rc != FTB_OK) return rc;
+    if (stats) std::memset(stats, 0, sizeof(*stats));
+    if (n == 0) return FTB_OK;
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    rc = byPrecision(p->precision, [&](auto r) -> int {
+        Launch<decltype(r)> fr;
+        int e = fr.begin(sc, pd, p, sc->L.features, stats && p->collect_stats, nullptr, nullptr);
+        if (e != FTB_OK) return e;
+        CK(pd->control.prepare(fr.counting, s));
+        CK(pd->control.resetQueue(s));
+        DevQuery q;
+        std::memset(&q, 0, sizeof(q));
+        q.rays = rays; q.n = n; q.n_groups = (int)((n + 31) / 32);
+        if (occlusion) {
+            q.max_t = max_t; q.blocked = blocked;
+        } else if (out) {
+            q.t = out->t; q.prim = out->prim_id; q.sub = out->sub_id;
+            q.p = out->p; q.normal = out->normal; q.colour = out->colour; q.surface = out->surface;
+        }
+        q.record = (q.p || q.normal || q.colour || q.surface) ? 1 : 0;
+        Control* c = pd->control.ctl();
+        q.group_counter = &c->tile_counter; q.overflow = &c->overflow; q.stats = c->stats;
+        if (stats) CK(cudaEventRecord(pd->ev0, s));
+        CK(fr.var->query(*fr.scene, q, fr.counting, pd->sm_count, s, &fr.launches));
+        if (stats) { CK(cudaEventRecord(pd->ev1, s)); stats->kernel_launches += fr.launches + 1; }  // + the control-block memset
+        return FTB_OK;
+    });
+    if (rc != FTB_OK) return rc;
+    bool overflow = false;
+    if (stats && (rc = finishStats(sc, pd, stats, s, &overflow)) != FTB_OK) return rc;
+    return overflow ? overflowError() : FTB_OK;
+}
+
+// The host entry points: a thin wrapper around queryDevice.  The rays (and max_t) are uploaded on the scene's stream, the
+// device entry point queues the queries there, the control block is read back (queryDevice does that itself when it fills
+// stats) and only then are the requested planes downloaded: on an overflow the caller's arrays are not written.  Synchronous.
+int queryHost(ftb_scene* sc, bool occlusion, const double* rays, const double* max_t, int64_t n, const ftb_render_params* p,
+              const ftb_hit_out* out, int32_t* blocked, ftb_stats* stats)
+{
+    const auto t0 = std::chrono::steady_clock::now();
+    int rc = checkQuery(sc, rays, max_t, n, p, occlusion, blocked);  // before the uploads read the caller's arrays
+    if (rc != FTB_OK || n == 0) return rc != FTB_OK ? rc : queryDevice(sc, occlusion, rays, max_t, n, p, out, blocked, stats, nullptr);
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    const cudaStream_t s = pd->stream;
+    CK(pd->rays.reserve((size_t)n * 48));
+    CK(cudaMemcpyAsync(pd->rays.p, rays, (size_t)n * 48, cudaMemcpyHostToDevice, s));
+    // every host array of the call with its bytes per ray: max_t (in) and blocked, or the requested planes; one device buffer
+    struct Plane { void* host; size_t per_ray; void* dev; };
+    const ftb_hit_out none = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    const ftb_hit_out& o = out ? *out : none;
+    Plane planes[7] = {{o.t, 8, nullptr}, {o.prim_id, 4, nullptr}, {o.sub_id, 4, nullptr}, {o.p, 24, nullptr},
+                       {o.normal, 24, nullptr}, {o.colour, 24, nullptr}, {o.surface, 32, nullptr}};
+    const int np = occlusion ? 2 : 7;
+    if (occlusion) { planes[0] = {const_cast<double*>(max_t), 8, nullptr}; planes[1] = {blocked, 4, nullptr}; }
+    size_t bytes = 0;
+    for (int k = 0; k < np; ++k) if (planes[k].host) bytes += ((planes[k].per_ray * (size_t)n + 255) & ~(size_t)255);
+    CK(pd->query.reserve(std::max<size_t>(bytes, 1)));
+    size_t at = 0;
+    for (int k = 0; k < np; ++k)
+        if (planes[k].host) { planes[k].dev = static_cast<char*>(pd->query.p) + at; at += ((planes[k].per_ray * (size_t)n + 255) & ~(size_t)255); }
+    const double* d_rays = static_cast<const double*>(pd->rays.p);
+    if (occlusion) {
+        CK(cudaMemcpyAsync(planes[0].dev, max_t, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+        rc = queryDevice(sc, true, d_rays, static_cast<const double*>(planes[0].dev), n, p, nullptr, static_cast<int32_t*>(planes[1].dev), stats, s);
+    } else {
+        const ftb_hit_out d = {static_cast<double*>(planes[0].dev), static_cast<int32_t*>(planes[1].dev), static_cast<int32_t*>(planes[2].dev),
+                               static_cast<double*>(planes[3].dev), static_cast<double*>(planes[4].dev), static_cast<double*>(planes[5].dev),
+                               static_cast<double*>(planes[6].dev)};
+        rc = queryDevice(sc, false, d_rays, nullptr, n, p, &d, nullptr, stats, s);
+    }
+    if (rc == FTB_OK && !stats) {  // with stats queryDevice has read the control block (and reported an overflow) already
+        bool overflow = false;
+        rc = finishStats(sc, pd, nullptr, s, &overflow);
+        if (rc == FTB_OK && overflow) rc = overflowError();
+    }
+    if (rc != FTB_OK) return rc;
+    for (int k = occlusion ? 1 : 0; k < np; ++k)
+        if (planes[k].host) CK(cudaMemcpyAsync(planes[k].host, planes[k].dev, planes[k].per_ray * (size_t)n, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return FTB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1282,6 +1391,29 @@ int ftb_shade_rays(ftb_scene* scene, const double* rays_od, int64_t n, const ftb
     if ((rc = finishStats(scene, pd, stats, s, &overflow)) != FTB_OK) return rc;
     if (stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return overflow ? overflowError() : FTB_OK;
+}
+
+int ftb_intersect_rays(ftb_scene* scene, const double* rays_od, int64_t n, const ftb_render_params* params, const ftb_hit_out* out, ftb_stats* stats)
+{
+    return queryHost(scene, false, rays_od, nullptr, n, params, out, nullptr, stats);
+}
+
+int ftb_occluded_rays(ftb_scene* scene, const double* rays_od, const double* max_t, int64_t n, const ftb_render_params* params, int32_t* blocked,
+                      ftb_stats* stats)
+{
+    return queryHost(scene, true, rays_od, max_t, n, params, nullptr, blocked, stats);
+}
+
+int ftb_intersect_rays_device(ftb_scene* scene, const double* d_rays_od, int64_t n, const ftb_render_params* params, const ftb_hit_out* d_out,
+                              ftb_stats* stats, void* stream)
+{
+    return queryDevice(scene, false, d_rays_od, nullptr, n, params, d_out, nullptr, stats, static_cast<cudaStream_t>(stream));
+}
+
+int ftb_occluded_rays_device(ftb_scene* scene, const double* d_rays_od, const double* d_max_t, int64_t n, const ftb_render_params* params,
+                             int32_t* d_blocked, ftb_stats* stats, void* stream)
+{
+    return queryDevice(scene, true, d_rays_od, d_max_t, n, params, nullptr, d_blocked, stats, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

@@ -182,6 +182,27 @@ struct DevFrame {
     int lit_leaf;
 };
 
+// A batch of ray queries (query_kernel, render.cuh): caller-supplied rays traced exactly as given, nearest hit or occlusion.
+// Every output pointer may be null (not wanted).
+struct DevQuery {
+    const double* rays;   // o.xyz d.xyz per ray
+    const double* max_t;  // occlusion queries: the segment's end per ray; nullptr = nearest-hit queries
+    long long n;          // rays
+    int n_groups;         // groups of 32 rays in the queue
+    int record;           // 1: some plane beyond t / prim / sub is wanted (finalise runs)
+    double* t;
+    int* prim;
+    int* sub;
+    double* p;        // 3 per ray
+    double* normal;   // 3 per ray
+    double* colour;   // 3 per ray
+    double* surface;  // 4 per ray: roughness, reflectance, shineyness, apply_lighting
+    int* blocked;     // occlusion queries
+    unsigned int* group_counter;
+    unsigned int* overflow;
+    unsigned long long* stats;  // ST_COUNT slots (stats kernels only)
+};
+
 #ifdef __CUDACC__
 // Block c of a mode-0 frame's work queue: its first pixel's slot in the tile buffer, its origin in the whole frame's sample
 // grid, its width and its pixel count (clipped to the window; 0 for a tile the last shard group lacks).
@@ -212,6 +233,7 @@ struct Variant {
     int unit_cap;    // UnitCap<R, feat>: samples per pixel one launch covers
     bool has_stats;  // the counting kernel is only compiled into the FT_ALL variants
     cudaError_t (*launch)(const DevScene<R>& s, const DevFrame<R>& f, bool stats, int sm_count, cudaStream_t stream, int* launches);
+    cudaError_t (*query)(const DevScene<R>& s, const DevQuery& q, bool stats, int sm_count, cudaStream_t stream, int* launches);
 };
 
 }  // namespace ftb

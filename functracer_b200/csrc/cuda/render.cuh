@@ -1851,4 +1851,98 @@ cudaError_t launch_render_impl(const DevScene<R>& s, const DevFrame<R>& f, bool 
     return cudaGetLastError();
 }
 
+// ---- ray queries (Scene.closest / Scene.lightIsBocked on caller-supplied rays) -----------------------------------------
+// A kernel of its own, so that render_kernel's code and register allocation stay exactly what they are.  Warps take groups of
+// 32 rays from the per-device queue counter (like mode 1 of render_kernel); each lane traces its ray exactly as given: no
+// slightOffset, no skipped leaf, no common-origin table (arbitrary rays share no origin).  Nearest queries (Q.max_t == nullptr)
+// report the renderer's winner and, with Q.record, the fragment finalise builds for it; occlusion queries report whether some
+// surface with applyLighting crosses the ray at 0 <= t < max_t.
+template <typename R, unsigned FEAT, bool STATS>
+__global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) query_kernel(const __grid_constant__ DevScene<R> S, const __grid_constant__ DevQuery Q)
+{
+    constexpr int WARPS = kBlockThreads / 32;
+    __shared__ int mesh_stack[MeshWalks<FEAT>::kPacket ? WARPS : 1][MeshWalks<FEAT>::kPacket ? kBspStack : 1];  // packetMesh: one walk per warp
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const bool any = Q.max_t != nullptr;
+    Counters<STATS> cn;
+    bool overflow = false;
+    for (;;) {
+        unsigned c = 0;
+        if (lane == 0) c = atomicAdd(Q.group_counter, 1u);
+        c = __shfl_sync(full, c, 0);
+        if (c >= (unsigned)Q.n_groups) break;
+        const long long i = (long long)c * 32 + lane;
+        const bool have = i < Q.n;
+        const unsigned tracing = __ballot_sync(full, have);  // the packet walk's lanes: those holding a ray
+        if (!have) continue;
+        const double* q = Q.rays + 6 * (size_t)i;
+        Ray<R> r;
+        r.o = mk<R>((R)__ldg(q), (R)__ldg(q + 1), (R)__ldg(q + 2));
+        r.d = mk<R>((R)__ldg(q + 3), (R)__ldg(q + 4), (R)__ldg(q + 5));
+        const R limit = any ? (R)__ldg(Q.max_t + i) : inf_<R>();
+        cn.add(any ? ST_SHADOW : ST_PRIMARY);
+        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, r, limit, any, -1, (const typename V4<R>::type*)nullptr, R(0), overflow, cn, tracing,
+                                                        &mesh_stack[MeshWalks<FEAT>::kPacket ? wib : 0][0]);
+        if (any) {
+            Q.blocked[i] = h.leaf >= 0 ? 1 : 0;
+            continue;
+        }
+        // the debug planes' expression (render_kernel), written out again so that render_kernel's code stays as it is
+        int prim = -1, sub = 0;
+        if (h.leaf >= 0) {
+            const int4 meta = __ldg(S.leaf_meta + h.leaf);
+            const int kind = meta.x & 0xff;
+            prim = meta.z;
+            sub = (kind == LEAF_CUBE || kind == LEAF_MESH || kind == LEAF_SOLIDCYL) ? h.sub : ((kind == LEAF_TRIANGLE) ? 0 : meta.w);
+        }
+        if (Q.prim) Q.prim[i] = prim;
+        if (Q.sub) Q.sub[i] = sub;
+        if (Q.t) Q.t[i] = h.leaf >= 0 ? (double)h.t : -1.0;
+        if (Q.record) {  // a kernel parameter: warp-uniform
+            double rec[13];  // p, normal, colour, roughness, reflectance, shineyness, apply_lighting; a miss is all zero
+#pragma unroll
+            for (int k = 0; k < 13; ++k) rec[k] = 0.0;
+            if (h.leaf >= 0) {
+                const Fragment<R> f = finalise<R, FEAT>(S, r, h);
+                rec[0] = f.p.x; rec[1] = f.p.y; rec[2] = f.p.z;
+                rec[3] = f.n.x; rec[4] = f.n.y; rec[5] = f.n.z;
+                rec[6] = f.colour.x; rec[7] = f.colour.y; rec[8] = f.colour.z;
+                rec[9] = f.roughness; rec[10] = f.reflectance; rec[11] = f.shineyness; rec[12] = f.applyLighting ? 1.0 : 0.0;
+            }
+            if (Q.p) { Q.p[3 * i] = rec[0]; Q.p[3 * i + 1] = rec[1]; Q.p[3 * i + 2] = rec[2]; }
+            if (Q.normal) { Q.normal[3 * i] = rec[3]; Q.normal[3 * i + 1] = rec[4]; Q.normal[3 * i + 2] = rec[5]; }
+            if (Q.colour) { Q.colour[3 * i] = rec[6]; Q.colour[3 * i + 1] = rec[7]; Q.colour[3 * i + 2] = rec[8]; }
+            if (Q.surface) { Q.surface[4 * i] = rec[9]; Q.surface[4 * i + 1] = rec[10]; Q.surface[4 * i + 2] = rec[11]; Q.surface[4 * i + 3] = rec[12]; }
+        }
+    }
+    if (overflow) atomicExch(Q.overflow, 1u);
+    if constexpr (STATS) {
+        for (int k = 0; k < ST_COUNT; ++k) {
+            unsigned long long v = cn.get(k);
+            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(full, v, o);
+            if (lane == 0 && v) atomicAdd(Q.stats + k, v);
+        }
+    }
+}
+
+template <typename R, unsigned FEAT, bool WITH_STATS>
+cudaError_t launch_query_impl(const DevScene<R>& s, const DevQuery& q, bool stats, int sm_count, cudaStream_t stream, int* launches)
+{
+    if (!WITH_STATS && stats) return cudaErrorInvalidValue;
+    int per_sm = 0;
+    cudaError_t e = stats ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, query_kernel<R, FEAT, WITH_STATS>, kBlockThreads, 0)
+                          : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, query_kernel<R, FEAT, false>, kBlockThreads, 0);
+    if (e != cudaSuccess) return e;
+    if (per_sm < 1) per_sm = 1;
+    // persistent grid: a multiple of the SM count, never more warps than there are groups of rays
+    const long long want = (long long)sm_count * per_sm, cap = ((long long)q.n_groups + (kBlockThreads / 32) - 1) / (kBlockThreads / 32);
+    int grid = (int)(want < cap ? want : cap);
+    if (grid < 1) grid = 1;
+    if (stats) query_kernel<R, FEAT, WITH_STATS><<<grid, kBlockThreads, 0, stream>>>(s, q);
+    else query_kernel<R, FEAT, false><<<grid, kBlockThreads, 0, stream>>>(s, q);
+    if (launches) ++*launches;
+    return cudaGetLastError();
+}
+
 }  // namespace ftb

@@ -360,6 +360,43 @@ int ftb_shade_rays(ftb_scene* scene, const double* rays_od, int64_t n,
                    const ftb_render_params* params, double* out_rgb,
                    const ftb_debug_out* dbg, ftb_stats* stats);
 
+/* ---- ray queries: Scene.closest (Scene.fs:112-118) and Scene.lightIsBocked (Scene.fs:119-121) ----------------------
+ * n caller-supplied rays (o.xyz, d.xyz doubles per ray, as for ftb_shade_rays), answered by the renderer's own trace.
+ *   - Rays are traced exactly as given: no 1e-4 slightOffset (that belongs to Shading, not to Scene.closest), and d need
+ *     not be unit length; t is in units of d.
+ *   - Nearest: the smallest t >= 0, the first in enumeration order on ties, as the renderer decides it.  The record is the
+ *     fragment the renderer shades (in FP32 a hit on a planar leaf is projected back onto its plane); prim_id / sub_id are
+ *     those of the debug planes of ftb_debug_out.  A miss: t = -1, prim_id = -1, sub_id = 0, every other requested plane 0.
+ *   - Occlusion: blocked[i] = 1 iff some surface with applyLighting crosses ray i at 0 <= t < max_t[i] (max_t may be +inf),
+ *     else 0.  No leaf is skipped: callers offset shadow-ray origins as the reference does (by 1e-4 n).
+ *   - params: only precision and collect_stats are read.  The counting kernel counts nearest queries as primary_rays and
+ *     occlusion queries as shadow_rays.  Calls run on the current device; a multi-GPU caller splits the batch itself.
+ *   - A query uses the scene's per-device control block, as a frame does: one frame or query in flight per scene and device.
+ *   - NULL scene or params, n < 0, or NULL rays / max_t / blocked with n > 0: FTB_ERR_BAD_ARG; n = 0 is OK; no CUDA device:
+ *     FTB_ERR_NO_DEVICE.  A CSG hit-stack overflow: FTB_ERR_HIT_OVERFLOW from the host entry points (which then leave the
+ *     caller's arrays unwritten), from
+ *     ftb_check_overflow after the device entry points (which never synchronise, except to fill stats). */
+typedef struct ftb_hit_out { /* any pointer may be NULL = not wanted; n entries of the given width each */
+    double* t;        /* n    nearest t >= 0 in units of d; -1 on a miss                               */
+    int32_t* prim_id; /* n    as in ftb_debug_out: -1 on a miss                                        */
+    int32_t* sub_id;  /* n    as ftb_debug_out                                                         */
+    double* p;        /* 3n   world hit point, as the shader receives it                               */
+    double* normal;   /* 3n   world normal after normalToWorld and the CSG flip                        */
+    double* colour;   /* 3n   surface colour after textures and hue shifts                             */
+    double* surface;  /* 4n   roughness, reflectance, shineyness, apply_lighting (0 / 1)               */
+} ftb_hit_out;
+
+/* Host buffers; synchronous.  out may be NULL (nothing wanted but stats). */
+int ftb_intersect_rays(ftb_scene* scene, const double* rays_od, int64_t n, const ftb_render_params* params,
+                       const ftb_hit_out* out, ftb_stats* stats);
+int ftb_occluded_rays(ftb_scene* scene, const double* rays_od, const double* max_t, int64_t n,
+                      const ftb_render_params* params, int32_t* blocked, ftb_stats* stats);
+/* The same on device pointers of the current device, queued on stream (a cudaStream_t, 0 = default stream). */
+int ftb_intersect_rays_device(ftb_scene* scene, const double* d_rays_od, int64_t n, const ftb_render_params* params,
+                              const ftb_hit_out* d_out, ftb_stats* stats, void* stream);
+int ftb_occluded_rays_device(ftb_scene* scene, const double* d_rays_od, const double* d_max_t, int64_t n,
+                             const ftb_render_params* params, int32_t* d_blocked, ftb_stats* stats, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -169,6 +169,11 @@ extern int ftb_render(nativeint scene, FtbCamera& camera, FtbRenderParams& p, na
 extern int ftb_render_window(nativeint scene, FtbCamera& camera, FtbRenderParams& p, int x0, int y0, int x1, int y1, nativeint outPixels, nativeint dbgOrNull, nativeint statsOrNull)
 [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
 extern int ftb_shade_rays(nativeint scene, nativeint raysOD, int64 n, FtbRenderParams& p, nativeint outRgb, nativeint dbgOrNull, nativeint statsOrNull)
+/// Scene.closest (Scene.fs:112-118) on n caller-supplied rays (o.xyz d.xyz, traced exactly as given, no slightOffset).
+/// hitOut is the address of a pinned nativeint[7]: the plane pointers of ftb_hit_out in its order (t, prim_id, sub_id, p,
+/// normal, colour, surface; 0n = not wanted)
+[<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+extern int ftb_intersect_rays(nativeint scene, nativeint raysOD, int64 n, FtbRenderParams& p, nativeint hitOut, nativeint statsOrNull)
 
 let lastError () = Marshal.PtrToStringAnsi (ftb_last_error ())
 let check rc = if rc <> 0 then failwithf "functracer_b200 status %d: %s" rc (lastError ())
