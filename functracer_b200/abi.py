@@ -140,4 +140,5 @@ EXPORTS = [
     "ftb_shade_rays", "ftb_band_rows", "ftb_assemble_rows_device", "ftb_host_copy_begin", "ftb_host_copy_finish",
     "ftb_check_overflow", "ftb_scene_build_info", "ftb_render_window", "ftb_render_window_tiles_device",
     "ftb_intersect_rays", "ftb_occluded_rays", "ftb_intersect_rays_device", "ftb_occluded_rays_device",
+    "ftb_intersect_all_rays", "ftb_intersect_all_rays_device",
 ]

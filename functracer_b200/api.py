@@ -82,9 +82,13 @@ def lib():
                            ("ftb_occluded_rays", [vp, dp, dp, C.c_int64, C.POINTER(abi.RenderParams), ip, C.POINTER(abi.Stats)]),
                            ("ftb_intersect_rays_device", [vp, dp, C.c_int64, C.POINTER(abi.RenderParams), C.POINTER(abi.HitOut),
                                                           C.POINTER(abi.Stats), vp]),
-                           ("ftb_occluded_rays_device", [vp, dp, dp, C.c_int64, C.POINTER(abi.RenderParams), ip, C.POINTER(abi.Stats), vp])):
+                           ("ftb_occluded_rays_device", [vp, dp, dp, C.c_int64, C.POINTER(abi.RenderParams), ip, C.POINTER(abi.Stats), vp]),
+                           ("ftb_intersect_all_rays", [vp, dp, C.c_int64, C.c_int32, C.c_double, C.c_double, C.POINTER(abi.RenderParams),
+                                                       C.POINTER(abi.HitOut), ip, C.POINTER(abi.Stats)]),
+                           ("ftb_intersect_all_rays_device", [vp, dp, C.c_int64, C.c_int32, C.c_double, C.c_double, C.POINTER(abi.RenderParams),
+                                                              C.POINTER(abi.HitOut), ip, C.POINTER(abi.Stats), vp])):
             if os.environ.get("FTB_LIB") and not hasattr(L, name):
-                setattr(L, name, None)  # an older A/B build of the same ABI without ray queries
+                setattr(L, name, None)  # an older A/B build of the same ABI without ray (or crossing) queries
             else:
                 getattr(L, name).argtypes = args
                 getattr(L, name).restype = C.c_int
@@ -117,6 +121,8 @@ def make_params(width, height, spp, jitter_xy=None, sampling=abi.SAMPLING_JITTER
 
 
 _OUT_DTYPE = {abi.OUT_RGB_F64: (np.float64, 3), abi.OUT_RGB_F32: (np.float32, 3), abi.OUT_RGBA8: (np.uint8, 4)}
+
+MAX_CROSSINGS = 64  # FTB_MAX_CROSSINGS: the most crossings a crossing query keeps per ray
 
 # the planes of a nearest-hit query (ftb_hit_out, in field order): ctypes element, numpy dtype, values per ray
 HIT_PLANES = ("t", "prim", "sub", "p", "normal", "colour", "surface")
@@ -252,6 +258,32 @@ class Scene:
                                                          C.byref(make_params(1, 1, 1, None, **kw)), C.cast(C.c_void_p(d_blocked_ptr), C.POINTER(C.c_int32)),
                                                          C.byref(stats) if stats is not None else None, C.c_void_p(stream)))
 
+    # -- Scene.intersect (Scene.fs:67-104): every crossing of explicit rays, sorted by t -----------------------------------
+    def intersect_all(self, rays_od, max_hits, t_min=-np.inf, t_max=np.inf, planes=HIT_PLANES, stats=None, **kw):
+        """The crossings of every ray [n, 6] with t_min <= t < t_max, sorted by t (equal t in Scene.intersect's order), traced
+        exactly as given.  Returns (counts [n], {plane: array}): counts may exceed max_hits (1 .. MAX_CROSSINGS), the planes hold
+        the first max_hits crossings of each ray, [n, max_hits] for t / prim / sub, [n, max_hits, 3] for p / normal / colour,
+        [n, max_hits, 4] for surface; unused slots read as a miss (t -1, prim -1, sub 0, 0 elsewhere).  kw: make_params'
+        precision, collect_stats."""
+        rays = np.ascontiguousarray(rays_od, dtype=np.float64).reshape(-1, 6)
+        n = rays.shape[0]
+        out, hit = _hit_planes(planes, n, max_hits)
+        counts = np.empty(n, dtype=np.int32)
+        _check(_query_entry("ftb_intersect_all_rays")(self._h, rays.ctypes.data_as(C.POINTER(C.c_double)), n, max_hits, t_min, t_max,
+                                                       C.byref(make_params(1, 1, 1, None, **kw)), C.byref(hit),
+                                                       counts.ctypes.data_as(C.POINTER(C.c_int32)), C.byref(stats) if stats is not None else None))
+        return counts, out
+
+    def intersect_all_device(self, d_rays_ptr, n, max_hits, d_counts_ptr, d_planes, t_min=-np.inf, t_max=np.inf, stream=0, stats=None, **kw):
+        """intersect_all() on DEVICE memory of the current device, queued on `stream`: d_rays_ptr = n * 6 doubles, d_counts_ptr =
+        n int32, d_planes = {plane name of HIT_PLANES: device address of n * max_hits entries} (missing / 0 = not wanted).
+        Does not synchronise unless stats is given."""
+        hit = abi.HitOut(*[C.cast(C.c_void_p(d_planes.get(name) or None), C.POINTER(ct)) for name, (ct, _, _) in zip(HIT_PLANES, _PLANE_TYPES)])
+        _check(_query_entry("ftb_intersect_all_rays_device")(self._h, C.cast(C.c_void_p(d_rays_ptr), C.POINTER(C.c_double)), n, max_hits, t_min,
+                                                              t_max, C.byref(make_params(1, 1, 1, None, **kw)), C.byref(hit),
+                                                              C.cast(C.c_void_p(d_counts_ptr), C.POINTER(C.c_int32)),
+                                                              C.byref(stats) if stats is not None else None, C.c_void_p(stream)))
+
     # -- device-buffer entry points (one process per GPU; pointers are raw device addresses) -----
     def render_tiles_device(self, p, d_tiles_ptr, stream=0, stats=False, camera=None, d_dbg=None, window=None):
         """d_dbg: optional (prim_ptr, sub_ptr, t_ptr) DEVICE addresses of per-sample debug planes (0 / None = not wanted).
@@ -297,15 +329,15 @@ class Scene:
         _check(lib().ftb_host_copy_finish(self._h))
 
 
-def _hit_planes(planes, n):
-    """({name: host array}, abi.HitOut pointing at them) for the requested planes."""
+def _hit_planes(planes, n, width=None):
+    """({name: host array}, abi.HitOut pointing at them) for the requested planes; width: entries per ray (crossing queries)."""
     unknown = set(planes) - set(HIT_PLANES)
     if unknown:
         raise ValueError("unknown planes %s (choose from %s)" % (sorted(unknown), HIT_PLANES))
     out, ptrs = {}, []
     for name, (ct, dt, k) in zip(HIT_PLANES, _PLANE_TYPES):
         if name in planes:
-            out[name] = np.empty((n, k) if k > 1 else n, dtype=dt)
+            out[name] = np.empty((n,) + ((width,) if width else ()) + ((k,) if k > 1 else ()), dtype=dt)
             ptrs.append(out[name].ctypes.data_as(C.POINTER(ct)))
         else:
             ptrs.append(None)

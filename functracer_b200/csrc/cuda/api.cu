@@ -136,6 +136,11 @@ FTB_FEAT_LIST_F32
     cudaError_t query_f64_##feat(const DevScene<double>&, const DevQuery&, bool, int, cudaStream_t, int*);
 FTB_FEAT_LIST_F64
 #undef X
+// the crossing queries' kernel (crossings.cu): generic FEAT only, one object per precision
+cudaError_t crossings_f32(const DevScene<float>&, const DevCrossings&, bool, int, cudaStream_t, int*);
+cudaError_t crossings_f64(const DevScene<double>&, const DevCrossings&, bool, int, cudaStream_t, int*);
+inline cudaError_t launchCrossings(const DevScene<float>& s, const DevCrossings& q, bool stats, int sm, cudaStream_t st, int* l) { return crossings_f32(s, q, stats, sm, st, l); }
+inline cudaError_t launchCrossings(const DevScene<double>& s, const DevCrossings& q, bool stats, int sm, cudaStream_t st, int* l) { return crossings_f64(s, q, stats, sm, st, l); }
 static const Variant<float> kVariantsF32[] = {
 #define X(feat) {(unsigned)(feat), UnitCap<float, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f32_##feat, query_f32_##feat},
     FTB_FEAT_LIST_F32
@@ -1066,6 +1071,100 @@ int queryHost(ftb_scene* sc, bool occlusion, const double* rays, const double* m
     return FTB_OK;
 }
 
+// ---- crossing queries -----------------------------------------------------------------------------------------------
+// The arguments of a crossing query that the nearest / occlusion queries do not have, then checkQuery's (which ends with the
+// device count): everything a caller can get wrong is reported before any device is looked for.
+int checkCrossings(const ftb_scene* sc, const double* rays, int64_t n, int32_t max_hits, double t_min, double t_max, const ftb_render_params* p,
+                   const int32_t* counts)
+{
+    if (max_hits < 1 || max_hits > FTB_MAX_CROSSINGS) return fail(FTB_ERR_BAD_ARG, "max_hits outside 1 .. FTB_MAX_CROSSINGS");
+    if (t_min != t_min || t_max != t_max || !(t_min < t_max)) return fail(FTB_ERR_BAD_ARG, "t_min or t_max is NaN, or t_min >= t_max");
+    if (n > 0 && !counts) return fail(FTB_ERR_BAD_ARG, "null argument: counts");
+    return checkQuery(sc, rays, nullptr, n, p, false, nullptr);
+}
+
+// The device entry point: one batch of crossing queries (device pointers) queued on `s` on the current device, with the
+// per-device control block, as queryDevice does for the other queries.  out may be null (counts only).
+int crossingsDevice(ftb_scene* sc, const double* rays, int64_t n, int32_t max_hits, double t_min, double t_max, const ftb_render_params* p,
+                    const ftb_hit_out* out, int32_t* counts, ftb_stats* stats, cudaStream_t s)
+{
+    int rc = checkCrossings(sc, rays, n, max_hits, t_min, t_max, p, counts);
+    if (rc != FTB_OK) return rc;
+    if (stats) std::memset(stats, 0, sizeof(*stats));
+    if (n == 0) return FTB_OK;
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    rc = byPrecision(p->precision, [&](auto r) -> int {
+        Launch<decltype(r)> fr;  // the scene on this device and the control block; the variant it picks is not used
+        int e = fr.begin(sc, pd, p, sc->L.features, stats && p->collect_stats, nullptr, nullptr);
+        if (e != FTB_OK) return e;
+        CK(pd->control.prepare(fr.counting, s));
+        CK(pd->control.resetQueue(s));
+        DevCrossings q;
+        std::memset(&q, 0, sizeof(q));
+        q.rays = rays; q.n = n; q.n_groups = (int)((n + 31) / 32);
+        q.max_hits = max_hits; q.t_min = t_min; q.t_max = t_max; q.counts = counts;
+        if (out) {
+            q.t = out->t; q.prim = out->prim_id; q.sub = out->sub_id;
+            q.p = out->p; q.normal = out->normal; q.colour = out->colour; q.surface = out->surface;
+        }
+        q.record = (q.p || q.normal || q.colour || q.surface) ? 1 : 0;
+        Control* c = pd->control.ctl();
+        q.group_counter = &c->tile_counter; q.overflow = &c->overflow; q.stats = c->stats;
+        if (stats) CK(cudaEventRecord(pd->ev0, s));
+        CK(launchCrossings(*fr.scene, q, fr.counting, pd->sm_count, s, &fr.launches));
+        if (stats) { CK(cudaEventRecord(pd->ev1, s)); stats->kernel_launches += fr.launches + 1; }  // + the control-block memset
+        return FTB_OK;
+    });
+    if (rc != FTB_OK) return rc;
+    bool overflow = false;
+    if (stats && (rc = finishStats(sc, pd, stats, s, &overflow)) != FTB_OK) return rc;
+    return overflow ? overflowError() : FTB_OK;
+}
+
+// The host entry point, the pattern of queryHost: upload the rays, queue the device entry, read the control block back, and
+// only then download counts and the requested planes (max_hits entries per ray): on an overflow nothing of the caller's is written.
+int crossingsHost(ftb_scene* sc, const double* rays, int64_t n, int32_t max_hits, double t_min, double t_max, const ftb_render_params* p,
+                  const ftb_hit_out* out, int32_t* counts, ftb_stats* stats)
+{
+    const auto t0 = std::chrono::steady_clock::now();
+    int rc = checkCrossings(sc, rays, n, max_hits, t_min, t_max, p, counts);
+    if (rc != FTB_OK || n == 0) return rc != FTB_OK ? rc : crossingsDevice(sc, rays, n, max_hits, t_min, t_max, p, out, counts, stats, nullptr);
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    const cudaStream_t s = pd->stream;
+    CK(pd->rays.reserve((size_t)n * 48));
+    CK(cudaMemcpyAsync(pd->rays.p, rays, (size_t)n * 48, cudaMemcpyHostToDevice, s));
+    // counts, then the requested planes with their bytes per ray; one device buffer
+    struct Plane { void* host; size_t per_ray; void* dev; };
+    const ftb_hit_out none = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    const ftb_hit_out& o = out ? *out : none;
+    const size_t k = (size_t)max_hits;
+    Plane planes[8] = {{counts, 4, nullptr}, {o.t, 8 * k, nullptr}, {o.prim_id, 4 * k, nullptr}, {o.sub_id, 4 * k, nullptr}, {o.p, 24 * k, nullptr},
+                       {o.normal, 24 * k, nullptr}, {o.colour, 24 * k, nullptr}, {o.surface, 32 * k, nullptr}};
+    size_t bytes = 0;
+    for (const Plane& pl : planes) if (pl.host) bytes += ((pl.per_ray * (size_t)n + 255) & ~(size_t)255);
+    CK(pd->query.reserve(bytes));
+    size_t at = 0;
+    for (Plane& pl : planes)
+        if (pl.host) { pl.dev = static_cast<char*>(pd->query.p) + at; at += ((pl.per_ray * (size_t)n + 255) & ~(size_t)255); }
+    const ftb_hit_out d = {static_cast<double*>(planes[1].dev), static_cast<int32_t*>(planes[2].dev), static_cast<int32_t*>(planes[3].dev),
+                           static_cast<double*>(planes[4].dev), static_cast<double*>(planes[5].dev), static_cast<double*>(planes[6].dev),
+                           static_cast<double*>(planes[7].dev)};
+    rc = crossingsDevice(sc, static_cast<const double*>(pd->rays.p), n, max_hits, t_min, t_max, p, &d, static_cast<int32_t*>(planes[0].dev), stats, s);
+    if (rc == FTB_OK && !stats) {  // with stats crossingsDevice has read the control block (and reported an overflow) already
+        bool overflow = false;
+        rc = finishStats(sc, pd, nullptr, s, &overflow);
+        if (rc == FTB_OK && overflow) rc = overflowError();
+    }
+    if (rc != FTB_OK) return rc;
+    for (const Plane& pl : planes)
+        if (pl.host) CK(cudaMemcpyAsync(pl.host, pl.dev, pl.per_ray * (size_t)n, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return FTB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1414,6 +1513,18 @@ int ftb_occluded_rays_device(ftb_scene* scene, const double* d_rays_od, const do
                              int32_t* d_blocked, ftb_stats* stats, void* stream)
 {
     return queryDevice(scene, true, d_rays_od, d_max_t, n, params, nullptr, d_blocked, stats, static_cast<cudaStream_t>(stream));
+}
+
+int ftb_intersect_all_rays(ftb_scene* scene, const double* rays_od, int64_t n, int32_t max_hits, double t_min, double t_max,
+                           const ftb_render_params* params, const ftb_hit_out* out, int32_t* counts, ftb_stats* stats)
+{
+    return crossingsHost(scene, rays_od, n, max_hits, t_min, t_max, params, out, counts, stats);
+}
+
+int ftb_intersect_all_rays_device(ftb_scene* scene, const double* d_rays_od, int64_t n, int32_t max_hits, double t_min, double t_max,
+                                  const ftb_render_params* params, const ftb_hit_out* d_out, int32_t* d_counts, ftb_stats* stats, void* stream)
+{
+    return crossingsDevice(scene, d_rays_od, n, max_hits, t_min, t_max, params, d_out, d_counts, stats, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

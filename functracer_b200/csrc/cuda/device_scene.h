@@ -203,6 +203,28 @@ struct DevQuery {
     unsigned long long* stats;  // ST_COUNT slots (stats kernels only)
 };
 
+// A batch of crossing queries (crossings_kernel, render.cuh): every crossing of each ray with t_min <= t < t_max, sorted by t,
+// the first max_hits of them kept.  Output planes are max_hits entries wide per ray; every output pointer but counts may be null.
+struct DevCrossings {
+    const double* rays;  // o.xyz d.xyz per ray
+    long long n;         // rays
+    int n_groups;        // groups of 32 rays in the queue
+    int max_hits;        // 1 .. FTB_MAX_CROSSINGS
+    int record;          // 1: some plane beyond t / prim / sub is wanted (finalise runs)
+    double t_min, t_max;
+    int* counts;
+    double* t;
+    int* prim;
+    int* sub;
+    double* p;        // 3 per entry
+    double* normal;   // 3 per entry
+    double* colour;   // 3 per entry
+    double* surface;  // 4 per entry: roughness, reflectance, shineyness, apply_lighting
+    unsigned int* group_counter;
+    unsigned int* overflow;
+    unsigned long long* stats;  // ST_COUNT slots (counting kernel only)
+};
+
 #ifdef __CUDACC__
 // Block c of a mode-0 frame's work queue: its first pixel's slot in the tile buffer, its origin in the whole frame's sample
 // grid, its width and its pixel count (clipped to the window; 0 for a tile the last shard group lacks).

@@ -1945,4 +1945,213 @@ cudaError_t launch_query_impl(const DevScene<R>& s, const DevQuery& q, bool stat
     return cudaGetLastError();
 }
 
+// ---- crossing queries (Scene.intersect on caller-supplied rays, sorted by t) -------------------------------------------
+// One kept crossing: 16 bytes in FP32.  leaf carries the CSG flip in bit 30; sub is HitInfo's (cube face, solidCylinder part,
+// triangle index); rank is a mesh triangle's seq (0 for every other crossing).
+template <typename R>
+struct Crossing {
+    R t;
+    int leaf, sub, rank;
+};
+
+// A lane's kept list: the first `cap` crossings with lo <= t < hi in the order (t, item, rank in the item's own list), and how many
+// there were.  Items arrive in enumeration order and leaf and CSG items report their lists in their own order, so an insertion
+// that passes only entries of strictly larger t keeps that order.  A mesh's crossings arrive in the BVH walk's order: they also
+// pass the entries of the same mesh (= the same leaf) with equal t and a larger seq, so the list does not depend on the walk.
+// The range test is in double on the t the caller receives, so that a narrower range returns exactly the sublist.
+template <typename R>
+struct CrossList {
+    static constexpr bool kIsRay = false;
+    Crossing<R>* e;
+    int cap, n, count;
+    double lo, hi;
+    int cur;  // leaf being intersected (intersectLeaf's sink protocol)
+    FTB_DEV bool before(R t, int leaf, int rank, bool mesh, const Crossing<R>& x) const
+    {
+        return t < x.t || (mesh && t == x.t && (x.leaf & 0x3fffffff) == leaf && rank < x.rank);
+    }
+    FTB_DEV void add(R t, int leaf, int sub, int rank, bool mesh)
+    {
+        const double td = (double)t;
+        if (!(td >= lo && td < hi)) return;
+        ++count;
+        if (n == cap && !before(t, leaf & 0x3fffffff, rank, mesh, e[cap - 1])) return;
+        int j = n < cap ? n : cap - 1;
+        while (j > 0 && before(t, leaf & 0x3fffffff, rank, mesh, e[j - 1])) { e[j] = e[j - 1]; --j; }
+        e[j].t = t; e[j].leaf = leaf; e[j].sub = sub; e[j].rank = rank;
+        if (n < cap) ++n;
+    }
+    FTB_DEV void hit(R t, int hsub) { add(t, cur, hsub, 0, false); }
+    FTB_DEV bool done() const { return false; }
+};
+
+// Every crossing of a mesh (BspMesh.intersect, BspMesh.fs:67-76): one private walk per lane over the device's BVH, which reports
+// each triangle the ray crosses.  Boxes are culled by the interval [0, tmax] only (boxEntry2: a mesh crossing has t > 1e-7).
+template <typename R, bool STATS>
+FTB_DEV void meshCrossings(const DevScene<R>& S, int root, int leaf, const Ray<R>& r, R tmax, CrossList<R>& list, bool& overflow, Counters<STATS>& cn)
+{
+    typedef typename V4<R>::type R4;
+    int stack[kBspStack];
+    int sp = 0;
+    int link = root;
+    const Vec<R> inv = mk<R>(R(1) / r.d.x, R(1) / r.d.y, R(1) / r.d.z);
+    for (;;) {
+        while (link >= 0) {
+            cn.add(ST_BSP_NODES);
+            const R4 b0 = ldg4<R>(S.bvh_node + 4 * link), b1 = ldg4<R>(S.bvh_node + 4 * link + 1), b2 = ldg4<R>(S.bvh_node + 4 * link + 2);
+            const int2 ch = nodeLinks<R>(ldg4<R>(S.bvh_node + 4 * link + 3));
+            R tl, tr;
+            boxEntry2<R>(b0, b1, b2, r.o, inv, tmax, tl, tr);
+            const bool hl = tl < inf_<R>(), hr = tr < inf_<R>();
+            if (hl && hr) {
+                if (sp < kBspStack) stack[sp++] = ch.y; else overflow = true;
+                link = ch.x;
+            } else if (hl || hr) {
+                link = hl ? ch.x : ch.y;
+            } else {
+                link = 0x7fffffff;  // nothing below: pop
+                break;
+            }
+        }
+        if (link < 0) {  // a run of <= 7 triangles
+            const int code = ~link, first = code >> 3, count = code & 7;
+            for (int i = 0; i < count; ++i) {
+                R t; R4 a0, a1;
+                cn.add(ST_TRI_TESTS_IN_MESH);
+                if (triangleT<R>(S.bvh_tris + 3 * (first + i), r, t, a0, a1)) list.add(t, leaf, (int)a1.w, (int)a0.w, true);
+            }
+        }
+        if (sp == 0) break;
+        link = stack[--sp];
+    }
+}
+
+// A kernel of its own (compiled in crossings.cu, generic FEAT only), so that render_kernel and query_kernel stay what they are.
+// Warps take groups of 32 rays from the per-device queue counter, like query_kernel; each lane walks every item in enumeration
+// order and skips only those whose bounding sphere the ray's LINE misses (traceScene's general test and slack; no behind-the-origin
+// cull: crossings at t < 0 count too).  Leaf items report through the leaf intersectors, CSG items (pairs included) through
+// evalCsg on the item's program, mesh items through meshCrossings.  With Q.record (warp-uniform) finalise builds each kept entry.
+template <typename R, unsigned FEAT, bool STATS>
+__global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) crossings_kernel(const __grid_constant__ DevScene<R> S, const __grid_constant__ DevCrossings Q)
+{
+    typedef typename V4<R>::type R4;
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31;
+    Counters<STATS> cn;
+    bool overflow = false;
+    Crossing<R> kept[FTB_MAX_CROSSINGS];
+    HitRec<R> stack[kHitCap];
+    for (;;) {
+        unsigned c = 0;
+        if (lane == 0) c = atomicAdd(Q.group_counter, 1u);
+        c = __shfl_sync(full, c, 0);
+        if (c >= (unsigned)Q.n_groups) break;
+        const long long i = (long long)c * 32 + lane;
+        if (i >= Q.n) continue;
+        const double* q = Q.rays + 6 * (size_t)i;
+        Ray<R> r;
+        r.o = mk<R>((R)__ldg(q), (R)__ldg(q + 1), (R)__ldg(q + 2));
+        r.d = mk<R>((R)__ldg(q + 3), (R)__ldg(q + 4), (R)__ldg(q + 5));
+        cn.add(ST_PRIMARY);
+        CrossList<R> list;
+        list.e = kept; list.cap = Q.max_hits; list.n = 0; list.count = 0; list.lo = Q.t_min; list.hi = Q.t_max; list.cur = 0;
+        const R tmax = (R)Q.t_max;
+        const R inv_len = R(1) / sqrt_(dot(r.d, r.d));
+        const Vec<R> du = mk<R>(r.d.x * inv_len, r.d.y * inv_len, r.d.z * inv_len);
+        for (int it = 0; it < S.n_items; ++it) {
+            const R4 bound = ldg4<R>(S.item_bound + it);  // xyz = centre, w = inflated radius^2 (+inf: unbounded)
+            const Vec<R> oc = mk<R>(bound.x - r.o.x, bound.y - r.o.y, bound.z - r.o.z);
+            const R b = dot(oc, du);
+            const R oc2 = dot(oc, oc);
+            cn.add(ST_BOUND_TESTS, bound.w < inf_<R>() ? 1u : 0u);
+            if (oc2 - b * b > bound.w + R(1e-6) * oc2) continue;  // the ray's line misses the bound: no crossing at any t
+            const int4 item = __ldg(S.items + it);
+            if ((item.x & 0xff) == ITEM_LEAF) {
+                const int kw = (item.x >> 12) & 0x1ff;
+                if ((kw & 0xff) == LEAF_MESH) {
+                    if constexpr ((FEAT & FT_MESH) != 0) {
+                        const bool identity = (kw >> 8) & 1;
+                        cn.add(ST_LEAF0 + LEAF_MESH);
+                        if (!identity) cn.add(ST_XFORM);
+                        const Ray<R> m = toModel<PackedXform<R, FEAT>::value, R>(S, item.y, identity, r);
+                        meshCrossings<R, STATS>(S, __ldg(S.mesh_root + __ldg(&S.leaf_meta[item.y].w)), item.y, m, tmax, list, overflow, cn);
+                    }
+                } else {
+                    list.cur = item.y;
+                    intersectLeaf<R, FEAT, STATS>(S, item.y, kw, r, list, cn);
+                }
+            } else if constexpr ((FEAT & (FT_CSG | FT_CSGN)) != 0) {
+                const int2 prog = __ldg(S.item_prog + it);  // every CSG item has its program, pairs too
+                const int nh = evalCsg<R, FEAT, STATS>(S, prog.x, prog.y, r, stack, overflow, cn);
+                for (int k = 0; k < nh; ++k) {  // sorted by t: the item's own list
+                    const unsigned id = stack[k].id;
+                    list.add(stack[k].t, (int)(id & kIdLeafMask) | ((id & kIdFlip) ? (1 << 30) : 0), (int)((id >> kIdSubShift) & 7u), 0, false);
+                }
+            }
+        }
+        Q.counts[i] = list.count;
+        const size_t base = (size_t)i * (size_t)Q.max_hits;
+        for (int k = 0; k < Q.max_hits; ++k) {
+            const bool have = k < list.n;
+            HitInfo<R> h;
+            h.t = R(0); h.leaf = -1; h.sub = 0; h.flip = 0;
+            if (have) { h.t = kept[k].t; h.leaf = kept[k].leaf & 0x3fffffff; h.sub = kept[k].sub; h.flip = (kept[k].leaf >> 30) & 1; }
+            // the debug planes' expression, as in query_kernel
+            int prim = -1, sub = 0;
+            if (have) {
+                const int4 meta = __ldg(S.leaf_meta + h.leaf);
+                const int kind = meta.x & 0xff;
+                prim = meta.z;
+                sub = (kind == LEAF_CUBE || kind == LEAF_MESH || kind == LEAF_SOLIDCYL) ? h.sub : ((kind == LEAF_TRIANGLE) ? 0 : meta.w);
+            }
+            const size_t e = base + k;
+            if (Q.prim) Q.prim[e] = prim;
+            if (Q.sub) Q.sub[e] = sub;
+            if (Q.t) Q.t[e] = have ? (double)h.t : -1.0;
+            if (Q.record) {  // a kernel parameter: warp-uniform
+                double rec[13];  // p, normal, colour, roughness, reflectance, shineyness, apply_lighting; an unused slot is all zero
+#pragma unroll
+                for (int j = 0; j < 13; ++j) rec[j] = 0.0;
+                if (have) {
+                    const Fragment<R> f = finalise<R, FEAT>(S, r, h);
+                    rec[0] = f.p.x; rec[1] = f.p.y; rec[2] = f.p.z;
+                    rec[3] = f.n.x; rec[4] = f.n.y; rec[5] = f.n.z;
+                    rec[6] = f.colour.x; rec[7] = f.colour.y; rec[8] = f.colour.z;
+                    rec[9] = f.roughness; rec[10] = f.reflectance; rec[11] = f.shineyness; rec[12] = f.applyLighting ? 1.0 : 0.0;
+                }
+                if (Q.p) { Q.p[3 * e] = rec[0]; Q.p[3 * e + 1] = rec[1]; Q.p[3 * e + 2] = rec[2]; }
+                if (Q.normal) { Q.normal[3 * e] = rec[3]; Q.normal[3 * e + 1] = rec[4]; Q.normal[3 * e + 2] = rec[5]; }
+                if (Q.colour) { Q.colour[3 * e] = rec[6]; Q.colour[3 * e + 1] = rec[7]; Q.colour[3 * e + 2] = rec[8]; }
+                if (Q.surface) { Q.surface[4 * e] = rec[9]; Q.surface[4 * e + 1] = rec[10]; Q.surface[4 * e + 2] = rec[11]; Q.surface[4 * e + 3] = rec[12]; }
+            }
+        }
+    }
+    if (overflow) atomicExch(Q.overflow, 1u);
+    if constexpr (STATS) {
+        for (int k = 0; k < ST_COUNT; ++k) {
+            unsigned long long v = cn.get(k);
+            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(full, v, o);
+            if (lane == 0 && v) atomicAdd(Q.stats + k, v);
+        }
+    }
+}
+
+template <typename R, unsigned FEAT>
+cudaError_t launch_crossings_impl(const DevScene<R>& s, const DevCrossings& q, bool stats, int sm_count, cudaStream_t stream, int* launches)
+{
+    int per_sm = 0;
+    cudaError_t e = stats ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, crossings_kernel<R, FEAT, true>, kBlockThreads, 0)
+                          : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, crossings_kernel<R, FEAT, false>, kBlockThreads, 0);
+    if (e != cudaSuccess) return e;
+    if (per_sm < 1) per_sm = 1;
+    // persistent grid: a multiple of the SM count, never more warps than there are groups of rays
+    const long long want = (long long)sm_count * per_sm, cap = ((long long)q.n_groups + (kBlockThreads / 32) - 1) / (kBlockThreads / 32);
+    int grid = (int)(want < cap ? want : cap);
+    if (grid < 1) grid = 1;
+    if (stats) crossings_kernel<R, FEAT, true><<<grid, kBlockThreads, 0, stream>>>(s, q);
+    else crossings_kernel<R, FEAT, false><<<grid, kBlockThreads, 0, stream>>>(s, q);
+    if (launches) ++*launches;
+    return cudaGetLastError();
+}
+
 }  // namespace ftb

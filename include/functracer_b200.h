@@ -397,6 +397,33 @@ int ftb_intersect_rays_device(ftb_scene* scene, const double* d_rays_od, int64_t
 int ftb_occluded_rays_device(ftb_scene* scene, const double* d_rays_od, const double* d_max_t, int64_t n,
                              const ftb_render_params* params, int32_t* d_blocked, ftb_stats* stats, void* stream);
 
+/* ---- crossing queries: Scene.intersect (Scene.fs:67-104), every crossing of a ray with the scene, sorted by t -----------
+ * n caller-supplied rays as above (o.xyz d.xyz, traced exactly as given, no slightOffset; t in units of d, so the segment
+ * from a to b is the ray (a, b - a) with t_max = 1).
+ *   - Ray i's crossings are the entries of Scene.intersect's list with t_min <= t < t_max.  t_min = -INFINITY gives the whole
+ *     list, including the crossings behind the origin (they set Csg.constructedSolid's inside state) and the t = 0 crossing
+ *     Plane.fs gives a ray parallel to a plane from its front side; t_min = 0 gives what lies ahead.
+ *   - counts[i] = the number of such crossings; it may exceed max_hits.
+ *   - Order: sorted by t, equal t in Scene.intersect's order (Seq.sortBy (fun h -> h.t), the order Scene.closest picks
+ *     from): the first crossing with t >= 0 is the one ftb_intersect_rays returns.
+ *   - The first min(counts[i], max_hits) crossings are written.  The planes of ftb_hit_out are max_hits entries wide per ray:
+ *     entry (i, k) is at i * max_hits + k (times the plane's width: 3 for p, normal, colour, 4 for surface).  Each entry is
+ *     the record ftb_intersect_rays gives, built for that crossing: t, prim_id, sub_id, p, normal (after the CSG flip),
+ *     colour, surface.  Unused slots read as a miss: t = -1, prim_id = -1, sub_id = 0, 0 in every other plane.
+ *   - out may be NULL (counts only); any plane pointer may be NULL = not wanted (left untouched).
+ *   - params: only precision and collect_stats are read; the counting kernel counts every ray as a primary ray.
+ *   - Bad arguments, checked before any device is looked for: FTB_ERR_BAD_ARG for a NULL scene or params, n < 0, NULL rays
+ *     or counts with n > 0, max_hits outside 1 .. FTB_MAX_CROSSINGS, t_min or t_max NaN, or t_min >= t_max.  n = 0 is OK;
+ *     no CUDA device: FTB_ERR_NO_DEVICE.
+ *   - A CSG hit-stack overflow is reported as by the other queries (the host entry then leaves the caller's arrays
+ *     unwritten); one frame or query in flight per scene and device; the device entry synchronises only to fill stats. */
+#define FTB_MAX_CROSSINGS 64
+int ftb_intersect_all_rays(ftb_scene* scene, const double* rays_od, int64_t n, int32_t max_hits, double t_min, double t_max,
+                           const ftb_render_params* params, const ftb_hit_out* out, int32_t* counts, ftb_stats* stats);
+int ftb_intersect_all_rays_device(ftb_scene* scene, const double* d_rays_od, int64_t n, int32_t max_hits, double t_min,
+                                  double t_max, const ftb_render_params* params, const ftb_hit_out* d_out, int32_t* d_counts,
+                                  ftb_stats* stats, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -174,6 +174,11 @@ extern int ftb_shade_rays(nativeint scene, nativeint raysOD, int64 n, FtbRenderP
 /// normal, colour, surface; 0n = not wanted)
 [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
 extern int ftb_intersect_rays(nativeint scene, nativeint raysOD, int64 n, FtbRenderParams& p, nativeint hitOut, nativeint statsOrNull)
+/// Scene.intersect (Scene.fs:67-104) on n caller-supplied rays: every crossing with tMin <= t < tMax, sorted by t (equal t in the
+/// reference's order), counts[i] crossings per ray (may exceed maxHits), the first maxHits of them written to the planes of
+/// hitOut (as for ftb_intersect_rays, maxHits entries per ray: entry (i, k) at i * maxHits + k; unused slots read as a miss)
+[<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+extern int ftb_intersect_all_rays(nativeint scene, nativeint raysOD, int64 n, int maxHits, float tMin, float tMax, FtbRenderParams& p, nativeint hitOut, int[] counts, nativeint statsOrNull)
 
 let lastError () = Marshal.PtrToStringAnsi (ftb_last_error ())
 let check rc = if rc <> 0 then failwithf "functracer_b200 status %d: %s" rc (lastError ())
