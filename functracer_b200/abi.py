@@ -117,6 +117,13 @@ class HitOut(C.Structure):
                 ("surface", C.POINTER(C.c_double))]
 
 
+class PathOut(C.Structure):
+    """ftb_path_out: the planes of a path query (any pointer may be NULL = not wanted)."""
+    _fields_ = [("levels", C.POINTER(C.c_int32)), ("colour", C.POINTER(C.c_double)), ("ray_od", C.POINTER(C.c_double)),
+                ("weight", C.POINTER(C.c_double)), ("hit", HitOut), ("intensity", C.POINTER(C.c_double)),
+                ("light_dir", C.POINTER(C.c_double)), ("light_colour", C.POINTER(C.c_double))]
+
+
 class Stats(C.Structure):
     _fields_ = [("primary_rays", C.c_uint64), ("shadow_rays", C.c_uint64), ("reflection_rays", C.c_uint64),
                 ("shaded_hits", C.c_uint64), ("leaf_tests", C.c_uint64 * 10),
@@ -140,5 +147,5 @@ EXPORTS = [
     "ftb_shade_rays", "ftb_band_rows", "ftb_assemble_rows_device", "ftb_host_copy_begin", "ftb_host_copy_finish",
     "ftb_check_overflow", "ftb_scene_build_info", "ftb_render_window", "ftb_render_window_tiles_device",
     "ftb_intersect_rays", "ftb_occluded_rays", "ftb_intersect_rays_device", "ftb_occluded_rays_device",
-    "ftb_intersect_all_rays", "ftb_intersect_all_rays_device",
+    "ftb_intersect_all_rays", "ftb_intersect_all_rays_device", "ftb_trace_paths", "ftb_trace_paths_device",
 ]

@@ -86,9 +86,13 @@ def lib():
                            ("ftb_intersect_all_rays", [vp, dp, C.c_int64, C.c_int32, C.c_double, C.c_double, C.POINTER(abi.RenderParams),
                                                        C.POINTER(abi.HitOut), ip, C.POINTER(abi.Stats)]),
                            ("ftb_intersect_all_rays_device", [vp, dp, C.c_int64, C.c_int32, C.c_double, C.c_double, C.POINTER(abi.RenderParams),
-                                                              C.POINTER(abi.HitOut), ip, C.POINTER(abi.Stats), vp])):
+                                                              C.POINTER(abi.HitOut), ip, C.POINTER(abi.Stats), vp]),
+                           ("ftb_trace_paths", [vp, dp, C.POINTER(C.c_uint64), C.c_int64, C.POINTER(abi.RenderParams), C.POINTER(abi.PathOut),
+                                                C.POINTER(abi.Stats)]),
+                           ("ftb_trace_paths_device", [vp, dp, C.POINTER(C.c_uint64), C.c_int64, C.POINTER(abi.RenderParams),
+                                                       C.POINTER(abi.PathOut), C.POINTER(abi.Stats), vp])):
             if os.environ.get("FTB_LIB") and not hasattr(L, name):
-                setattr(L, name, None)  # an older A/B build of the same ABI without ray (or crossing) queries
+                setattr(L, name, None)  # an older A/B build of the same ABI without ray (crossing, path) queries
             else:
                 getattr(L, name).argtypes = args
                 getattr(L, name).restype = C.c_int
@@ -128,6 +132,25 @@ MAX_CROSSINGS = 64  # FTB_MAX_CROSSINGS: the most crossings a crossing query kee
 HIT_PLANES = ("t", "prim", "sub", "p", "normal", "colour", "surface")
 _PLANE_TYPES = ((C.c_double, np.float64, 1), (C.c_int32, np.int32, 1), (C.c_int32, np.int32, 1), (C.c_double, np.float64, 3),
                 (C.c_double, np.float64, 3), (C.c_double, np.float64, 3), (C.c_double, np.float64, 4))
+
+MAX_PATH_LEVELS = 64  # FTB_MAX_PATH_LEVELS: recursion_limit + 1 of a path query is at most this
+# the planes of a path query (ftb_path_out; the hit planes are HIT_PLANES, with "hit_colour" for ftb_hit_out's colour):
+# name -> (ctypes element, numpy dtype, shape after n: "D" = levels per ray, "L" = lights)
+PATH_PLANES = {
+    "levels": (C.c_int32, np.int32, ()), "colour": (C.c_double, np.float64, (3,)), "ray": (C.c_double, np.float64, ("D", 6)),
+    "weight": (C.c_double, np.float64, ("D",)), "t": (C.c_double, np.float64, ("D",)), "prim": (C.c_int32, np.int32, ("D",)),
+    "sub": (C.c_int32, np.int32, ("D",)), "p": (C.c_double, np.float64, ("D", 3)), "normal": (C.c_double, np.float64, ("D", 3)),
+    "hit_colour": (C.c_double, np.float64, ("D", 3)), "surface": (C.c_double, np.float64, ("D", 4)),
+    "intensity": (C.c_double, np.float64, ("D", "L")), "light_dir": (C.c_double, np.float64, ("D", "L", 3)),
+    "light_colour": (C.c_double, np.float64, ("D", "L", 3)),
+}
+
+
+def _path_out(ptrs):
+    """abi.PathOut from {plane name of PATH_PLANES: ctypes pointer} (missing = NULL)."""
+    g = lambda name: ptrs.get(name)  # noqa: E731
+    hit = abi.HitOut(g("t"), g("prim"), g("sub"), g("p"), g("normal"), g("hit_colour"), g("surface"))
+    return abi.PathOut(g("levels"), g("colour"), g("ray"), g("weight"), hit, g("intensity"), g("light_dir"), g("light_colour"))
 
 
 class Scene:
@@ -283,6 +306,50 @@ class Scene:
                                                               t_max, C.byref(make_params(1, 1, 1, None, **kw)), C.byref(hit),
                                                               C.cast(C.c_void_p(d_counts_ptr), C.POINTER(C.c_int32)),
                                                               C.byref(stats) if stats is not None else None, C.c_void_p(stream)))
+
+    # -- Shading.getColourForRay (Shading.fs:109-147) on explicit rays, level by level and light by light -------------------
+    def trace_paths(self, rays_od, sample_keys=None, recursion_limit=8, seed=1234, planes=tuple(PATH_PLANES), stats=None, **kw):
+        """Why each ray [n, 6] has the colour ftb_shade_rays gives it.  The rays are shaded as shade() shades them (slightOffset
+        included); sample_keys [n] uint64 are the soft lights' RNG keys (None: the ray's index, as shade() uses).  Returns
+        {plane: array} for the requested planes of PATH_PLANES: levels [n], colour [n, 3], and per level (D = recursion_limit
+        + 1) ray [n, D, 6], weight / t / prim / sub [n, D], p / normal / hit_colour [n, D, 3], surface [n, D, 4], and per level
+        and light (L lights) intensity [n, D, L], light_dir / light_colour [n, D, L, 3].  kw: make_params' precision,
+        collect_stats."""
+        unknown = set(planes) - set(PATH_PLANES)
+        if unknown:
+            raise ValueError("unknown planes %s (choose from %s)" % (sorted(unknown), sorted(PATH_PLANES)))
+        rays = np.ascontiguousarray(rays_od, dtype=np.float64).reshape(-1, 6)
+        n = rays.shape[0]
+        keys = None
+        if sample_keys is not None:
+            keys = np.ascontiguousarray(sample_keys, dtype=np.uint64).reshape(-1)
+            if keys.size != n:
+                raise ValueError("sample_keys must hold one key per ray")
+        dims = {"D": max(0, recursion_limit) + 1, "L": self.parsed.desc_ptr.contents.n_lights}
+        out, ptrs = {}, {}
+        for name in planes:
+            ct, dt, shape = PATH_PLANES[name]
+            out[name] = np.empty((n,) + tuple(dims.get(k, k) for k in shape), dtype=dt)
+            ptrs[name] = out[name].ctypes.data_as(C.POINTER(ct))
+        po = _path_out(ptrs)
+        p = make_params(1, 1, 1, None, recursion_limit=recursion_limit, seed=seed, **kw)
+        _check(_query_entry("ftb_trace_paths")(self._h, rays.ctypes.data_as(C.POINTER(C.c_double)),
+                                                keys.ctypes.data_as(C.POINTER(C.c_uint64)) if keys is not None else None, n,
+                                                C.byref(p), C.byref(po), C.byref(stats) if stats is not None else None))
+        return out
+
+    def trace_paths_device(self, d_rays_ptr, n, d_planes, d_keys_ptr=0, recursion_limit=8, seed=1234, stream=0, stats=None, **kw):
+        """trace_paths() on DEVICE memory of the current device, queued on `stream`: d_rays_ptr = n * 6 doubles, d_keys_ptr =
+        n uint64 (0 = the ray's index), d_planes = {plane name of PATH_PLANES: device address} (missing / 0 = not wanted),
+        sized as trace_paths() returns them.  Does not synchronise unless stats is given."""
+        unknown = set(d_planes) - set(PATH_PLANES)
+        if unknown:
+            raise ValueError("unknown planes %s (choose from %s)" % (sorted(unknown), sorted(PATH_PLANES)))
+        po = _path_out({name: C.cast(C.c_void_p(d_planes.get(name) or None), C.POINTER(PATH_PLANES[name][0])) for name in PATH_PLANES})
+        p = make_params(1, 1, 1, None, recursion_limit=recursion_limit, seed=seed, **kw)
+        _check(_query_entry("ftb_trace_paths_device")(self._h, C.cast(C.c_void_p(d_rays_ptr), C.POINTER(C.c_double)),
+                                                       C.cast(C.c_void_p(d_keys_ptr or None), C.POINTER(C.c_uint64)), n, C.byref(p),
+                                                       C.byref(po), C.byref(stats) if stats is not None else None, C.c_void_p(stream)))
 
     # -- device-buffer entry points (one process per GPU; pointers are raw device addresses) -----
     def render_tiles_device(self, p, d_tiles_ptr, stream=0, stats=False, camera=None, d_dbg=None, window=None):

@@ -141,6 +141,11 @@ cudaError_t crossings_f32(const DevScene<float>&, const DevCrossings&, bool, int
 cudaError_t crossings_f64(const DevScene<double>&, const DevCrossings&, bool, int, cudaStream_t, int*);
 inline cudaError_t launchCrossings(const DevScene<float>& s, const DevCrossings& q, bool stats, int sm, cudaStream_t st, int* l) { return crossings_f32(s, q, stats, sm, st, l); }
 inline cudaError_t launchCrossings(const DevScene<double>& s, const DevCrossings& q, bool stats, int sm, cudaStream_t st, int* l) { return crossings_f64(s, q, stats, sm, st, l); }
+// the path queries' kernel (paths.cu): generic FEAT only, one object per precision
+cudaError_t paths_f32(const DevScene<float>&, const DevPaths&, bool, int, cudaStream_t, int*);
+cudaError_t paths_f64(const DevScene<double>&, const DevPaths&, bool, int, cudaStream_t, int*);
+inline cudaError_t launchPaths(const DevScene<float>& s, const DevPaths& q, bool stats, int sm, cudaStream_t st, int* l) { return paths_f32(s, q, stats, sm, st, l); }
+inline cudaError_t launchPaths(const DevScene<double>& s, const DevPaths& q, bool stats, int sm, cudaStream_t st, int* l) { return paths_f64(s, q, stats, sm, st, l); }
 static const Variant<float> kVariantsF32[] = {
 #define X(feat) {(unsigned)(feat), UnitCap<float, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f32_##feat, query_f32_##feat},
     FTB_FEAT_LIST_F32
@@ -1165,6 +1170,109 @@ int crossingsHost(ftb_scene* sc, const double* rays, int64_t n, int32_t max_hits
     return FTB_OK;
 }
 
+// ---- path queries ---------------------------------------------------------------------------------------------------
+// The argument a path query adds (the recursion limit, which sizes its planes), then checkQuery's (which ends with the device
+// count): everything a caller can get wrong is reported before any device is looked for.
+int checkPaths(const ftb_scene* sc, const double* rays, int64_t n, const ftb_render_params* p)
+{
+    if (p && (p->recursion_limit < 0 || p->recursion_limit > FTB_MAX_PATH_LEVELS - 1)) return fail(FTB_ERR_BAD_ARG, "recursion_limit outside 0 .. FTB_MAX_PATH_LEVELS - 1");
+    return checkQuery(sc, rays, nullptr, n, p, false, nullptr);
+}
+
+// The device entry point: one batch of path queries (device pointers) queued on `s` on the current device, with the per-device
+// control block, as queryDevice does for the other queries.  out may be null (stats only).
+int pathsDevice(ftb_scene* sc, const double* rays, const uint64_t* keys, int64_t n, const ftb_render_params* p, const ftb_path_out* out,
+                ftb_stats* stats, cudaStream_t s)
+{
+    int rc = checkPaths(sc, rays, n, p);
+    if (rc != FTB_OK) return rc;
+    if (stats) std::memset(stats, 0, sizeof(*stats));
+    if (n == 0) return FTB_OK;
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    rc = byPrecision(p->precision, [&](auto r) -> int {
+        Launch<decltype(r)> fr;  // the scene on this device and the control block; the variant it picks is not used
+        int e = fr.begin(sc, pd, p, sc->L.features, stats && p->collect_stats, nullptr, nullptr);
+        if (e != FTB_OK) return e;
+        CK(pd->control.prepare(fr.counting, s));
+        CK(pd->control.resetQueue(s));
+        DevPaths q;
+        std::memset(&q, 0, sizeof(q));
+        q.rays = rays; q.sample_keys = reinterpret_cast<const unsigned long long*>(keys); q.n = n; q.n_groups = (int)((n + 31) / 32);
+        q.recursion_limit = p->recursion_limit; q.seed = p->seed;
+        if (out) {
+            q.levels = out->levels; q.colour = out->colour; q.ray_od = out->ray_od; q.weight = out->weight;
+            q.t = out->hit.t; q.prim = out->hit.prim_id; q.sub = out->hit.sub_id;
+            q.p = out->hit.p; q.normal = out->hit.normal; q.hit_colour = out->hit.colour; q.surface = out->hit.surface;
+            q.intensity = out->intensity; q.light_dir = out->light_dir; q.light_colour = out->light_colour;
+        }
+        q.record = (q.p || q.normal || q.hit_colour || q.surface) ? 1 : 0;
+        Control* c = pd->control.ctl();
+        q.group_counter = &c->tile_counter; q.overflow = &c->overflow; q.stats = c->stats;
+        if (stats) CK(cudaEventRecord(pd->ev0, s));
+        CK(launchPaths(*fr.scene, q, fr.counting, pd->sm_count, s, &fr.launches));
+        if (stats) { CK(cudaEventRecord(pd->ev1, s)); stats->kernel_launches += fr.launches + 1; }  // + the control-block memset
+        return FTB_OK;
+    });
+    if (rc != FTB_OK) return rc;
+    bool overflow = false;
+    if (stats && (rc = finishStats(sc, pd, stats, s, &overflow)) != FTB_OK) return rc;
+    return overflow ? overflowError() : FTB_OK;
+}
+
+// The host entry point, the pattern of crossingsHost: upload the rays and keys, queue the device entry, read the control block
+// back, and only then download the requested planes (D = recursion_limit + 1 level entries per ray, D * L light entries): on an
+// overflow nothing of the caller's is written.
+int pathsHost(ftb_scene* sc, const double* rays, const uint64_t* keys, int64_t n, const ftb_render_params* p, const ftb_path_out* out,
+              ftb_stats* stats)
+{
+    const auto t0 = std::chrono::steady_clock::now();
+    int rc = checkPaths(sc, rays, n, p);
+    if (rc != FTB_OK || n == 0) return rc != FTB_OK ? rc : pathsDevice(sc, rays, keys, n, p, out, stats, nullptr);
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    const cudaStream_t s = pd->stream;
+    CK(pd->rays.reserve((size_t)n * 48));
+    CK(cudaMemcpyAsync(pd->rays.p, rays, (size_t)n * 48, cudaMemcpyHostToDevice, s));
+    // the keys (in), then the requested planes with their bytes per ray; one device buffer
+    struct Plane { void* host; size_t per_ray; void* dev; };
+    ftb_path_out o;
+    std::memset(&o, 0, sizeof(o));
+    if (out) o = *out;
+    const size_t D = (size_t)p->recursion_limit + 1, DL = D * sc->lights.size();
+    Plane planes[15] = {{const_cast<uint64_t*>(keys), 8, nullptr}, {o.levels, 4, nullptr}, {o.colour, 24, nullptr}, {o.ray_od, 48 * D, nullptr},
+                        {o.weight, 8 * D, nullptr}, {o.hit.t, 8 * D, nullptr}, {o.hit.prim_id, 4 * D, nullptr}, {o.hit.sub_id, 4 * D, nullptr},
+                        {o.hit.p, 24 * D, nullptr}, {o.hit.normal, 24 * D, nullptr}, {o.hit.colour, 24 * D, nullptr}, {o.hit.surface, 32 * D, nullptr},
+                        {o.intensity, 8 * DL, nullptr}, {o.light_dir, 24 * DL, nullptr}, {o.light_colour, 24 * DL, nullptr}};
+    size_t bytes = 0;
+    for (const Plane& pl : planes) if (pl.host) bytes += ((pl.per_ray * (size_t)n + 255) & ~(size_t)255);
+    CK(pd->query.reserve(std::max<size_t>(bytes, 1)));
+    size_t at = 0;
+    for (Plane& pl : planes)
+        if (pl.host) { pl.dev = static_cast<char*>(pd->query.p) + at; at += ((pl.per_ray * (size_t)n + 255) & ~(size_t)255); }
+    if (keys) CK(cudaMemcpyAsync(planes[0].dev, keys, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+    ftb_path_out d;
+    d.levels = static_cast<int32_t*>(planes[1].dev); d.colour = static_cast<double*>(planes[2].dev);
+    d.ray_od = static_cast<double*>(planes[3].dev); d.weight = static_cast<double*>(planes[4].dev);
+    d.hit = {static_cast<double*>(planes[5].dev), static_cast<int32_t*>(planes[6].dev), static_cast<int32_t*>(planes[7].dev),
+             static_cast<double*>(planes[8].dev), static_cast<double*>(planes[9].dev), static_cast<double*>(planes[10].dev),
+             static_cast<double*>(planes[11].dev)};
+    d.intensity = static_cast<double*>(planes[12].dev); d.light_dir = static_cast<double*>(planes[13].dev);
+    d.light_colour = static_cast<double*>(planes[14].dev);
+    rc = pathsDevice(sc, static_cast<const double*>(pd->rays.p), static_cast<const uint64_t*>(planes[0].dev), n, p, &d, stats, s);
+    if (rc == FTB_OK && !stats) {  // with stats pathsDevice has read the control block (and reported an overflow) already
+        bool overflow = false;
+        rc = finishStats(sc, pd, nullptr, s, &overflow);
+        if (rc == FTB_OK && overflow) rc = overflowError();
+    }
+    if (rc != FTB_OK) return rc;
+    for (int k = 1; k < 15; ++k)
+        if (planes[k].host && planes[k].per_ray) CK(cudaMemcpyAsync(planes[k].host, planes[k].dev, planes[k].per_ray * (size_t)n, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return FTB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1525,6 +1633,18 @@ int ftb_intersect_all_rays_device(ftb_scene* scene, const double* d_rays_od, int
                                   const ftb_render_params* params, const ftb_hit_out* d_out, int32_t* d_counts, ftb_stats* stats, void* stream)
 {
     return crossingsDevice(scene, d_rays_od, n, max_hits, t_min, t_max, params, d_out, d_counts, stats, static_cast<cudaStream_t>(stream));
+}
+
+int ftb_trace_paths(ftb_scene* scene, const double* rays_od, const uint64_t* sample_keys, int64_t n, const ftb_render_params* params,
+                    const ftb_path_out* out, ftb_stats* stats)
+{
+    return pathsHost(scene, rays_od, sample_keys, n, params, out, stats);
+}
+
+int ftb_trace_paths_device(ftb_scene* scene, const double* d_rays_od, const uint64_t* d_sample_keys, int64_t n, const ftb_render_params* params,
+                           const ftb_path_out* d_out, ftb_stats* stats, void* stream)
+{
+    return pathsDevice(scene, d_rays_od, d_sample_keys, n, params, d_out, stats, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

@@ -225,6 +225,35 @@ struct DevCrossings {
     unsigned long long* stats;  // ST_COUNT slots (counting kernel only)
 };
 
+// A batch of path queries (path_kernel, paths.cu): getColourForRay on caller-supplied rays, every level and light recorded.
+// Level planes are depth entries wide per ray, light planes depth * n_lights; every output pointer may be null.
+struct DevPaths {
+    const double* rays;                     // o.xyz d.xyz per ray
+    const unsigned long long* sample_keys;  // RNG key per ray; nullptr = the ray's index (what ftb_shade_rays uses)
+    long long n;                            // rays
+    int n_groups;                           // groups of 32 rays in the queue
+    int recursion_limit;                    // depth = recursion_limit + 1 levels
+    unsigned long long seed;
+    int record;  // 1: some hit plane beyond t / prim / sub is wanted
+    int* levels;
+    double* colour;        // 3 per ray
+    double* ray_od;        // 6 per level
+    double* weight;        // 1 per level
+    double* t;             // 1 per level
+    int* prim;             // 1 per level
+    int* sub;              // 1 per level
+    double* p;             // 3 per level
+    double* normal;        // 3 per level
+    double* hit_colour;    // 3 per level
+    double* surface;       // 4 per level: roughness, reflectance, shineyness, apply_lighting
+    double* intensity;     // 1 per (level, light)
+    double* light_dir;     // 3 per (level, light)
+    double* light_colour;  // 3 per (level, light)
+    unsigned int* group_counter;
+    unsigned int* overflow;
+    unsigned long long* stats;  // ST_COUNT slots (counting kernel only)
+};
+
 #ifdef __CUDACC__
 // Block c of a mode-0 frame's work queue: its first pixel's slot in the tile buffer, its origin in the whole frame's sample
 // grid, its width and its pixel count (clipped to the window; 0 for a tile the last shard group lacks).

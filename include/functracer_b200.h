@@ -424,6 +424,51 @@ int ftb_intersect_all_rays_device(ftb_scene* scene, const double* d_rays_od, int
                                   double t_max, const ftb_render_params* params, const ftb_hit_out* d_out, int32_t* d_counts,
                                   ftb_stats* stats, void* stream);
 
+/* ---- path queries: why a ray has its colour (Shading.getColourForRay, Shading.fs:109-147) ----------------------------------
+ * n caller-supplied rays as for ftb_shade_rays (o.xyz d.xyz).  Each is shaded as ftb_shade_rays shades it, and every level
+ * (bounce) of getColourForRay is reported: its ray, nearest hit and weight, and per light the shadow intensity, the light
+ * direction and the colour shadeLight gives.  D = params->recursion_limit + 1 level entries per ray, L = the scene's light count:
+ * entry (i, k) is at i * D + k, entry (i, k, l) at (i * D + k) * L + l, each times the plane's width.
+ *   - Rays and keys: the level-0 ray and every reflected ray get the 1e-4 slightOffset, and hit.t is measured along the offset
+ *     ray (as the debug planes of ftb_debug_out measure it).  Soft lights draw from ftb_rng.h with params->seed, depth
+ *     recursion_limit - limit and sample key sample_keys[i]; NULL sample_keys means key i, which is what ftb_shade_rays uses.
+ *     So a frame sample's primary ray with key (py * gw + px) * spp + s gives that sample's path.
+ *   - Colour: colour[i] is the sum the renderer forms: per level, local = 0, then local += light_colour[l] in light order, then
+ *     colour += W * local; reflecting multiplies W by L * reflectance.  In FP64 this sum, colour and ftb_shade_rays' output
+ *     for the same ray and key are bit-identical.  In FP32 the query runs the generic kernel where ftb_shade_rays may run the
+ *     scene's specialised one, so the two agree to FP32 rounding, not bit for bit.
+ *   - Levels: levels[i] counts the nearest-hit rays traced (1 .. D).  A level that misses reads t = -1, prim_id = -1,
+ *     sub_id = 0 and 0 in every other hit plane and every light plane; its ray and weight are written.  Entries after
+ *     levels[i] read as a miss with weight 0 and a zero ray.  With L = 0 nothing is shaded or reflected: level 0 is recorded
+ *     and the colour is 0.
+ *   - Shadow rays that are not traced: an unlit surface, or an Oren-Nayar surface without a specular term, reports intensity 1
+ *     (its colour does not depend on it); a soft light with 0 samples reports NaN, as the reference computes 0 / 0.
+ *   - params: only precision, seed, recursion_limit and collect_stats are read.  The counting kernel counts primary, shadow
+ *     and reflection rays and shaded hits as ftb_shade_rays' counting kernel does for the same rays; leaf and bound tests also
+ *     agree unless a frame's common-origin bound table answers some of ftb_shade_rays' bound tests (scenes of 8 or more
+ *     top-level items with point lights), which this query does not use.
+ *   - Bad arguments, checked before any device is looked for: FTB_ERR_BAD_ARG for a NULL scene or params, n < 0, NULL rays
+ *     with n > 0, a bad precision, or recursion_limit outside 0 .. FTB_MAX_PATH_LEVELS - 1.  n = 0 is OK; no CUDA device:
+ *     FTB_ERR_NO_DEVICE.
+ *   - A hit-stack overflow is reported as by the other queries (the host entry then leaves the caller's arrays unwritten);
+ *     one frame or query in flight per scene and device; the device entry synchronises only to fill stats. */
+#define FTB_MAX_PATH_LEVELS 64
+typedef struct ftb_path_out {  /* any pointer may be NULL = not wanted (left untouched) */
+    int32_t* levels;           /* n      levels traced, 1 .. D                                                        */
+    double* colour;            /* 3n     the ray's colour: ftb_shade_rays' value for this ray and key                 */
+    double* ray_od;            /* 6nD    each level's ray (o.xyz d.xyz) before slightOffset                           */
+    double* weight;            /* nD     the level's running weight W                                                 */
+    ftb_hit_out hit;           /* nD each the level's nearest hit, planes as in ftb_hit_out                           */
+    double* intensity;         /* nDL    shadow intensity of light l at level k                                       */
+    double* light_dir;         /* 3nDL   lightDirection (Shading.fs:44-48) at the hit point                           */
+    double* light_colour;      /* 3nDL   shadeLight's colour for light l (specular + diffuse, or the unlit surface
+                                         colour); the reflection is in the next level's W                             */
+} ftb_path_out;
+int ftb_trace_paths(ftb_scene* scene, const double* rays_od, const uint64_t* sample_keys, int64_t n,
+                    const ftb_render_params* params, const ftb_path_out* out, ftb_stats* stats);
+int ftb_trace_paths_device(ftb_scene* scene, const double* d_rays_od, const uint64_t* d_sample_keys, int64_t n,
+                           const ftb_render_params* params, const ftb_path_out* d_out, ftb_stats* stats, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

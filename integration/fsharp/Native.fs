@@ -179,6 +179,13 @@ extern int ftb_intersect_rays(nativeint scene, nativeint raysOD, int64 n, FtbRen
 /// hitOut (as for ftb_intersect_rays, maxHits entries per ray: entry (i, k) at i * maxHits + k; unused slots read as a miss)
 [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
 extern int ftb_intersect_all_rays(nativeint scene, nativeint raysOD, int64 n, int maxHits, float tMin, float tMax, FtbRenderParams& p, nativeint hitOut, int[] counts, nativeint statsOrNull)
+/// Shading.getColourForRay (Shading.fs:109-147) level by level on n caller-supplied rays, shaded as ftb_shade_rays shades them.
+/// pathOut is the address of a pinned nativeint[14]: the plane pointers of ftb_path_out in its order (levels, colour, ray_od,
+/// weight, the 7 of ftb_hit_out, intensity, light_dir, light_colour; 0n = not wanted).  D = p.recursionLimit + 1 level entries
+/// per ray (entry (i, k) at i * D + k), L lights per level (entry (i, k, l) at (i * D + k) * L + l).  keysOrNull: n uint64
+/// sample keys of the soft lights' RNG, 0n = the ray's index (what ftb_shade_rays uses)
+[<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+extern int ftb_trace_paths(nativeint scene, nativeint raysOD, nativeint keysOrNull, int64 n, FtbRenderParams& p, nativeint pathOut, nativeint statsOrNull)
 
 let lastError () = Marshal.PtrToStringAnsi (ftb_last_error ())
 let check rc = if rc <> 0 then failwithf "functracer_b200 status %d: %s" rc (lastError ())
