@@ -148,4 +148,5 @@ EXPORTS = [
     "ftb_check_overflow", "ftb_scene_build_info", "ftb_render_window", "ftb_render_window_tiles_device",
     "ftb_intersect_rays", "ftb_occluded_rays", "ftb_intersect_rays_device", "ftb_occluded_rays_device",
     "ftb_intersect_all_rays", "ftb_intersect_all_rays_device", "ftb_trace_paths", "ftb_trace_paths_device",
+    "ftb_frame_rays", "ftb_frame_rays_device", "ftb_shade_samples", "ftb_shade_samples_device",
 ]

@@ -90,9 +90,17 @@ def lib():
                            ("ftb_trace_paths", [vp, dp, C.POINTER(C.c_uint64), C.c_int64, C.POINTER(abi.RenderParams), C.POINTER(abi.PathOut),
                                                 C.POINTER(abi.Stats)]),
                            ("ftb_trace_paths_device", [vp, dp, C.POINTER(C.c_uint64), C.c_int64, C.POINTER(abi.RenderParams),
-                                                       C.POINTER(abi.PathOut), C.POINTER(abi.Stats), vp])):
+                                                       C.POINTER(abi.PathOut), C.POINTER(abi.Stats), vp]),
+                           ("ftb_frame_rays", [vp, C.POINTER(abi.Camera), C.POINTER(abi.RenderParams)] + [C.c_int32] * 4
+                            + [dp, C.POINTER(C.c_uint64)]),
+                           ("ftb_frame_rays_device", [vp, C.POINTER(abi.Camera), C.POINTER(abi.RenderParams)] + [C.c_int32] * 4
+                            + [dp, C.POINTER(C.c_uint64), vp]),
+                           ("ftb_shade_samples", [vp, dp, C.POINTER(C.c_uint64), C.c_int64, C.POINTER(abi.RenderParams), vp,
+                                                  C.POINTER(abi.DebugOut), C.POINTER(abi.Stats)]),
+                           ("ftb_shade_samples_device", [vp, dp, C.POINTER(C.c_uint64), C.c_int64, C.POINTER(abi.RenderParams), vp,
+                                                         C.POINTER(abi.DebugOut), C.POINTER(abi.Stats), vp])):
             if os.environ.get("FTB_LIB") and not hasattr(L, name):
-                setattr(L, name, None)  # an older A/B build of the same ABI without ray (crossing, path) queries
+                setattr(L, name, None)  # an older A/B build of the same ABI without ray (crossing, path) queries or sample shading
             else:
                 getattr(L, name).argtypes = args
                 getattr(L, name).restype = C.c_int
@@ -350,6 +358,78 @@ class Scene:
         _check(_query_entry("ftb_trace_paths_device")(self._h, C.cast(C.c_void_p(d_rays_ptr), C.POINTER(C.c_double)),
                                                        C.cast(C.c_void_p(d_keys_ptr or None), C.POINTER(C.c_uint64)), n, C.byref(p),
                                                        C.byref(po), C.byref(stats) if stats is not None else None, C.c_void_p(stream)))
+
+    # -- a frame's own samples (SamplingStrategy.generateRays / blendPixels, Image.fs:100-116) in the caller's hands ------------
+    def frame_rays(self, window, width, height, spp, jitter_xy=None, camera=None, **kw):
+        """The primary ray and RNG key of every sample of window (x0, y0, x1, y1) of the width x height frame, as render_window
+        generates them.  Returns (rays [n, 6] o.xyz d.xyz before slightOffset, keys [n] uint64), n entries in the debug planes'
+        order: (x1-x0)*(y1-y0)*spp in jitter sampling, (x1-x0+1)*(y1-y0+1) corners in corner sampling.  kw: make_params'
+        sampling, precision, seed."""
+        p = make_params(width, height, spp, jitter_xy, **kw)
+        x0, y0, x1, y1 = (int(v) for v in window)
+        n = max(0, x1 - x0 + 1) * max(0, y1 - y0 + 1) if p.sampling == abi.SAMPLING_CORNER else max(0, x1 - x0) * max(0, y1 - y0) * spp
+        rays = np.empty((n, 6), dtype=np.float64)
+        keys = np.empty(n, dtype=np.uint64)
+        cam = camera if camera is not None else self.parsed.camera_ptr
+        _check(_query_entry("ftb_frame_rays")(self._h, cam, C.byref(p), x0, y0, x1, y1, rays.ctypes.data_as(C.POINTER(C.c_double)),
+                                               keys.ctypes.data_as(C.POINTER(C.c_uint64))))
+        return rays, keys
+
+    def frame_rays_device(self, p, window, d_rays_ptr, d_keys_ptr, stream=0, camera=None):
+        """frame_rays() into DEVICE memory of the current device, queued on `stream`: d_rays_ptr = n * 6 doubles, d_keys_ptr = n
+        uint64 (either 0 = not wanted); p: make_params(...)."""
+        cam = camera if camera is not None else self.parsed.camera_ptr
+        _check(_query_entry("ftb_frame_rays_device")(self._h, cam, C.byref(p), *[int(v) for v in window],
+                                                      C.cast(C.c_void_p(d_rays_ptr or None), C.POINTER(C.c_double)),
+                                                      C.cast(C.c_void_p(d_keys_ptr or None), C.POINTER(C.c_uint64)), C.c_void_p(stream)))
+
+    def shade_samples(self, rays_od, spp, sample_keys=None, debug=False, stats=False, out=None, **kw):
+        """Shades n_pixels * spp rays [n_pixels * spp, 6] (sample s of pixel i = ray i * spp + s) and blends each pixel as
+        render() blends a jitter-mode pixel.  sample_keys [n_pixels * spp] uint64 are the RNG keys (None: the ray's index).
+        Returns render()'s dict with rgb [n_pixels, C] and debug planes of n_pixels * spp entries.  kw: make_params' precision,
+        seed, recursion_limit, out_format, collect_stats."""
+        rays = np.ascontiguousarray(rays_od, dtype=np.float64).reshape(-1, 6)
+        if spp < 1 or rays.shape[0] % spp:
+            raise ValueError("the ray count must be a multiple of spp >= 1")
+        n_pix, n = rays.shape[0] // spp, rays.shape[0]
+        keys = None
+        if sample_keys is not None:
+            keys = np.ascontiguousarray(sample_keys, dtype=np.uint64).reshape(-1)
+            if keys.size != n:
+                raise ValueError("sample_keys must hold one key per ray")
+        if stats:
+            kw.setdefault("collect_stats", 1)
+        p = make_params(1, 1, spp, None, **kw)
+        dt, ch = _OUT_DTYPE[p.out_format]
+        if out is None:
+            out = np.empty((n_pix, ch), dtype=dt)
+        assert out.dtype == dt and out.size == n_pix * ch and out.flags["C_CONTIGUOUS"]
+        prim = sub = t = dbg = None
+        if debug:
+            prim = np.full(n, -2, dtype=np.int32)
+            sub = np.zeros(n, dtype=np.int32)
+            t = np.zeros(n, dtype=np.float64)
+            dbg = abi.DebugOut(prim.ctypes.data_as(C.POINTER(C.c_int32)), sub.ctypes.data_as(C.POINTER(C.c_int32)),
+                               t.ctypes.data_as(C.POINTER(C.c_double)))
+        st = abi.Stats() if stats else None
+        _check(_query_entry("ftb_shade_samples")(self._h, rays.ctypes.data_as(C.POINTER(C.c_double)),
+                                                  keys.ctypes.data_as(C.POINTER(C.c_uint64)) if keys is not None else None, n_pix, C.byref(p),
+                                                  out.ctypes.data_as(C.c_void_p), C.byref(dbg) if dbg else None,
+                                                  C.byref(st) if st is not None else None))
+        return dict(rgb=out, prim=prim, sub=sub, t=t, stats=st)
+
+    def shade_samples_device(self, d_rays_ptr, n_pixels, p, d_out_ptr, d_keys_ptr=0, d_dbg=None, stream=0, stats=None):
+        """shade_samples() on DEVICE memory of the current device, queued on `stream`: d_rays_ptr = n_pixels * p.spp * 6 doubles,
+        d_keys_ptr = n_pixels * p.spp uint64 (0 = the ray's index), d_out_ptr = n_pixels pixels in p.out_format, d_dbg = optional
+        (prim_ptr, sub_ptr, t_ptr) of n_pixels * p.spp entries (0 = not wanted).  Does not synchronise unless stats is given."""
+        dbg = None
+        if d_dbg is not None:
+            dbg = abi.DebugOut(C.cast(C.c_void_p(d_dbg[0] or None), C.POINTER(C.c_int32)), C.cast(C.c_void_p(d_dbg[1] or None), C.POINTER(C.c_int32)),
+                               C.cast(C.c_void_p(d_dbg[2] or None), C.POINTER(C.c_double)))
+        _check(_query_entry("ftb_shade_samples_device")(self._h, C.cast(C.c_void_p(d_rays_ptr or None), C.POINTER(C.c_double)),
+                                                         C.cast(C.c_void_p(d_keys_ptr or None), C.POINTER(C.c_uint64)), n_pixels, C.byref(p),
+                                                         C.c_void_p(d_out_ptr or None), C.byref(dbg) if dbg is not None else None,
+                                                         C.byref(stats) if stats is not None else None, C.c_void_p(stream)))
 
     # -- device-buffer entry points (one process per GPU; pointers are raw device addresses) -----
     def render_tiles_device(self, p, d_tiles_ptr, stream=0, stats=False, camera=None, d_dbg=None, window=None):

@@ -129,11 +129,13 @@ namespace ftb {
 static_assert((unsigned)FT_TABLE == kFeatOriginTable, "lower.h and device_scene.h disagree on the table feature bit");
 // kernel variants compiled by the Makefile (render_variant.cu), listed through -DFTB_FEAT_LIST_F32 / _F64
 #define X(feat) cudaError_t launch_f32_##feat(const DevScene<float>&, const DevFrame<float>&, bool, int, cudaStream_t, int*); \
-    cudaError_t query_f32_##feat(const DevScene<float>&, const DevQuery&, bool, int, cudaStream_t, int*);
+    cudaError_t query_f32_##feat(const DevScene<float>&, const DevQuery&, bool, int, cudaStream_t, int*); \
+    cudaError_t samples_f32_##feat(const DevScene<float>&, const DevFrame<float>&, const unsigned long long*, bool, int, cudaStream_t, int*);
 FTB_FEAT_LIST_F32
 #undef X
 #define X(feat) cudaError_t launch_f64_##feat(const DevScene<double>&, const DevFrame<double>&, bool, int, cudaStream_t, int*); \
-    cudaError_t query_f64_##feat(const DevScene<double>&, const DevQuery&, bool, int, cudaStream_t, int*);
+    cudaError_t query_f64_##feat(const DevScene<double>&, const DevQuery&, bool, int, cudaStream_t, int*); \
+    cudaError_t samples_f64_##feat(const DevScene<double>&, const DevFrame<double>&, const unsigned long long*, bool, int, cudaStream_t, int*);
 FTB_FEAT_LIST_F64
 #undef X
 // the crossing queries' kernel (crossings.cu): generic FEAT only, one object per precision
@@ -146,13 +148,18 @@ cudaError_t paths_f32(const DevScene<float>&, const DevPaths&, bool, int, cudaSt
 cudaError_t paths_f64(const DevScene<double>&, const DevPaths&, bool, int, cudaStream_t, int*);
 inline cudaError_t launchPaths(const DevScene<float>& s, const DevPaths& q, bool stats, int sm, cudaStream_t st, int* l) { return paths_f32(s, q, stats, sm, st, l); }
 inline cudaError_t launchPaths(const DevScene<double>& s, const DevPaths& q, bool stats, int sm, cudaStream_t st, int* l) { return paths_f64(s, q, stats, sm, st, l); }
+// ftb_frame_rays' kernel (frame_rays.cu): one object per precision
+cudaError_t frame_rays_f32(const DevFrame<float>&, long long, double*, unsigned long long*, int, cudaStream_t);
+cudaError_t frame_rays_f64(const DevFrame<double>&, long long, double*, unsigned long long*, int, cudaStream_t);
+inline cudaError_t launchFrameRays(const DevFrame<float>& f, long long n, double* r, unsigned long long* k, int sm, cudaStream_t st) { return frame_rays_f32(f, n, r, k, sm, st); }
+inline cudaError_t launchFrameRays(const DevFrame<double>& f, long long n, double* r, unsigned long long* k, int sm, cudaStream_t st) { return frame_rays_f64(f, n, r, k, sm, st); }
 static const Variant<float> kVariantsF32[] = {
-#define X(feat) {(unsigned)(feat), UnitCap<float, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f32_##feat, query_f32_##feat},
+#define X(feat) {(unsigned)(feat), UnitCap<float, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f32_##feat, query_f32_##feat, samples_f32_##feat},
     FTB_FEAT_LIST_F32
 #undef X
 };
 static const Variant<double> kVariantsF64[] = {
-#define X(feat) {(unsigned)(feat), UnitCap<double, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f64_##feat, query_f64_##feat},
+#define X(feat) {(unsigned)(feat), UnitCap<double, (unsigned)(feat)>::value, (feat) == FT_ALL, launch_f64_##feat, query_f64_##feat, samples_f64_##feat},
     FTB_FEAT_LIST_F64
 #undef X
 };
@@ -697,6 +704,19 @@ bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render
     return true;
 }
 
+// The frame's sample offsets on the device (F.jitter).  CornerSampling.generateRays (Image.fs:128-132): every corner ray uses the
+// offset (-0.5, +0.5).
+template <typename R>
+int uploadJitter(PerDevice* pd, const ftb_render_params* p, const FrameGeom& g, DevFrame<R>& F, cudaStream_t stream)
+{
+    std::vector<R> j = {R(-0.5), R(0.5)};
+    if (!g.corner) j.assign(p->jitter_xy, p->jitter_xy + 2 * (size_t)g.spp);
+    CK(pd->jitter.reserve(j.size() * sizeof(R)));
+    CK(cudaMemcpyAsync(pd->jitter.p, j.data(), j.size() * sizeof(R), cudaMemcpyHostToDevice, stream));  // pageable source: staged before return
+    F.jitter = static_cast<const R*>(pd->jitter.p);
+    return FTB_OK;
+}
+
 // Runs fn(R()) with R the real type of `precision`.
 template <typename Fn> int byPrecision(int precision, Fn&& fn) { return precision == FTB_PRECISION_FP64_VERIFY ? fn(double()) : fn(float()); }
 
@@ -738,12 +758,7 @@ struct Launch {
         F.tiles_x_magic = (g.tiles_x > 1 && (unsigned long long)g.n_tiles * (unsigned long long)g.tiles_x < (1ull << 32)) ? (unsigned)((1ull << 32) / (unsigned)g.tiles_x) + 1u : 0u;
         F.n_local_tiles = g.n_local_tiles; F.shard_index = g.shard_index; F.shard_count = g.shard_count;
         fillCamera<R>(F, *cam, p->width, p->height);
-        // CornerSampling.generateRays (Image.fs:128-132): every corner ray uses the offset (-0.5, +0.5)
-        std::vector<R> j = {R(-0.5), R(0.5)};
-        if (!g.corner) j.assign(p->jitter_xy, p->jitter_xy + 2 * (size_t)g.spp);
-        CK(pd->jitter.reserve(j.size() * sizeof(R)));
-        CK(cudaMemcpyAsync(pd->jitter.p, j.data(), j.size() * sizeof(R), cudaMemcpyHostToDevice, stream));  // pageable source: staged before return
-        F.jitter = static_cast<const R*>(pd->jitter.p);
+        if ((rc = uploadJitter<R>(pd, p, g, F, stream)) != FTB_OK) return rc;
         // tile order: cached per (camera, frame geometry, window, recursion limit, sample offsets); recomputed + uploaded only
         // when they change.  The order lists the window's local tiles: an order cached for another window would name tiles this
         // one lacks.  Which tiles are clear depends on how far the samples stray from their pixel centres.
@@ -773,8 +788,26 @@ struct Launch {
         if (stats) CK(cudaEventRecord(pd->ev0, stream));
         return FTB_OK;
     }
-    // One launch covers at most UnitCap samples per pixel; more samples = more passes over the same tiles, each continuing the
-    // left fold of the previous one (so the blend order is still Array.average's).
+    // One launch covers at most UnitCap samples per pixel; more samples = more passes over the same tiles (pixels), each continuing
+    // the left fold of the previous one (so the blend order is still Array.average's).  setPass sets up the pass that starts at
+    // sample s_base: for frames (launchChunk) and for ftb_shade_samples alike, so both cut a pixel's samples into the same passes,
+    // runs and fold segments.
+    void setPass(int s_base)
+    {
+        F.s_base = s_base;
+        F.s_count = std::min(var->unit_cap, F.spp - s_base);
+        // run length: cheap samples amortise the dealing over up to 8 consecutive samples of a pixel, as long as
+        // every pixel still splits into >= 8 runs (the chain a lane can be stuck with stays 1/8 of a pixel)
+        // Large meshes deal single samples: a traversal's cost varies so much between neighbouring samples that a lane
+        // stuck with a run of them holds its warp back (measured -11..-14 % on the 355 k mesh; +3 % on the 960-triangle
+        // one and +7 % on moon the other way).
+        const int runMax = scene->mesh_packet ? 1 : 8;
+        int run = 1;
+        while (run < runMax && F.s_count % (run * 2) == 0 && F.s_count / (run * 2) >= 8) run *= 2;
+        F.run = run;
+        const unsigned rpp = (unsigned)(F.s_count / run);
+        F.rpp_magic = rpp <= 1 ? 0u : (unsigned)((1ull << 32) / rpp) + 1u;
+    }
     // Work-queue granularity.  A lane takes runs of samples, a warp takes blocks of pixels from the atomic queue.  The block is
     // the indivisible quantum of the tail, so it shrinks (32 = 8x4 ... 1 pixel) until there are >= 24 blocks per resident
     // warp, but never below one warp-round of samples per block (and big frames keep big blocks, which also bounds the number
@@ -795,19 +828,7 @@ struct Launch {
         F.n_blocks = traced * (FTB_TILE_PIXELS / ppb);
         F.n_clear_blocks = (ntile - traced) * (FTB_TILE_PIXELS / ppb);
         for (int s_base = 0; s_base < F.spp; s_base += var->unit_cap) {
-            F.s_base = s_base;
-            F.s_count = std::min(var->unit_cap, F.spp - s_base);
-            // run length: cheap samples amortise the dealing over up to 8 consecutive samples of a pixel, as long as
-            // every pixel still splits into >= 8 runs (the chain a lane can be stuck with stays 1/8 of a pixel)
-            // Large meshes deal single samples: a traversal's cost varies so much between neighbouring samples that a lane
-            // stuck with a run of them holds its warp back (measured -11..-14 % on the 355 k mesh; +3 % on the 960-triangle
-            // one and +7 % on moon the other way).
-            const int runMax = scene->mesh_packet ? 1 : 8;
-            int run = 1;
-            while (run < runMax && F.s_count % (run * 2) == 0 && F.s_count / (run * 2) >= 8) run *= 2;
-            F.run = run;
-            const unsigned rpp = (unsigned)(F.s_count / run);
-            F.rpp_magic = rpp <= 1 ? 0u : (unsigned)((1ull << 32) / rpp) + 1u;
+            setPass(s_base);
             CK(pd->control.resetQueue(stream));
             CK(launchKernel(stream));
             if (F.n_clear_blocks > 0) {
@@ -1273,6 +1294,171 @@ int pathsHost(ftb_scene* sc, const double* rays, const uint64_t* keys, int64_t n
     return FTB_OK;
 }
 
+// ---- a frame's own samples: ftb_frame_rays and ftb_shade_samples ----------------------------------------------------------
+// ftb_frame_rays reads width, height, spp, sampling, jitter_xy, precision and seed; the window and those fields are checked as
+// ftb_render_window checks them (frameGeom), the fields it does not read are not.  Then the device count: everything a caller can
+// get wrong is reported before any device is looked for.
+int checkFrameRays(const ftb_scene* sc, const ftb_camera* cam, const ftb_render_params* p, const Window& win, FrameGeom& g)
+{
+    if (!sc || !cam || !p) return fail(FTB_ERR_BAD_ARG, "null argument");
+    ftb_render_params q = *p;
+    q.out_format = FTB_OUT_RGB_F64; q.shard_index = q.shard_count = 0; q.band_index = q.band_count = 0; q.n_gpus = 0;
+    int rc = frameGeom(&q, g, &win);
+    if (rc != FTB_OK) return rc;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device: functracer_b200 has no CPU path"); }
+    return FTB_OK;
+}
+
+// The device entry point: the window's rays and keys (device pointers, either may be null) queued on `s` on the current device.
+int frameRaysDevice(ftb_scene* sc, const ftb_camera* cam, const ftb_render_params* p, const Window& win, double* rays, uint64_t* keys, cudaStream_t s)
+{
+    FrameGeom g;
+    int rc = checkFrameRays(sc, cam, p, win, g);
+    if (rc != FTB_OK) return rc;
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    return byPrecision(p->precision, [&](auto r) -> int {
+        typedef decltype(r) R;
+        DevFrame<R> F;  // the fields primaryRay reads, filled as prepareFrame fills them
+        std::memset(&F, 0, sizeof(F));
+        F.gw = g.gw; F.gh = g.gh; F.spp = g.spp; F.seed = p->seed;
+        F.wx0 = g.wx0; F.wy0 = g.wy0; F.wx1 = g.wx0 + g.ww; F.wy1 = g.wy0 + g.wh;
+        fillCamera<R>(F, *cam, p->width, p->height);
+        int e = uploadJitter<R>(pd, p, g, F, s);
+        if (e != FTB_OK) return e;
+        CK(launchFrameRays(F, g.n_samples, rays, reinterpret_cast<unsigned long long*>(keys), pd->sm_count, s));
+        return FTB_OK;
+    });
+}
+
+// The host entry point: the device entry into scratch on the scene's stream, then the downloads.  Synchronous.
+int frameRaysHost(ftb_scene* sc, const ftb_camera* cam, const ftb_render_params* p, const Window& win, double* rays, uint64_t* keys)
+{
+    FrameGeom g;
+    int rc = checkFrameRays(sc, cam, p, win, g);
+    if (rc != FTB_OK) return rc;
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    const cudaStream_t s = pd->stream;
+    const size_t n = (size_t)g.n_samples;
+    if (rays) CK(pd->rays.reserve(n * 48));
+    if (keys) CK(pd->query.reserve(n * 8));
+    rc = frameRaysDevice(sc, cam, p, win, rays ? static_cast<double*>(pd->rays.p) : nullptr, keys ? static_cast<uint64_t*>(pd->query.p) : nullptr, s);
+    if (rc != FTB_OK) return rc;
+    if (rays) CK(cudaMemcpyAsync(rays, pd->rays.p, n * 48, cudaMemcpyDeviceToHost, s));
+    if (keys) CK(cudaMemcpyAsync(keys, pd->query.p, n * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    return FTB_OK;
+}
+
+inline size_t pixelBytes(int out_format) { return out_format == FTB_OUT_RGB_F64 ? 24 : (out_format == FTB_OUT_RGB_F32 ? 12 : 4); }
+
+// ftb_shade_samples' arguments, then the device count: everything a caller can get wrong is reported before any device is looked
+// for.  The pixel count is also bounded: the kernel indexes pixels with 32-bit integers.
+int checkSamples(const ftb_scene* sc, const double* rays, int64_t n_pixels, const ftb_render_params* p, const void* out)
+{
+    if (!sc || !p || n_pixels < 0 || (n_pixels > 0 && (!rays || !out))) return fail(FTB_ERR_BAD_ARG, "null argument or negative pixel count");
+    if (p->spp < 1) return fail(FTB_ERR_BAD_ARG, "spp < 1");
+    if (n_pixels > 0x7fffff00LL || n_pixels > (int64_t)FTB_TILE_PIXELS * 0x7fffff00LL / 2 / p->spp) return fail(FTB_ERR_BAD_ARG, "too many samples");
+    if (p->precision != FTB_PRECISION_FP32 && p->precision != FTB_PRECISION_FP64_VERIFY) return fail(FTB_ERR_BAD_ARG, "bad precision");
+    if (p->out_format < FTB_OUT_RGB_F64 || p->out_format > FTB_OUT_RGBA8) return fail(FTB_ERR_BAD_ARG, "bad output format");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { (void)cudaGetLastError(); return fail(FTB_ERR_NO_DEVICE, "no CUDA device: functracer_b200 has no CPU path"); }
+    return FTB_OK;
+}
+
+// Queues one batch on `s` (n_pixels > 0, arguments checked): the passes of samples_kernel with the variant the scene's frames run
+// (ftb_shade_rays' choice), then the conversion into pd->out.  The flat pixel buffer is the tile buffer of a 16-pixel-wide frame
+// of ceil(n / 16) rows (pixel i is (i % 16, i / 16) there), so assemble_kernel writes the pixels in order in out_format; pd->out
+// holds the first n_pixels of them when the queued work is done.
+int samplesLaunch(ftb_scene* sc, PerDevice* pd, const double* rays, const uint64_t* keys, int64_t n_pixels, const ftb_render_params* p,
+                  const ftb_debug_out* dbg, ftb_stats* stats, cudaStream_t s)
+{
+    const int rows = (int)((n_pixels + FTB_TILE_W - 1) / FTB_TILE_W);
+    CK(pd->tiles.reserve((size_t)rows * FTB_TILE_W * 3 * realSize(p->precision)));
+    CK(pd->out.reserve((size_t)rows * FTB_TILE_W * pixelBytes(p->out_format)));
+    FrameGeom fg;
+    std::memset(&fg, 0, sizeof(fg));
+    fg.width = FTB_TILE_W; fg.height = rows; fg.tiles_x = 1; fg.shard_count = 1;
+    return byPrecision(p->precision, [&](auto r) -> int {
+        Launch<decltype(r)> fr;
+        int e = fr.begin(sc, pd, p, sc->L.features, stats && p->collect_stats, pd->tiles.p, dbg);
+        if (e != FTB_OK) return e;
+        CK(pd->control.prepare(fr.counting, s));
+        auto& F = fr.F;
+        F.mode = 2; F.spp = p->spp; F.n_rays = n_pixels; F.n_blocks = (int)((n_pixels + 31) / 32); F.rays = rays; F.shard_count = 1;
+        if (stats) CK(cudaEventRecord(pd->ev0, s));
+        for (int s_base = 0; s_base < F.spp; s_base += fr.var->unit_cap) {
+            fr.setPass(s_base);
+            CK(pd->control.resetQueue(s));
+            CK(fr.var->samples(*fr.scene, F, reinterpret_cast<const unsigned long long*>(keys), fr.counting, pd->sm_count, s, &fr.launches));
+        }
+        if (stats) { CK(cudaEventRecord(pd->ev1, s)); stats->kernel_launches += fr.launches + 2; }  // + the control-block memset and the assembly
+        const void* bufs[1] = {pd->tiles.p};
+        return launchAssemble(p, fg, bufs, pd->out.p, s, 0, rows);
+    });
+}
+
+// The device entry point: device pointers, queued on `s`; synchronises only to fill stats.
+int samplesDevice(ftb_scene* sc, const double* rays, const uint64_t* keys, int64_t n_pixels, const ftb_render_params* p, void* out,
+                  const ftb_debug_out* dbg, ftb_stats* stats, cudaStream_t s)
+{
+    int rc = checkSamples(sc, rays, n_pixels, p, out);
+    if (rc != FTB_OK) return rc;
+    if (stats) std::memset(stats, 0, sizeof(*stats));
+    if (n_pixels == 0) return FTB_OK;
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    if ((rc = samplesLaunch(sc, pd, rays, keys, n_pixels, p, dbg && dbg->prim_id ? dbg : nullptr, stats, s)) != FTB_OK) return rc;
+    CK(cudaMemcpyAsync(out, pd->out.p, (size_t)n_pixels * pixelBytes(p->out_format), cudaMemcpyDeviceToDevice, s));
+    bool overflow = false;
+    if (stats && (rc = finishStats(sc, pd, stats, s, &overflow)) != FTB_OK) return rc;
+    return overflow ? overflowError() : FTB_OK;
+}
+
+// The host entry point, the pattern of pathsHost: upload the rays and keys, queue the batch, read the control block back, and only
+// then download the pixels and the requested debug planes: on an overflow nothing of the caller's is written.  Synchronous.
+int samplesHost(ftb_scene* sc, const double* rays, const uint64_t* keys, int64_t n_pixels, const ftb_render_params* p, void* out,
+                const ftb_debug_out* dbg, ftb_stats* stats)
+{
+    const auto t0 = std::chrono::steady_clock::now();
+    int rc = checkSamples(sc, rays, n_pixels, p, out);
+    if (rc != FTB_OK || n_pixels == 0) return rc != FTB_OK ? rc : samplesDevice(sc, rays, keys, n_pixels, p, out, nullptr, stats, nullptr);
+    PerDevice* pd = nullptr;
+    if ((rc = currentDevice(sc, &pd)) != FTB_OK) return rc;
+    if (stats) std::memset(stats, 0, sizeof(*stats));
+    const cudaStream_t s = pd->stream;
+    const size_t n = (size_t)n_pixels * (size_t)p->spp;  // rays
+    CK(pd->rays.reserve(n * 48));
+    CK(cudaMemcpyAsync(pd->rays.p, rays, n * 48, cudaMemcpyHostToDevice, s));
+    if (keys) {
+        CK(pd->query.reserve(n * 8));
+        CK(cudaMemcpyAsync(pd->query.p, keys, n * 8, cudaMemcpyHostToDevice, s));
+    }
+    ftb_debug_out d = {nullptr, nullptr, nullptr};
+    if (dbg && dbg->prim_id) {
+        CK(pd->dbg_prim.reserve(n * 4)); d.prim_id = static_cast<int32_t*>(pd->dbg_prim.p);
+        if (dbg->sub_id) { CK(pd->dbg_sub.reserve(n * 4)); d.sub_id = static_cast<int32_t*>(pd->dbg_sub.p); }
+        if (dbg->t) { CK(pd->dbg_t.reserve(n * 8)); d.t = static_cast<double*>(pd->dbg_t.p); }
+    }
+    rc = samplesLaunch(sc, pd, static_cast<const double*>(pd->rays.p), keys ? static_cast<const uint64_t*>(pd->query.p) : nullptr, n_pixels, p,
+                       d.prim_id ? &d : nullptr, stats, s);
+    if (rc != FTB_OK) return rc;
+    bool overflow = false;
+    if ((rc = finishStats(sc, pd, stats, s, &overflow)) != FTB_OK) return rc;
+    if (overflow) return overflowError();
+    CK(cudaMemcpyAsync(out, pd->out.p, (size_t)n_pixels * pixelBytes(p->out_format), cudaMemcpyDeviceToHost, s));
+    if (d.prim_id) {
+        CK(cudaMemcpyAsync(dbg->prim_id, d.prim_id, n * 4, cudaMemcpyDeviceToHost, s));
+        if (d.sub_id) CK(cudaMemcpyAsync(dbg->sub_id, d.sub_id, n * 4, cudaMemcpyDeviceToHost, s));
+        if (d.t) CK(cudaMemcpyAsync(dbg->t, d.t, n * 8, cudaMemcpyDeviceToHost, s));
+    }
+    CK(cudaStreamSynchronize(s));
+    if (stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return FTB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1645,6 +1831,30 @@ int ftb_trace_paths_device(ftb_scene* scene, const double* d_rays_od, const uint
                            const ftb_path_out* d_out, ftb_stats* stats, void* stream)
 {
     return pathsDevice(scene, d_rays_od, d_sample_keys, n, params, d_out, stats, static_cast<cudaStream_t>(stream));
+}
+
+int ftb_frame_rays(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params, int32_t x0, int32_t y0, int32_t x1, int32_t y1,
+                   double* rays_od, uint64_t* sample_keys)
+{
+    return frameRaysHost(scene, camera, params, Window{x0, y0, x1, y1}, rays_od, sample_keys);
+}
+
+int ftb_frame_rays_device(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params, int32_t x0, int32_t y0, int32_t x1, int32_t y1,
+                          double* d_rays_od, uint64_t* d_sample_keys, void* stream)
+{
+    return frameRaysDevice(scene, camera, params, Window{x0, y0, x1, y1}, d_rays_od, d_sample_keys, static_cast<cudaStream_t>(stream));
+}
+
+int ftb_shade_samples(ftb_scene* scene, const double* rays_od, const uint64_t* sample_keys, int64_t n_pixels, const ftb_render_params* params,
+                      void* out, const ftb_debug_out* dbg, ftb_stats* stats)
+{
+    return samplesHost(scene, rays_od, sample_keys, n_pixels, params, out, dbg, stats);
+}
+
+int ftb_shade_samples_device(ftb_scene* scene, const double* d_rays_od, const uint64_t* d_sample_keys, int64_t n_pixels, const ftb_render_params* params,
+                             void* d_out, const ftb_debug_out* d_dbg, ftb_stats* stats, void* stream)
+{
+    return samplesDevice(scene, d_rays_od, d_sample_keys, n_pixels, params, d_out, d_dbg, stats, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

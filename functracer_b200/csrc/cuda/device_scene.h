@@ -139,7 +139,7 @@ struct DevScene {
 
 template <typename R>
 struct DevFrame {
-    int mode;  // 0 = camera sample grid, 1 = explicit ray list
+    int mode;  // 0 = camera sample grid, 1 = explicit ray list (render_kernel); samples_kernel: explicit rays, spp per pixel (2)
     int gw, gh;  // the whole frame's sample grid (W x H, or (W+1) x (H+1) in corner mode): ray directions and RNG keys
     int spp;              // samples per pixel of the whole frame
     int s_base, s_count;  // this launch renders samples [s_base, s_base + s_count) of every pixel (s_count <= UnitCap)
@@ -285,6 +285,9 @@ struct Variant {
     bool has_stats;  // the counting kernel is only compiled into the FT_ALL variants
     cudaError_t (*launch)(const DevScene<R>& s, const DevFrame<R>& f, bool stats, int sm_count, cudaStream_t stream, int* launches);
     cudaError_t (*query)(const DevScene<R>& s, const DevQuery& q, bool stats, int sm_count, cudaStream_t stream, int* launches);
+    // samples_kernel (ftb_shade_samples): f in mode 2, f.n_rays pixels of f.spp rays each; keys may be null (the rays' indices)
+    cudaError_t (*samples)(const DevScene<R>& s, const DevFrame<R>& f, const unsigned long long* keys, bool stats, int sm_count, cudaStream_t stream,
+                           int* launches);
 };
 
 }  // namespace ftb

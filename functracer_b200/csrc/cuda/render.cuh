@@ -1851,6 +1851,354 @@ cudaError_t launch_render_impl(const DevScene<R>& s, const DevFrame<R>& f, bool 
     return cudaGetLastError();
 }
 
+// ---- sample shading (ftb_shade_samples: explicit rays, spp samples per pixel, blended as a frame blends them) -------------
+// render_kernel with a third mode, F.mode = 2: F.n_rays pixels of F.spp explicit rays each.  Sample s of pixel i is ray i * spp + s
+// with RNG key keys[i * spp + s] (keys == nullptr: i * spp + s), and its debug entry is i * spp + s.  Warps take 32 pixels at a
+// time from the per-device queue as mode 1 takes 32 rays (the pixels are flat: a block is one row of 32), and deal them in mode
+// 0's passes, runs and units, so foldUnit folds every pixel with the segmentation a frame of that spp and variant uses.
+// A kernel of its own, so that render_kernel's code stays exactly what it is (its register allocation moves with any edit to the
+// code it inlines, DESIGN.md §8).  And a copy of render_kernel's body with only the lines of mode 2 changed, mode 0's code kept
+// although mode 2 never runs it: in FP32 the compiler's choice of fused multiply-adds inside the inlined trace and shading code
+// depends on the code around it, and a copy pared down to mode 2 rounded some hit distances of the house scene one ulp apart from
+// the frame's.  Kept this way, the trace and shading compile to the same instructions as render_kernel's (DESIGN.md §3).
+template <typename R, unsigned FEAT, bool STATS>
+__global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) samples_kernel(const __grid_constant__ DevScene<R> S, const __grid_constant__ DevFrame<R> F,
+                                                                                        const unsigned long long* keys)
+{
+    typedef typename V4<R>::type R4;
+    constexpr int CAP = UnitCap<R, FEAT>::value;
+    constexpr int WARPS = kBlockThreads / 32;
+    __shared__ R ring_col[WARPS][kRingSlots][CAP * 3];
+    constexpr bool kTable = FTB_FAST_BOUNDS != 0 && (FEAT & FT_TABLE) != 0;
+    __shared__ int ring_hdr[WARPS][kRingSlots][4];  // out slot of the block's pixel 0, block width, first pixel, pixel count
+    __shared__ int mesh_stack[MeshWalks<FEAT>::kPacket ? WARPS : 1][MeshWalks<FEAT>::kPacket ? kBspStack : 1];  // packetMesh: one walk per warp
+    __shared__ R4 origin_tab[kTable ? kOriginCap : 1];
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const unsigned lt_mask = (1u << lane) - 1u;
+    Counters<STATS> cn;
+
+    // Common-origin bound table.  Most rays start at one of a handful of points: primary rays at the camera, shadow rays
+    // (traced from the fragment towards the light) end at a point light.  For such a ray the object-level bound test
+    // "the line passes within r of the centre and the bound is not behind the origin" is b >= sqrt(|oc|^2 - r^2) with
+    // b = oc . unit(d): the right-hand side depends on (origin, item) only.  Row 0 = camera, row 1 + l = light l (sign
+    // flipped, the ray points at it; a crossing between fragment and light is ahead of the light looking back).
+    // Like the general form the test may keep a miss but never drops a hit.  Rounding budget (tests/test_bound_table_budget.py
+    // replays it in float32 against exact geometry): (1) in FP32 b is off by <= 4.8e-7 |oc| (rsqrt 2 ulp, three products), the
+    // row's |oc|^2 by 3.6e-7 |oc|^2 and the approximate sqrt moves the threshold by 2 ulp: together < 1.8e-6 |oc|^2 of the
+    // 8e-6 |oc|^2 slack in the threshold.  (2) The traced line does not pass exactly through the common point: a primary ray
+    // starts at fl(camera + 1e-4 d), g <= 1e-7 |camera| off the ideal line; a shadow ray's rounded direction (fl(L - P)
+    // normalised: 1.7e-7 rad) misses the light by g <= 1.7e-7 tmax.  An offset g changes |oc|^2 - b^2 by <= 2 |oc| g + g^2,
+    // of which the remaining 6e-6 |oc|^2 of the threshold slack absorbs all but 2 |oc| g - 6e-6 |oc|^2 <= g^2 / 6e-6 (the
+    // maximum over |oc|): adding sqrt(g^2 / 6e-6) = 410 g to b covers it for every item, i.e. 4.1e-5 |camera| resp.
+    // 7e-5 tmax.  The per-ray slack actually added is 2e-4 |camera| for primary rays and 4e-4 tmax for shadow rays (5x).
+    // -inf = always a candidate (unbounded, or the origin inside the bound).
+    const bool fastBounds = kTable && originTableFits(S);
+    const bool fastPrimary = fastBounds && F.mode == 0 && !((FEAT & FT_RNG) != 0 && F.has_focus);
+    if (fastBounds) buildOriginTable<R>(S, F, origin_tab);
+    bool overflow = false;
+
+    // warp-uniform cursors: the pixel block (or 32 rays) taken from the per-GPU queue, and the unit being dealt from it
+    int blk_slot0 = 0, blk_x0 = 0, blk_y0 = 0, blk_w = 1, blk_npix = 0, blk_pos = 0;
+    int u_slot = 0, u_p0 = 0, u_pos = 0, u_n = 0;  // u_pos / u_n count RUNS of F.run consecutive samples of one pixel
+    int remaining[kRingSlots];
+    bool busy[kRingSlots];
+#pragma unroll
+    for (int k = 0; k < kRingSlots; ++k) { remaining[k] = 0; busy[k] = false; }
+    bool exhausted = false;
+
+    // per-lane sample / path state
+    // where this lane's sample is parked, in one register (the kernel is register-bound: every register saved is a spill less):
+    // bits 0..11 = position in the slot, bits 12..15 = ring slot, bits 16.. = samples left in this lane's run
+    int rpos = 0;
+    int px = 0, py = 0, sj = 0;      // pixel, sample index within the pixel
+    // Index of the sample in the reference's full-frame ray list (RNG key, explicit-ray index), also in a window.  Variants
+    // with in-path randomness carry it (two registers); nothing else needs it.
+    constexpr bool kCarryIndex = (FEAT & FT_RNG) != 0;
+    unsigned long long sampleIndex = 0;
+    bool retire = false;             // a sample of this lane finished in the previous iteration (for the unit's count)
+    Vec<R> scol = mk<R>(R(0), R(0), R(0));
+    int phase = PH_IDLE, limit = 0;  // limit: bounces left; the bounce depth (RNG key) is recursion_limit - limit
+    R weight = R(1), tmax = R(0);
+    Ray<R> ray;            // the ray to trace next: path ray (un-offset) in PH_NEAREST, shadow ray in PH_SHADOW
+    Vec<R> pathD;          // direction of the current path ray (viewRay.d of the fragment being shaded)
+    ray.o = mk<R>(R(0), R(0), R(0)); ray.d = ray.o; pathD = ray.o;
+    Fragment<R> f;
+    f.p = ray.o; f.n = ray.o; f.colour = ray.o; f.roughness = f.reflectance = f.shineyness = R(0); f.applyLighting = false;
+    Vec<R> local = ray.o;  // sum over lights at the current level
+    int li = 0, sk = 0, occluded = 0;
+    const int scount = F.mode != 1 ? F.s_count : 1;  // samples per pixel in this pass
+    const int spp = F.mode != 1 ? F.spp : 1;          // samples per pixel of the frame
+    const int run = F.mode != 1 ? F.run : 1;          // consecutive samples of one pixel a lane takes at a time (divides scount)
+    const int rpp = scount / run;                     // runs per pixel
+    const int ppu = max(1, min(32, CAP / scount));    // pixels per unit
+    const int foldQuads = (sizeof(R) == 4 && ppu <= 2) ? 1 : 0;  // see foldUnit
+
+    for (;;) {
+        // ---- fold units whose last sample has landed (colours were parked when each path ended) ---------------------
+        if (__any_sync(full, retire)) {
+            __syncwarp();  // the parked colours of every lane are visible to the lanes that fold
+            unsigned doneSlots = 0;
+#pragma unroll
+            for (int k = 0; k < kRingSlots; ++k) {
+                remaining[k] -= __popc(__ballot_sync(full, retire && ((rpos >> 12) & 0xf) == k));
+                if (busy[k] && remaining[k] == 0) { doneSlots |= 1u << k; busy[k] = false; }
+            }
+            while (doneSlots) {  // rare relative to the trace: one out-of-line copy keeps the hot loop small
+                const int k = __ffs(doneSlots) - 1;
+                doneSlots &= doneSlots - 1;
+                foldUnit<R>(&ring_col[wib][k][0], &ring_hdr[wib][k][0], F.out, scount, spp, F.s_base, lane, foldQuads);
+            }
+            retire = false;
+            __syncwarp();
+        }
+        // ---- deal runs of samples to idle lanes (ballot + popc = warp scan) -------------------------------------------
+        bool need = phase == PH_IDLE;
+        unsigned m = __ballot_sync(full, need);
+        while (m && !exhausted) {
+            if (u_pos >= u_n) {  // open the next unit
+                int freeSlot = -1;
+#pragma unroll
+                for (int k = kRingSlots - 1; k >= 0; --k) if (!busy[k]) freeSlot = k;
+                if (freeSlot < 0) break;  // every slot still has a sample in flight: idle lanes wait one iteration
+                if (blk_pos >= blk_npix) {  // the warp takes the next pixel block (32 rays) from the per-GPU queue
+                    unsigned c = 0;
+                    if (lane == 0) c = atomicAdd(F.tile_counter, 1u);
+                    c = __shfl_sync(full, c, 0);
+                    if (c >= (unsigned)F.n_blocks) { exhausted = true; break; }
+                    blk_pos = 0;
+                    if (F.mode == 0) {
+                        openBlock<R>(F, c, blk_slot0, blk_x0, blk_y0, blk_w, blk_npix);
+                    } else {
+                        const long long first = (long long)c * 32;
+                        blk_slot0 = (int)first;
+                        blk_w = 32;
+                        blk_npix = (int)min(32LL, F.n_rays - first);
+                    }
+                    if (blk_npix <= 0) continue;
+                }
+                const int np = min(ppu, blk_npix - blk_pos);
+                u_slot = freeSlot; u_p0 = blk_pos; u_pos = 0; u_n = np * rpp;
+                blk_pos += np;
+#pragma unroll
+                for (int k = 0; k < kRingSlots; ++k) if (k == freeSlot) { busy[k] = true; remaining[k] = np * scount; }
+                if (lane == 0) {
+                    ring_hdr[wib][u_slot][0] = blk_slot0; ring_hdr[wib][u_slot][1] = blk_w; ring_hdr[wib][u_slot][2] = u_p0; ring_hdr[wib][u_slot][3] = np;
+                }
+            }
+            const int rank = __popc(m & lt_mask);
+            const int avail = u_n - u_pos;
+            if (need && rank < avail) {
+                const int q = u_pos + rank;                                      // run index within the unit
+                const int pu = rpp == 1 ? q : (int)__umulhi((unsigned)q, F.rpp_magic);  // pixel within the unit = q / rpp
+                const int pj = u_p0 + pu;                                        // pixel within the block
+                sj = F.s_base + (q - pu * rpp) * run;
+                rpos = (q * run) | (u_slot << 12) | (run << 16);
+                if (F.mode == 0) {
+                    const int ly = blk_w == 8 ? (pj >> 3) : pj / blk_w;
+                    px = blk_x0 + (pj - ly * blk_w); py = blk_y0 + ly;
+                    if constexpr (kCarryIndex) sampleIndex = ((unsigned long long)py * (unsigned)F.gw + (unsigned)px) * (unsigned)spp + (unsigned)sj;
+                } else {
+                    px = blk_slot0 + pj; py = 0;  // the ray's index
+                    if constexpr (kCarryIndex) sampleIndex = (unsigned long long)(unsigned)px;
+                }
+                phase = PH_START;
+                need = false;
+            }
+            u_pos += min(__popc(m), avail);
+            m = __ballot_sync(full, need);
+        }
+        if (phase == PH_START) {  // a new sample: dealt just now, or the next one of this lane's run
+            if (F.mode == 0) ray = primaryRay<R, FEAT>(F, px, py, sj, sampleIndex);
+            else {  // mode 2: sample sj of pixel px is ray px * spp + sj, with RNG key keys[that] (nullptr: the ray's index)
+                const size_t ri = (size_t)(unsigned)px * (unsigned)spp + (unsigned)sj;
+                if constexpr (kCarryIndex) sampleIndex = keys ? __ldg(keys + ri) : (unsigned long long)ri;
+                const double* q = F.rays + 6 * ri;
+                ray.o = mk<R>((R)__ldg(q), (R)__ldg(q + 1), (R)__ldg(q + 2));
+                ray.d = mk<R>((R)__ldg(q + 3), (R)__ldg(q + 4), (R)__ldg(q + 5));
+            }
+            phase = PH_NEAREST; limit = F.recursion_limit; weight = R(1);
+            scol = mk<R>(R(0), R(0), R(0));
+            cn.add(ST_PRIMARY);
+        }
+        if (!__any_sync(full, phase != PH_IDLE)) break;
+        // Phase alignment.  A warp whose lanes are in different phases runs every iteration at the pace of its slowest kind
+        // of work (a nearest-hit query on a mesh walks ~60 BVH nodes, a shadow query ~10, a miss none) and diverges in
+        // the result handling below.  Shadow-phase lanes go first and nearest-phase lanes hold for that iteration, so
+        // the lanes of a warp fall into step: everyone traces primary / bounce rays together, then everyone traces
+        // shadow rays together.  Scheduling only: a held lane traces the same ray one iteration later.
+        // Measured: -28 % on the full-size mesh, -12 % house, -8 % night-house, -5 % moon, +-0 cfg2.
+        bool hold = false;
+        if constexpr (FTB_PHASE_ALIGN != 0) hold = __any_sync(full, phase == PH_SHADOW) && phase == PH_NEAREST;
+        // all lanes that trace in this iteration have a row in the common-origin table?  (warp-uniform)
+        bool tabled = false;
+        if (fastBounds) {
+            const bool mine = phase == PH_NEAREST ? (fastPrimary && limit == F.recursion_limit) : tmax < realmax_<R>();  // finite tmax: a point light
+            tabled = !__any_sync(full, phase != PH_IDLE && !hold && !mine);
+        }
+        unsigned tracing = full;  // variants with the packet walk: the lanes that trace a ray in this iteration
+        if constexpr (MeshWalks<FEAT>::kPacket) tracing = __ballot_sync(full, !(phase == PH_IDLE || hold));
+        if (phase == PH_IDLE || hold) continue;
+
+        // ---- trace this lane's current ray: the one expensive step ------------------------------------------------
+        Ray<R> tr = ray;
+        if (phase == PH_NEAREST) {  // slightOffset (Shading.fs:129): d is NOT normalised
+            tr.o = ray.o + R(0.0001) * ray.d;
+            pathD = ray.d;
+        } else cn.add(ST_SHADOW);
+        // FP32 build: a ray that starts on a top-level plane / square / circle and heads away from it has no crossing with
+        // that leaf at t >= 0 (the reference's 1e-4 offsets put the only crossing at t < 0).  Far from the origin FP32 cannot
+        // represent those offsets (at the horizon of a ground plane 1e-4 * d.y ~ 1e-8 next to |y| ~ 2), the crossing lands
+        // on t = 0 or beyond and the plane reflects / shadows itself.  Such rays skip that one leaf; nothing else changes.
+        int skipLeaf = -1;
+        if constexpr (sizeof(R) == 4 && (FEAT & FT_PLANAR) != 0) {  // `f` is still the fragment this bounce / shadow ray starts from
+            if (f.planarLeaf >= 0 && (phase == PH_NEAREST ? limit < F.recursion_limit : dot(ray.d, f.n) >= R(0))) skipLeaf = f.planarLeaf;
+        }
+        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, tr, phase == PH_NEAREST ? inf_<R>() : tmax, phase == PH_SHADOW, skipLeaf,
+                                                        tabled ? origin_tab + (phase == PH_NEAREST ? 0 : 1 + li) * tabStride(S.n_items) : nullptr,
+                                                        phase == PH_NEAREST ? F.primary_slack : R(4e-4) * tmax,
+                                                        overflow, cn, tracing, &mesh_stack[MeshWalks<FEAT>::kPacket ? wib : 0][0]);
+
+        // ---- consume the result -----------------------------------------------------------------------------------------
+        bool got = false;       // an intensity for light `li` is ready
+        R intensity = R(0);
+        if (phase == PH_NEAREST) {
+            if (limit == F.recursion_limit && F.dbg_prim) {
+                int prim = -1, sub = 0;
+                if (h.leaf >= 0) {
+                    const int4 meta = __ldg(S.leaf_meta + h.leaf);
+                    const int kind = meta.x & 0xff;
+                    prim = meta.z;
+                    sub = (kind == LEAF_CUBE || kind == LEAF_MESH || kind == LEAF_SOLIDCYL) ? h.sub : ((kind == LEAF_TRIANGLE) ? 0 : meta.w);
+                }
+                const unsigned long long at = F.mode == 0 ? ((unsigned long long)(unsigned)(py - F.wy0) * (unsigned)F.dbg_w + (unsigned)(px - F.wx0)) * (unsigned)spp + (unsigned)sj
+                                                          : (unsigned long long)(unsigned)px * (unsigned)spp + (unsigned)sj;
+                F.dbg_prim[at] = prim;
+                if (F.dbg_sub) F.dbg_sub[at] = sub;
+                if (F.dbg_t) F.dbg_t[at] = h.leaf >= 0 ? (double)h.t : -1.0;
+            }
+            if (h.leaf < 0 || S.n_lights <= 0) {  // miss: empty sum (Shading.fs:137-139)
+                R* c = &ring_col[wib][0][3 * (((rpos >> 12) & 0xf) * CAP + (rpos & 0xfff))];
+                c[0] = scol.x; c[1] = scol.y; c[2] = scol.z;
+                retire = true;
+                rpos -= 0xffff;  // one sample fewer in the run, one position further
+                if ((rpos >> 16) > 0) { ++sj; if constexpr (kCarryIndex) ++sampleIndex; phase = PH_START; } else phase = PH_IDLE;
+                continue;
+            }
+            cn.add(ST_SHADED);
+            f = finalise<R, FEAT>(S, tr, h);
+            local = mk<R>(R(0), R(0), R(0));
+            li = 0;
+            ray.o = f.p + R(0.0001) * f.n;  // shadowRayOrigin (Shading.fs:111), the same for every light
+        } else {
+            const bool blocked = h.leaf >= 0;
+            const int2 lk = __ldg(S.light_i + li);
+            if (lk.x == FTB_LIGHT_SOFT_DIRECTIONAL) {  // softShadowLightIntensity (Shading.fs:24-31)
+                if constexpr ((FEAT & FT_RNG) != 0) {
+                    occluded += blocked ? 1 : 0;
+                    ++sk;
+                    if (sk < lk.y) {
+                        const R4 la = ldg4<R>(S.light_a + li);
+                        ray.d = jitterVector<R>(F.seed, sampleIndex, (unsigned)(F.recursion_limit - limit), (unsigned)li, (unsigned)sk, la.w, -mk<R>(la.x, la.y, la.z));
+                        continue;  // next sample of the same light
+                    }
+                    intensity = (R)(lk.y - occluded) / (R)lk.y;
+                }
+            } else if (lk.x == FTB_LIGHT_POINT) {
+                const R4 lb = ldg4<R>(S.light_b + li);
+                intensity = blocked ? R(0) : R(1) / (lb.x + tmax * (lb.y + tmax * lb.z));  // Light.attenuate (Light.fs:16-17)
+            } else {
+                intensity = blocked ? R(0) : R(1);
+            }
+            got = true;
+        }
+        // advance through the lights until one needs a shadow ray or the level is complete
+        for (;;) {
+            if (got) { local = local + shadeLight<R, FEAT>(S, f, pathD, li, intensity); ++li; got = false; }
+            if (li >= S.n_lights) break;
+            // fragments whose colour ignores the light's intensity need no shadow ray: unlit surfaces
+            // (shadeIfRequired) and Oren-Nayar surfaces without a specular term (Shading.fs:50-63, 85-86)
+            bool needShadow = f.applyLighting;
+            if constexpr ((FEAT & FT_ROUGH) != 0) needShadow = needShadow && !(f.roughness != R(0) && !(f.shineyness > R(0)));
+            if (!needShadow) { intensity = R(1); got = true; continue; }
+            const int2 lk = __ldg(S.light_i + li);
+            if constexpr (sizeof(R) == 4 && (FEAT & FT_PLANAR) != 0) {
+                // A primary fragment on the ground of a lit tile (lit_tiles.h): the host proved this directional light's shadow
+                // rays unblocked, so their traced intensity would be 1 exactly ((n - 0) / n for a soft light).  Counted as traced.
+                if (F.lit_tiles && li < 8 && limit == F.recursion_limit && f.planarLeaf == F.lit_leaf && lk.x != FTB_LIGHT_POINT &&
+                    ((__ldg(F.lit_tiles + ((py - F.wy0) / FTB_TILE_H) * F.tiles_x + (px - F.wx0) / FTB_TILE_W) >> li) & 1)) {
+                    cn.add(ST_SHADOW, lk.x == FTB_LIGHT_SOFT_DIRECTIONAL ? (unsigned)lk.y : 1u);
+                    intensity = R(1); got = true; continue;
+                }
+            }
+            const R4 la = ldg4<R>(S.light_a + li);
+            const Vec<R> lv = mk<R>(la.x, la.y, la.z);
+            if (lk.x == FTB_LIGHT_POINT) {  // shadowLightIntensity (Shading.fs:33-42)
+                const Vec<R> dvec = lv - ray.o;
+                tmax = length(dvec);
+                ray.d = normalise(dvec);
+            } else if (lk.x == FTB_LIGHT_SOFT_DIRECTIONAL) {
+                if (lk.y <= 0) { intensity = (R)(lk.y - 0) / (R)lk.y; got = true; continue; }  // 0/0: NaN like the reference
+                if constexpr ((FEAT & FT_RNG) != 0) {
+                    sk = 0; occluded = 0;
+                    tmax = realmax_<R>();
+                    ray.d = jitterVector<R>(F.seed, sampleIndex, (unsigned)(F.recursion_limit - limit), (unsigned)li, 0u, la.w, -lv);
+                }
+            } else {
+                tmax = realmax_<R>();
+                ray.d = -lv;
+            }
+            phase = PH_SHADOW;
+            break;
+        }
+        if (li < S.n_lights) continue;  // a shadow ray is pending
+        // ---- level complete (getColourForRay's Seq.sumBy, Shading.fs:139) -----------------------------------------------
+        scol = scol + weight * local;
+        // reflectionShader (Shading.fs:89-98) sits inside the per-light sum: L identical re-traces => weight L * reflectance
+        if (f.applyLighting && f.reflectance > R(0) && limit > 0) {
+            weight = weight * ((R)S.n_lights * f.reflectance);
+            ray.o = f.p; ray.d = reflect(f.n, pathD);
+            --limit;
+            phase = PH_NEAREST;
+            cn.add(ST_REFLECTION);
+        } else {  // the sample is complete: park its colour in the unit's slot; take the next sample of the run, if any
+            R* c = &ring_col[wib][0][3 * (((rpos >> 12) & 0xf) * CAP + (rpos & 0xfff))];
+            c[0] = scol.x; c[1] = scol.y; c[2] = scol.z;
+            retire = true;
+            rpos -= 0xffff;  // one sample fewer in the run, one position further
+            if ((rpos >> 16) > 0) { ++sj; if constexpr (kCarryIndex) ++sampleIndex; phase = PH_START; } else phase = PH_IDLE;
+        }
+    }
+    if (overflow) atomicExch(F.overflow, 1u);
+    if constexpr (STATS) {
+        for (int i = 0; i < ST_COUNT; ++i) {
+            unsigned long long v = cn.get(i);
+            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(full, v, o);
+            if (lane == 0 && v) atomicAdd(F.stats + i, v);
+        }
+    }
+}
+
+template <typename R, unsigned FEAT, bool WITH_STATS>
+cudaError_t launch_samples_impl(const DevScene<R>& s, const DevFrame<R>& f, const unsigned long long* keys, bool stats, int sm_count, cudaStream_t stream,
+                                int* launches)
+{
+    if (!WITH_STATS && stats) return cudaErrorInvalidValue;
+    int per_sm = 0;
+    cudaError_t e = stats ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, samples_kernel<R, FEAT, WITH_STATS>, kBlockThreads, 0)
+                          : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, samples_kernel<R, FEAT, false>, kBlockThreads, 0);
+    if (e != cudaSuccess) return e;
+    if (per_sm < 1) per_sm = 1;
+    // persistent grid: a multiple of the SM count, never more warps than there are blocks of 32 pixels
+    const long long want = (long long)sm_count * per_sm, cap = ((long long)f.n_blocks + (kBlockThreads / 32) - 1) / (kBlockThreads / 32);
+    int grid = (int)(want < cap ? want : cap);
+    if (grid < 1) grid = 1;
+    if (stats) samples_kernel<R, FEAT, WITH_STATS><<<grid, kBlockThreads, 0, stream>>>(s, f, keys);
+    else samples_kernel<R, FEAT, false><<<grid, kBlockThreads, 0, stream>>>(s, f, keys);
+    if (launches) ++*launches;
+    return cudaGetLastError();
+}
+
 // ---- ray queries (Scene.closest / Scene.lightIsBocked on caller-supplied rays) -----------------------------------------
 // A kernel of its own, so that render_kernel's code and register allocation stay exactly what they are.  Warps take groups of
 // 32 rays from the per-device queue counter (like mode 1 of render_kernel); each lane traces its ray exactly as given: no

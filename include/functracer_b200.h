@@ -469,6 +469,45 @@ int ftb_trace_paths(ftb_scene* scene, const double* rays_od, const uint64_t* sam
 int ftb_trace_paths_device(ftb_scene* scene, const double* d_rays_od, const uint64_t* d_sample_keys, int64_t n,
                            const ftb_render_params* params, const ftb_path_out* d_out, ftb_stats* stats, void* stream);
 
+/* ---- a frame's own samples: SamplingStrategy.generateRays / blendPixels (Image.fs:100-116) with the rays in the caller's hands ----
+ * ftb_frame_rays writes the primary ray and RNG key of every sample of the window [x0, x1) x [y0, y1) of the frame camera + params
+ * describe, exactly as the render kernel generates them:
+ *   - entries in the debug planes' order and count (see ftb_render_window): jitter sampling (x1-x0)*(y1-y0)*spp entries, sample-major
+ *     within a pixel, pixels row-major within the window; corner sampling the (x1-x0+1)*(y1-y0+1) corner grid;
+ *   - rays_od: o.xyz d.xyz before slightOffset and after depth-of-field jitter, the kernel's own values widened to double (FP32 rays
+ *     narrow back exactly); sample_keys: (py * gw + px) * spp + s, gw the frame's sample-grid width (width, or width + 1 for corners);
+ *   - params: only width, height, spp, sampling, jitter_xy, precision and seed are read, and checked as ftb_render_window checks them
+ *     (the window too), before any device is looked for; either output pointer may be NULL.
+ * ftb_shade_samples shades n_pixels * spp caller-supplied rays (sample s of pixel i is ray i * spp + s) and blends each pixel as
+ * ftb_render blends a jitter-mode pixel: Array.average in sample order, in the same passes and fold segments a frame of that spp uses
+ * in the same kernel variant.  Each ray is shaded as ftb_shade_rays shades it, with the RNG key sample_keys[i * spp + s]
+ * (NULL: the ray's index i * spp + s; with spp = 1 that is what ftb_shade_rays uses).
+ *   - out: n_pixels pixels in params->out_format (RGBA8: Image.write's quantisation); dbg, if given, holds n_pixels * spp entries per
+ *     plane, as ftb_shade_rays' debug planes do; planes not asked for are not touched.
+ *   - params: only spp (>= 1), precision, seed, recursion_limit, out_format and collect_stats are read.  sampling is not: corner
+ *     frames blend across pixels.  The variant is picked from the scene's features, as for ftb_shade_rays.
+ *   - Contract: shading a window's ftb_frame_rays output with its keys and the same params gives ftb_render_window's result for that
+ *     window bit for bit, in every out_format and in the debug planes.  Always in FP64; in FP32 whenever the frame runs the variant this
+ *     call runs.  A depth-of-field frame adds FT_RNG to the scene's features and may run another variant: its FP32 pixels then agree
+ *     only to FP32 rounding.
+ *   - The counting kernel counts primary, shadow and reflection rays and shaded hits as the frame's counting kernel does for the same
+ *     samples (the frame adds its clear tiles' samples and the shadow rays it skips on lit ground tiles, as it counts them).
+ *   - Bad arguments, checked before any device is looked for: FTB_ERR_BAD_ARG for a NULL scene or params, n_pixels < 0, spp < 1,
+ *     NULL rays or out with n_pixels > 0, more than 0x7fffff00 pixels or n_pixels * spp past ftb_shade_rays' ray limit, a bad precision
+ *     or out_format.  n_pixels = 0 is OK; no CUDA device: FTB_ERR_NO_DEVICE.
+ *   - A hit-stack overflow is reported as by the queries (the host entry then leaves the caller's arrays unwritten); one frame or query
+ *     in flight per scene and device; the device entries synchronise only to fill stats. */
+int ftb_frame_rays(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params,
+                   int32_t x0, int32_t y0, int32_t x1, int32_t y1, double* rays_od, uint64_t* sample_keys);
+int ftb_frame_rays_device(ftb_scene* scene, const ftb_camera* camera, const ftb_render_params* params,
+                          int32_t x0, int32_t y0, int32_t x1, int32_t y1, double* d_rays_od, uint64_t* d_sample_keys,
+                          void* stream);
+int ftb_shade_samples(ftb_scene* scene, const double* rays_od, const uint64_t* sample_keys, int64_t n_pixels,
+                      const ftb_render_params* params, void* out, const ftb_debug_out* dbg, ftb_stats* stats);
+int ftb_shade_samples_device(ftb_scene* scene, const double* d_rays_od, const uint64_t* d_sample_keys, int64_t n_pixels,
+                             const ftb_render_params* params, void* d_out, const ftb_debug_out* d_dbg, ftb_stats* stats,
+                             void* stream);
+
 #ifdef __cplusplus
 }
 #endif

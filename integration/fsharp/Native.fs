@@ -186,6 +186,17 @@ extern int ftb_intersect_all_rays(nativeint scene, nativeint raysOD, int64 n, in
 /// sample keys of the soft lights' RNG, 0n = the ray's index (what ftb_shade_rays uses)
 [<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
 extern int ftb_trace_paths(nativeint scene, nativeint raysOD, nativeint keysOrNull, int64 n, FtbRenderParams& p, nativeint pathOut, nativeint statsOrNull)
+/// SamplingStrategy.generateRays (Image.fs:100-111) as the render kernel runs it: the primary ray (o.xyz d.xyz, before
+/// slightOffset, after depth-of-field jitter) and the RNG key ((py * gw + px) * spp + s) of every sample of the window
+/// [x0, x1) x [y0, y1), in the debug planes' order (sample-major within a pixel; corner sampling: the corner grid).
+/// raysODOrNull: 6 doubles per sample, keysOrNull: one uint64 per sample (0n = not wanted)
+[<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+extern int ftb_frame_rays(nativeint scene, FtbCamera& camera, FtbRenderParams& p, int x0, int y0, int x1, int y1, nativeint raysODOrNull, nativeint keysOrNull)
+/// Shading.shade + JitterSampling.blendPixels (Image.fs:112-116) on caller-supplied rays: nPixels * p.spp rays (sample s of pixel
+/// i is ray i * p.spp + s), each shaded as ftb_shade_rays shades it with the RNG key keysOrNull[i * spp + s] (0n = the ray's
+/// index), each pixel blended as ftb_render blends it; out = nPixels pixels in p.outFormat (2 = RGBA8: Image.write's bytes)
+[<DllImport(Lib, CallingConvention = CallingConvention.Cdecl)>]
+extern int ftb_shade_samples(nativeint scene, nativeint raysOD, nativeint keysOrNull, int64 nPixels, FtbRenderParams& p, nativeint out, nativeint dbgOrNull, nativeint statsOrNull)
 
 let lastError () = Marshal.PtrToStringAnsi (ftb_last_error ())
 let check rc = if rc <> 0 then failwithf "functracer_b200 status %d: %s" rc (lastError ())
