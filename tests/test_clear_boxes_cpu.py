@@ -56,8 +56,12 @@ extern "C" int ftb_probe_clear(const ftb_scene_desc* d, const ftb_camera* c, con
 
 @pytest.fixture(scope="module")
 def probe(tmp_path_factory):
-    d = tmp_path_factory.mktemp("boxes_probe")
-    src, so = os.path.join(str(d), "probe.cpp"), os.path.join(str(d), "libprobe.so")
+    return build_probe(str(tmp_path_factory.mktemp("boxes_probe")))
+
+
+def build_probe(d):
+    """The probe library, compiled into directory d."""
+    src, so = os.path.join(d, "probe.cpp"), os.path.join(d, "libprobe.so")
     open(src, "w").write(PROBE % dict(csrc=CSRC))
     subprocess.check_call(["g++", "-O1", "-std=c++17", "-fPIC", "-shared", "-o", so, src] +
                           [os.path.join(CSRC, "cuda", f) for f in ("clear_boxes.cpp", "tiles.cpp", "lower.cpp")])

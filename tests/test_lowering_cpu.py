@@ -86,8 +86,12 @@ LARGE_MESH = 32768  # api.cu kLargeMesh
 
 @pytest.fixture(scope="module")
 def probe(tmp_path_factory):
-    d = tmp_path_factory.mktemp("lower_probe")
-    src, so = os.path.join(str(d), "probe.cpp"), os.path.join(str(d), "libprobe.so")
+    return build_probe(str(tmp_path_factory.mktemp("lower_probe")))
+
+
+def build_probe(d):
+    """The probe library, compiled into directory d."""
+    src, so = os.path.join(d, "probe.cpp"), os.path.join(d, "libprobe.so")
     open(src, "w").write(PROBE % dict(csrc=CSRC, tests=os.path.dirname(os.path.abspath(__file__))))
     subprocess.check_call(["g++", "-O1", "-std=c++17", "-fPIC", "-shared", "-o", so, src, os.path.join(CSRC, "cuda", "lower.cpp")])
     lib = C.CDLL(so)
