@@ -132,6 +132,7 @@ static_assert((unsigned)FT_TABLE == kFeatOriginTable, "lower.h and device_scene.
     cudaError_t query_f32_##feat(const DevScene<float>&, const DevQuery&, bool, int, cudaStream_t, int*); \
     cudaError_t samples_f32_##feat(const DevScene<float>&, const DevFrame<float>&, const unsigned long long*, bool, int, cudaStream_t, int*);
 FTB_FEAT_LIST_F32
+FTB_FEAT_LIST_F32_TMASK
 #undef X
 #define X(feat) cudaError_t launch_f64_##feat(const DevScene<double>&, const DevFrame<double>&, bool, int, cudaStream_t, int*); \
     cudaError_t query_f64_##feat(const DevScene<double>&, const DevQuery&, bool, int, cudaStream_t, int*); \
@@ -163,6 +164,12 @@ static const Variant<double> kVariantsF64[] = {
     FTB_FEAT_LIST_F64
 #undef X
 };
+// the FT_TMASK instances (-DFTB_FEAT_LIST_F32_TMASK): picked by withTileMasks, never by pickCover
+static const Variant<float> kTMaskVariantsF32[] = {
+#define X(feat) {(unsigned)(feat), UnitCap<float, (unsigned)(feat)>::value, false, launch_f32_##feat, query_f32_##feat, samples_f32_##feat},
+    FTB_FEAT_LIST_F32_TMASK
+#undef X
+};
 template <typename R> struct VariantTable;
 template <> struct VariantTable<float> { static const Variant<float>* begin() { return kVariantsF32; } static int size() { return (int)(sizeof(kVariantsF32) / sizeof(kVariantsF32[0])); } };
 template <> struct VariantTable<double> { static const Variant<double>* begin() { return kVariantsF64; } static int size() { return (int)(sizeof(kVariantsF64) / sizeof(kVariantsF64[0])); } };
@@ -190,6 +197,16 @@ const Variant<R>* pickVariant(unsigned need, bool stats)
         if (w && w->feat != FT_ALL) return w;
     }
     return v;
+}
+// The instance of variant v that reads the per-tile item masks (FT_TMASK), if one is compiled: FP32 only.
+template <typename R>
+const Variant<R>* withTileMasks(const Variant<R>* v)
+{
+    if constexpr (sizeof(R) == 4) {
+        for (const Variant<float>& w : kTMaskVariantsF32)
+            if (w.feat == (v->feat | (unsigned)FT_TMASK)) return &w;
+    }
+    return nullptr;
 }
 }  // namespace ftb
 
@@ -314,7 +331,7 @@ struct PerDevice {
     cudaStream_t stream = nullptr;  // owned; used by the host-buffer entry points
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, done = nullptr;
     ControlBlock control;
-    DevBuf jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order, lit;
+    DevBuf jitter, tiles, out, dbg_prim, dbg_sub, dbg_t, rays, order, lit, items;
     DevBuf query;  // the host-buffer ray queries: max_t and the requested output planes
     std::vector<int> chunk_first;          // first position in the tile order of every chunk (+ end)
     std::vector<int> chunk_clear;          // position in the tile order where every chunk's clear tiles start
@@ -324,6 +341,7 @@ struct PerDevice {
     std::vector<unsigned char> order_key;  // what the cached tile order was computed for
     bool order_valid = false;
     int lit_leaf = -1;  // the cached lit-tile mask's ground leaf (in `lit`); -1: no tile is lit
+    bool items_valid = false;  // `items` holds the cached per-tile item masks, and they pay (computeTileOrder)
     std::vector<DevBuf> peer_tiles;  // on the gather device: one per remote shard
 
     PerDevice() = default;
@@ -339,7 +357,7 @@ struct PerDevice {
             if (stream) cudaStreamSynchronize(stream);
             if (copy_stream) cudaStreamSynchronize(copy_stream);
             f32.release(); f64.release();
-            for (DevBuf* b : {&control.buf, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order, &lit, &query}) b->release();
+            for (DevBuf* b : {&control.buf, &jitter, &tiles, &out, &dbg_prim, &dbg_sub, &dbg_t, &rays, &order, &lit, &items, &query}) b->release();
             for (DevBuf& b : peer_tiles) b.release();
             if (ev0) cudaEventDestroy(ev0);
             if (ev1) cudaEventDestroy(ev1);
@@ -669,16 +687,23 @@ inline int bandPixelRow(int k, int n, int tiles_y, int height) { return std::min
 // tiles first, so the tail consists of cheap ones.  Ordering cannot change any pixel: tiles are independent.
 // Clear tiles (tiles.h: no primary sample hits anything, by the items' spheres and boxes, clear_boxes.h) go last in each chunk, from chunk_clear[k] on: the kernel writes
 // their pixels without tracing.
-// lit / lit_leaf: the window's lit ground tiles (lit_tiles.h), indexed by the window's tile, not the shard's.
+// lit / lit_leaf: the window's lit ground tiles (lit_tiles.h), items: the window's per-tile item masks (tiles.h), both indexed by
+// the window's tile, not the shard's.  items is left empty when there are none or when they do not pay: they must leave at most
+// kTileMaskKept of the bits the spheres alone keep in the traced tiles, or the FT_TMASK instance's extra path costs more than they
+// save (measured, profiles/r7a_tile_items_ab.txt: repeat keeps 0.41 of them and runs 6.0 % faster; house keeps 0.61 and night-house
+// 0.81, and both run 1.5 % and 5.0 % slower with the masks).
+constexpr double kTileMaskKept = 0.5;
 // Returns false when every tile has the same estimate and none is clear (no order needed).
 bool computeTileOrder(const ftb_scene& sc, const ftb_camera& c, const ftb_render_params& p, const FrameGeom& g, int n_chunks, std::vector<int>& order,
-                      std::vector<int>& chunk_first, std::vector<int>& chunk_clear, std::vector<unsigned char>& lit, int& lit_leaf)
+                      std::vector<int>& chunk_first, std::vector<int>& chunk_clear, std::vector<unsigned char>& lit, int& lit_leaf, std::vector<unsigned>& items)
 {
     std::vector<float> cost;
     std::vector<unsigned char> clear;
     const TileGrid grid = {g.wx0, g.wy0, g.ww, g.wh, g.tiles_x, g.tiles_y};
     const std::vector<ImageRect> boxes = itemBoxRects(sc.L, c, p.width, p.height);
-    const bool any = estimateTiles(sc.L, (int)sc.lights.size(), c, p.width, p.height, p.recursion_limit, sampleOffsetExtent(p), grid, cost, clear, &boxes);
+    double kept = 1.0;
+    const bool any = estimateTiles(sc.L, (int)sc.lights.size(), c, p.width, p.height, p.recursion_limit, sampleOffsetExtent(p), grid, cost, clear, &boxes, &items, &kept);
+    if (kept > kTileMaskKept) items.clear();
     lit_leaf = litTiles(sc.L, sc.lights.data(), (int)sc.lights.size(), c, p.width, p.height, sampleOffsetExtent(p), grid, lit);
     // chunks = bands of tile rows (only used unsharded), see bandFirstRow
     auto tileOf = [&](int l) { return tileOfLocal(l, g.shard_index, g.shard_count); };
@@ -771,7 +796,8 @@ struct Launch {
         if (key != pd->order_key) {
             std::vector<int> order;
             std::vector<unsigned char> lit;
-            pd->order_valid = computeTileOrder(*sc, *cam, *p, g, n_chunks, order, pd->chunk_first, pd->chunk_clear, lit, pd->lit_leaf);
+            std::vector<unsigned> items;
+            pd->order_valid = computeTileOrder(*sc, *cam, *p, g, n_chunks, order, pd->chunk_first, pd->chunk_clear, lit, pd->lit_leaf, items);
             if (pd->order_valid) {
                 CK(pd->order.reserve(order.size() * sizeof(int)));
                 CK(cudaMemcpyAsync(pd->order.p, order.data(), order.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
@@ -780,11 +806,22 @@ struct Launch {
                 CK(pd->lit.reserve(lit.size()));
                 CK(cudaMemcpyAsync(pd->lit.p, lit.data(), lit.size(), cudaMemcpyHostToDevice, stream));
             }
-            if (pd->order_valid || pd->lit_leaf >= 0) CK(cudaStreamSynchronize(stream));  // `order` and `lit` are pageable locals
+            pd->items_valid = !items.empty();
+            if (pd->items_valid) {
+                CK(pd->items.reserve(items.size() * sizeof(unsigned)));
+                CK(cudaMemcpyAsync(pd->items.p, items.data(), items.size() * sizeof(unsigned), cudaMemcpyHostToDevice, stream));
+            }
+            // `order`, `lit` and `items` are pageable locals
+            if (pd->order_valid || pd->lit_leaf >= 0 || pd->items_valid) CK(cudaStreamSynchronize(stream));
             pd->order_key.swap(key);
         }
         F.lit_tiles = pd->lit_leaf >= 0 ? static_cast<const unsigned char*>(pd->lit.p) : nullptr;
         F.lit_leaf = pd->lit_leaf;
+        // the masks are proven for the FP32 kernels' rounding (tiles.h, clear_boxes.h); the FP64 build and the counting kernel
+        // trace every item
+        if (pd->items_valid) {
+            if (const Variant<R>* m = withTileMasks<R>(var)) { var = m; F.tile_items = static_cast<const unsigned*>(pd->items.p); }
+        }
         if (stats) CK(cudaEventRecord(pd->ev0, stream));
         return FTB_OK;
     }

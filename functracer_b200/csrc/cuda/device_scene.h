@@ -74,7 +74,9 @@ enum Feature : unsigned {
                        // (instruction footprint) and pairs whose operand is a run of leaves (lower.cpp, render.cuh csgPair)
     FT_MESHPK = 0x800,  // a LARGE mesh: mesh leaves are walked by the whole warp (render.cuh packetMesh) instead of by each lane (intersectMesh);
                         // variants with FT_MESH but without this bit only contain the per-lane walk, FT_ALL contains both (DevScene::mesh_packet)
-    FT_ALL = 0xfff
+    FT_ALL = 0xfff,
+    FT_TMASK = 0x1000  // not a scene feature: a variant that reads the per-tile item masks (DevFrame::tile_items, render.cuh TileMasks),
+                       // compiled beside the plain one for the Makefile's F32_TMASK_FEATS; api.cu launches it when the masks pay
 };
 
 enum StatSlot : int {
@@ -180,6 +182,10 @@ struct DevFrame {
     // every primary fragment of the tile on leaf lit_leaf sees directional light k unblocked (lit_tiles.h); nullptr: none
     const unsigned char* lit_tiles;
     int lit_leaf;
+    // mode 0, FP32 kernels, scenes of <= 32 items: one word per tile of the window's grid (global tile index), bit i = item i may
+    // be hit by a primary ray of the tile (tiles.h); the tile's primary rays trace no other item.  Set only for the FT_TMASK
+    // variants (api.cu prepareFrame).  nullptr: every item
+    const unsigned* tile_items;
 };
 
 // A batch of ray queries (query_kernel, render.cuh): caller-supplied rays traced exactly as given, nearest hit or occlusion.

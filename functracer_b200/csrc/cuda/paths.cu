@@ -144,7 +144,7 @@ __global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) path_ke
         if constexpr (sizeof(R) == 4 && (FEAT & FT_PLANAR) != 0) {
             if (f.planarLeaf >= 0 && (phase == PH_NEAREST ? limit < P.recursion_limit : dot(ray.d, f.n) >= R(0))) skipLeaf = f.planarLeaf;
         }
-        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, tr, phase == PH_NEAREST ? inf_<R>() : tmax, phase == PH_SHADOW, skipLeaf, (const R4*)nullptr, R(0),
+        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, tr, phase == PH_NEAREST ? inf_<R>() : tmax, phase == PH_SHADOW, skipLeaf, ~0u, (const R4*)nullptr, R(0),
                                                         overflow, cn, tracing, &mesh_stack[MeshWalks<FEAT>::kPacket ? wib : 0][0]);
 
         // ---- consume the result ---------------------------------------------------------------------------------------------

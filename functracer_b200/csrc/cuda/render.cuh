@@ -171,6 +171,11 @@ FTB_DEV F2 dup2(float x) { return pk2(x, x); }
 //   origin and direction through a matrix row as one pair: the variants of the simple scenes (moon -1.3 %); it costs the CSG variants
 //   72 bytes of spills for nothing (repeat +0.7 %, house -0.3 %, hollow-sphere +0.5 %).
 template <typename R, unsigned FEAT> struct PackedBounds { static constexpr bool value = sizeof(R) == 4 && (FEAT & (FT_PAIRG | FT_CSGN)) != 0; };
+// Per-tile item masks (DevFrame::tile_items) for primary rays: only in the variants compiled with FT_TMASK (the Makefile's
+// F32_TMASK_FEATS).  The extra path costs the house-family kernel 5.5-7.3 % whether or not a frame has masks
+// (profiles/r7a_tile_items_ab.txt), so it lives in a second instance of that variant, which api.cu launches only for frames whose
+// masks drop enough of phase A's candidates (repeat -6.0 %); every other frame runs the plain instance, which has no such path.
+template <typename R, unsigned FEAT> struct TileMasks { static constexpr bool value = sizeof(R) == 4 && (FEAT & FT_TMASK) != 0; };
 template <typename R, unsigned FEAT> struct PackedXform { static constexpr bool value = sizeof(R) == 4 && (FEAT & (FT_CUBE | FT_ROUND | FT_MESH | FT_CSG | FT_CSGN)) == 0; };
 
 template <typename R>
@@ -1000,9 +1005,11 @@ struct HitInfo {
 //   tab != nullptr (warp-uniform): every lane of this call traces a ray whose bound tests can be answered from its row
 //   of the common-origin table (primary rays from the camera, shadow rays towards a point light; built in the kernel's
 //   prologue); tabSlack = how far the ray's actual line can pass from that common point, as a distance along the ray.
+//   allow: the items of the first batch this ray may trace at all (a primary ray: its tile's mask, DevFrame::tile_items, which
+//   exists for scenes of one batch only); ~0u: every item.
 template <typename R, unsigned FEAT, bool STATS>
-FTB_DEV HitInfo<R> traceScene(const DevScene<R>& S, const Ray<R>& wr, R limit, bool any, int skipLeaf, const typename V4<R>::type* tab, R tabSlack, bool& overflow, Counters<STATS>& cn,
-                              unsigned tracing, int* wstack)
+FTB_DEV HitInfo<R> traceScene(const DevScene<R>& S, const Ray<R>& wr, R limit, bool any, int skipLeaf, unsigned allow, const typename V4<R>::type* tab, R tabSlack, bool& overflow,
+                              Counters<STATS>& cn, unsigned tracing, int* wstack)
 {
     typedef typename V4<R>::type R4;
     constexpr int kUnroll = BoundUnroll<FEAT>::value;  // (#pragma unroll takes constants, not macros)
@@ -1092,6 +1099,7 @@ FTB_DEV HitInfo<R> traceScene(const DevScene<R>& S, const Ray<R>& wr, R limit, b
                 }
             }
         }
+        cand &= allow;
         if (any) cand &= __ldg(S.item_casts + (base >> 5));  // items with nothing that has applyLighting cannot block (Scene.fs:121)
         unsigned meshCand = 0;  // mesh items are walked by the whole warp after this lane's other candidates
         constexpr bool kPacket = MeshWalks<FEAT>::kPacket;
@@ -1696,7 +1704,14 @@ __global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) render_
         if constexpr (sizeof(R) == 4 && (FEAT & FT_PLANAR) != 0) {  // `f` is still the fragment this bounce / shadow ray starts from
             if (f.planarLeaf >= 0 && (phase == PH_NEAREST ? limit < F.recursion_limit : dot(ray.d, f.n) >= R(0))) skipLeaf = f.planarLeaf;
         }
-        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, tr, phase == PH_NEAREST ? inf_<R>() : tmax, phase == PH_SHADOW, skipLeaf,
+        // A primary ray of a camera-grid frame traces only the items its tile's mask keeps (tiles.h): the others provably give
+        // it no crossing that the trace would report.
+        unsigned allow = ~0u;
+        if constexpr (TileMasks<R, FEAT>::value) {
+            if (F.tile_items && phase == PH_NEAREST && limit == F.recursion_limit)
+                allow = __ldg(F.tile_items + ((py - F.wy0) / FTB_TILE_H) * F.tiles_x + (px - F.wx0) / FTB_TILE_W);
+        }
+        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, tr, phase == PH_NEAREST ? inf_<R>() : tmax, phase == PH_SHADOW, skipLeaf, allow,
                                                         tabled ? origin_tab + (phase == PH_NEAREST ? 0 : 1 + li) * tabStride(S.n_items) : nullptr,
                                                         phase == PH_NEAREST ? F.primary_slack : R(4e-4) * tmax,
                                                         overflow, cn, tracing, &mesh_stack[MeshWalks<FEAT>::kPacket ? wib : 0][0]);
@@ -2054,7 +2069,7 @@ __global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) samples
         if constexpr (sizeof(R) == 4 && (FEAT & FT_PLANAR) != 0) {  // `f` is still the fragment this bounce / shadow ray starts from
             if (f.planarLeaf >= 0 && (phase == PH_NEAREST ? limit < F.recursion_limit : dot(ray.d, f.n) >= R(0))) skipLeaf = f.planarLeaf;
         }
-        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, tr, phase == PH_NEAREST ? inf_<R>() : tmax, phase == PH_SHADOW, skipLeaf,
+        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, tr, phase == PH_NEAREST ? inf_<R>() : tmax, phase == PH_SHADOW, skipLeaf, ~0u,
                                                         tabled ? origin_tab + (phase == PH_NEAREST ? 0 : 1 + li) * tabStride(S.n_items) : nullptr,
                                                         phase == PH_NEAREST ? F.primary_slack : R(4e-4) * tmax,
                                                         overflow, cn, tracing, &mesh_stack[MeshWalks<FEAT>::kPacket ? wib : 0][0]);
@@ -2230,7 +2245,7 @@ __global__ void __launch_bounds__(kBlockThreads, MinBlocks<FEAT>::value) query_k
         r.d = mk<R>((R)__ldg(q + 3), (R)__ldg(q + 4), (R)__ldg(q + 5));
         const R limit = any ? (R)__ldg(Q.max_t + i) : inf_<R>();
         cn.add(any ? ST_SHADOW : ST_PRIMARY);
-        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, r, limit, any, -1, (const typename V4<R>::type*)nullptr, R(0), overflow, cn, tracing,
+        const HitInfo<R> h = traceScene<R, FEAT, STATS>(S, r, limit, any, -1, ~0u, (const typename V4<R>::type*)nullptr, R(0), overflow, cn, tracing,
                                                         &mesh_stack[MeshWalks<FEAT>::kPacket ? wib : 0][0]);
         if (any) {
             Q.blocked[i] = h.leaf >= 0 ? 1 : 0;

@@ -40,13 +40,15 @@ double sampleOffsetExtent(const ftb_render_params& p)
 constexpr double kRel = 1e-5;
 
 bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int width, int height, int recursion_limit, double offset, const TileGrid& g,
-                   std::vector<float>& cost, std::vector<unsigned char>& clear, const std::vector<ImageRect>* box_rects)
+                   std::vector<float>& cost, std::vector<unsigned char>& clear, const std::vector<ImageRect>* box_rects, std::vector<unsigned>* items,
+                   double* kept)
 {
     const double kPiHalf = 1.5707963267948966;
     const CameraBasis b = cameraBasis(c, width, height);
     const size_t n_tiles = (size_t)g.tiles_x * g.tiles_y;
     cost.assign(n_tiles, 1.0f);
     clear.assign(n_tiles, 0);
+    if (items) items->clear();
     const double slack = offset + 0.05;  // pixels: the samples' offsets from their pixel centres and FP32 rounding of the image-plane position
     const double camR = std::sqrt(dot(b.o, b.o));
     const double primarySlack = 2e-4 * camR;  // DevFrame::primary_slack
@@ -60,20 +62,27 @@ bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int widt
         hi = t1 >= kPiHalf ? 1e300 : std::tan(t1);
         return true;
     };
-    // Clear tiles need the pinhole camera's rays (depth of field moves their origins) and an orthonormal basis (the projection
-    // below assumes one), and every unbounded item must be a top-level plane: (row . d, row . o + w) = the ray's y in the plane's frame.
-    bool clearable = !c.has_focus && std::isfinite(b.pw) && std::isfinite(b.ph) && b.pw > 0 && b.ph > 0 && std::isfinite(b.tlx) && std::isfinite(b.tly) &&
-                     std::isfinite(camR) && std::fabs(dot(b.i, b.i) - 1) < 1e-9 && std::fabs(dot(b.k, b.k) - 1) < 1e-9 && std::fabs(dot(b.i, b.k)) < 1e-9;
-    struct Plane { V3 row; double w; };
+    // The per-tile item masks need the pinhole camera's rays (depth of field moves their origins) and an orthonormal basis (the
+    // projection below assumes one).  An unbounded item keeps its bit everywhere unless it is a top-level plane:
+    // (row . d, row . o + w) = the ray's y in the plane's frame.
+    const bool pinhole = !c.has_focus && std::isfinite(b.pw) && std::isfinite(b.ph) && b.pw > 0 && b.ph > 0 && std::isfinite(b.tlx) && std::isfinite(b.tly) &&
+                         std::isfinite(camR) && std::fabs(dot(b.i, b.i) - 1) < 1e-9 && std::fabs(dot(b.k, b.k) - 1) < 1e-9 && std::fabs(dot(b.i, b.k)) < 1e-9;
+    struct Plane { V3 row; double w; unsigned bit; };
     std::vector<Plane> planes;
-    std::vector<unsigned char> touched(n_tiles, 0);
+    // mask[t] bit min(i, 31): item i may have a crossing with a primary ray of tile t that the kernel would report (items past
+    // the 31st share the last bit, so that mask == 0 still means "nothing")
+    std::vector<unsigned> mask(n_tiles, 0u);
+    // wide[t]: the bits the spheres alone keep, every unbounded item's included (the items phase A may keep for the tile)
+    std::vector<unsigned> wide(n_tiles, 0u);
     bool any = false;
     for (size_t item = 0; item < L.items.size(); ++item) {
         const Item& it = L.items[item];
+        const unsigned bit = 1u << std::min<size_t>(item, 31);
         if (it.bound_r < 0) {  // unbounded: the same cost everywhere
             const Leaf* lf = it.kind == ITEM_LEAF ? &L.leaves[(size_t)it.a] : nullptr;
-            if (!lf || lf->kind != LEAF_PLANE) clearable = false;
-            else planes.push_back(lf->identity ? Plane{{0, 1, 0}, 0} : Plane{{lf->w2m[4], lf->w2m[5], lf->w2m[6]}, lf->w2m[7]});
+            if (lf && lf->kind == LEAF_PLANE) planes.push_back(lf->identity ? Plane{{0, 1, 0}, 0, bit} : Plane{{lf->w2m[4], lf->w2m[5], lf->w2m[6]}, lf->w2m[7], bit});
+            else for (unsigned& m : mask) m |= bit;
+            for (unsigned& m : wide) m |= bit;
             continue;
         }
         double w = 1.0;
@@ -117,13 +126,15 @@ bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int widt
                 for (int tx = tx0; tx <= tx1; ++tx) cost[(size_t)ty * g.tiles_x + tx] += (float)w;
             any = true;
         }
-        // the tiles that are not clear: the radius beyond which the kernel's bound test drops the item for every primary ray -
-        // the device's inflated radius (api.cu uploadScene), widened by the 1e-6 |oc|^2 of the general test or by the 8e-6 |oc|^2
-        // and the primary slack of the common-origin table (render.cuh), and by the FP32 rounding of the ray and of the bound's
-        // centre - and the samples' largest offset from their pixel centres
+        // the tiles whose mask keeps the item: the radius beyond which the kernel's bound test drops the item for every primary
+        // ray - the device's inflated radius (api.cu uploadScene), widened by the 1e-6 |oc|^2 of the general test or by the
+        // 8e-6 |oc|^2 and the primary slack of the common-origin table (render.cuh), and by the FP32 rounding of the ray and of
+        // the bound's centre - and the samples' largest offset from their pixel centres
         const double ri = it.bound_r * 1.002 + 1e-5;
         const double r = std::sqrt(ri * ri + 2e-5 * oc * oc + 2.0 * oc * primarySlack + primarySlack * primarySlack) + kRel * (oc + camR + std::sqrt(dot(cen, cen)));
         if (!tileRect(r, slack)) continue;
+        for (int ty = ty0; ty <= ty1; ++ty)
+            for (int tx = tx0; tx <= tx1; ++tx) wide[(size_t)ty * g.tiles_x + tx] |= bit;
         if (box_rects && (*box_rects)[item].valid) {  // and that the item's boxes leave traced
             const ImageRect& q = (*box_rects)[item];
             const int sx0 = tx0, sx1 = tx1, sy0 = ty0, sy1 = ty1;
@@ -131,41 +142,43 @@ bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int widt
             tx0 = std::max(tx0, sx0); tx1 = std::min(tx1, sx1); ty0 = std::max(ty0, sy0); ty1 = std::min(ty1, sy1);
         }
         for (int ty = ty0; ty <= ty1; ++ty)
-            for (int tx = tx0; tx <= tx1; ++tx) touched[(size_t)ty * g.tiles_x + tx] = 1;
+            for (int tx = tx0; tx <= tx1; ++tx) mask[(size_t)ty * g.tiles_x + tx] |= bit;
     }
-    if (!clearable) return any;
+    if (!pinhole) return any;
     // A plane (y = 0 in its frame, Plane.fs) has no crossing at t >= 0 with a ray whose origin is strictly on one side and whose
     // direction leads away from it: t = -oy / dy < 0.  Plane.fs answers t = 0 for a ray parallel to it (|dy| < 1e-7) from below
     // or on it, so |dy| must stay clear of 1e-7 too.  dy is affine in the image-plane position (u, v) of the sample and the tile's
     // samples lie in a rectangle of (u, v): its corners bound dy over the whole tile.  The offset origin camera + 1e-4 d only
     // moves further away from the plane.
-    std::vector<double> side(planes.size());
-    for (size_t q = 0; q < planes.size(); ++q) {
-        const Plane& pl = planes[q];
-        const double oy = dot(pl.row, b.o) + pl.w;
-        side[q] = oy > 0 ? 1.0 : -1.0;
-    }
     for (int ty = 0; ty < g.tiles_y; ++ty)
         for (int tx = 0; tx < g.tiles_x; ++tx) {
             const size_t t = (size_t)ty * g.tiles_x + tx;
-            if (touched[t]) continue;
             const double c0 = g.wx0 + tx * FTB_TILE_W - slack, c1 = g.wx0 + tx * FTB_TILE_W + (FTB_TILE_W - 1) + slack;
             const double r0 = g.wy0 + ty * FTB_TILE_H - slack, r1 = g.wy0 + ty * FTB_TILE_H + (FTB_TILE_H - 1) + slack;
             const double us[2] = {b.tlx + c0 * b.pw, b.tlx + c1 * b.pw}, vs[2] = {b.tly - r0 * b.ph, b.tly - r1 * b.ph};
             // the scale of the rounding errors of d (absolute errors of jx, jy next to |tlx|, |tly|)
             const double dScale = std::sqrt(1.0 + std::max(us[0] * us[0], us[1] * us[1]) + std::max(vs[0] * vs[0], vs[1] * vs[1])) + std::fabs(b.tlx) + std::fabs(b.tly);
-            bool ok = true;
-            for (size_t q = 0; q < planes.size() && ok; ++q) {
-                const Plane& pl = planes[q];
+            for (const Plane& pl : planes) {
                 const double n = std::sqrt(dot(pl.row, pl.row));
                 const double oy = dot(pl.row, b.o) + pl.w;
-                ok = side[q] * oy > kRel * (n * (camR + dScale) + std::fabs(pl.w));
+                const double side = oy > 0 ? 1.0 : -1.0;
+                bool ok = side * oy > kRel * (n * (camR + dScale) + std::fabs(pl.w));
                 const double dk = dot(pl.row, b.k), di = dot(pl.row, b.i), dj = dot(pl.row, b.j);
                 for (int a = 0; a < 2 && ok; ++a)
-                    for (int e = 0; e < 2 && ok; ++e) ok = side[q] * (dk + us[a] * di + vs[e] * dj) > 1.0001e-7 + kRel * n * dScale;
+                    for (int e = 0; e < 2 && ok; ++e) ok = side * (dk + us[a] * di + vs[e] * dj) > 1.0001e-7 + kRel * n * dScale;
+                if (!ok) mask[t] |= pl.bit;
             }
-            clear[t] = ok ? 1 : 0;
+            clear[t] = mask[t] == 0 ? 1 : 0;
         }
+    if (items && L.items.size() <= 32) {
+        if (kept) {
+            double k = 0, w = 0;
+            for (size_t t = 0; t < n_tiles; ++t)
+                if (!clear[t]) { k += __builtin_popcount(mask[t]); w += __builtin_popcount(wide[t]); }
+            *kept = w > 0 ? k / w : 1.0;
+        }
+        items->swap(mask);
+    }
     return any;
 }
 

@@ -1,5 +1,6 @@
 // tiles.h — host-side estimates of a camera-grid frame's 16 x 16 tiles, before any ray is traced: the work each tile may
-// cost (api.cu orders the tiles by it) and which tiles provably see nothing (the kernel writes those without tracing).
+// cost (api.cu orders the tiles by it), which items each tile's primary rays can see (the kernel traces only those) and which
+// tiles provably see nothing (the kernel writes those without tracing).
 // Host-only C++, so that the CPU tests can run it on the real lowering.
 #pragma once
 
@@ -33,13 +34,19 @@ double sampleOffsetExtent(const ftb_render_params& p);
 
 // For every tile of the window, row-major:
 //   cost[t]  = 1 + the work weight of every item whose bounding sphere a primary ray of tile t may touch;
-//   clear[t] = 1 when no primary sample of tile t has a crossing at t >= 0 with anything: no item's bounding sphere is
-//              touched, and every unbounded item is a top-level plane that all of the tile's rays leave behind.  Such a
+//   items[t] = bit i set when item i may give a primary sample of tile t a crossing that the kernel reports: its bounding sphere
+//              is touched (and, with box_rects, its boxes' rectangle too), or it is unbounded and not a top-level plane that
+//              all of the tile's rays leave behind.  A clear bit: the item can be left out of the tile's primary rays' trace
+//              without changing any result.  Filled only for the pinhole camera and scenes of at most 32 items, else empty.
+//   clear[t] = 1 when no primary sample of tile t has a crossing at t >= 0 with anything: the tile's mask is 0.  Such a
 //              sample's colour is exactly zero.  Never set with depth of field or an unbounded item of another kind.
 // `offset` = sampleOffsetExtent.  Returns false when no bounded item touches the window (every cost is 1).
 // box_rects (per item, clear_boxes.h), when given: an item whose valid rectangle, widened by the samples' pixel slack, misses
-// a tile does not keep that tile from being clear even where its sphere is touched.  The costs use the spheres only.
+// a tile keeps no bit in that tile even where its sphere is touched.  The costs use the spheres only.
+// kept, with items filled: over the traced tiles, the bits the masks keep per bit the spheres alone keep (every unbounded item
+// counted as kept by both): how much of phase A's candidate work the masks leave.
 bool estimateTiles(const Lowered& L, int n_lights, const ftb_camera& c, int width, int height, int recursion_limit, double offset, const TileGrid& g,
-                   std::vector<float>& cost, std::vector<unsigned char>& clear, const std::vector<ImageRect>* box_rects = nullptr);
+                   std::vector<float>& cost, std::vector<unsigned char>& clear, const std::vector<ImageRect>* box_rects = nullptr,
+                   std::vector<unsigned>* items = nullptr, double* kept = nullptr);
 
 }  // namespace ftb
